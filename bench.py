@@ -3,8 +3,14 @@
 converge) of the per-locus Latent-Class-Model EM on synthetic 10M-fragment, ~20k-locus human-shaped
 batches (BASELINE.json configs[1]; generator strawberry_b200.synth.human_shaped, seeds 2, 3, ...).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR writes what the timed legs computed in their last step, as a caller of the path receives it, to
+DIR/<name>.npy (float64; integer outputs converted exactly): theta / fpkm / frac / tpm / keep per isoform and iters /
+status per locus of the headline, the same with a bias_ prefix plus bias_beta / bias_outer of the bias leg, and giant_*
+of the giant leg (no TPM there: a wave's TPM uses a placeholder denominator). With N > 1 ranks every rank writes its own
+loci as <name>.rank<r>.npy. The inputs are seeded, so two builds run with the same arguments can be compared file by file.
 
 A step = one pass of the hot path (EM to convergence + FPKM/frac/filter epilogue + TPM denominator) over
 the job. `value` is timed with the loci resident in HBM (CUDA events inside libsbq on the stream the
@@ -191,7 +197,10 @@ def main():
     ap.add_argument("--giant-rows", type=int, default=1_000_000)
     ap.add_argument("--giant-loci", type=int, default=200)
     ap.add_argument("--giant-wave", type=int, default=25, help="giant loci resident at once per GPU (~0.7 GB each)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step of every leg as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -298,6 +307,7 @@ def main():
     hd = timed_legs(q, pinned, total_reads, args.steps, args.warmup)
     clk.__exit__(None, None, None)
     st, launches, res = hd["st"], hd["launches"], hd["res"]
+    outputs = dict(res)                  # --dump-outputs: the headline's last resident step, then the other legs add theirs
     ms_per_step, e2e_per_step = reduce_max(hd["ms"], hd["e2e_s"])
     total_frag_iters, total_alg, total_launches = reduce_sum(st["frag_iters"], st["alg_bytes"], st["kernel_launches"])
     em_ms_max, = reduce_max(st["em_ms"])
@@ -374,18 +384,24 @@ def main():
     # ---- bias-in-EM leg: BASELINE configs[2] (the same 10M batch with per-row covariates), LPT-partitioned over the ranks
     if not args.no_bias:
         try:
-            line["bias"] = bias_leg(args, api, partition, synth, local_rank, rank, world, flush, reduce_max, reduce_sum, barrier, tpm_exchange)
+            line["bias"] = bias_leg(args, api, partition, synth, local_rank, rank, world, flush, reduce_max, reduce_sum, barrier, tpm_exchange, outputs)
         except Exception as e:
             line["bias"] = {"error": repr(e)}
 
     # ---- giant-locus leg: BASELINE configs[3], generated on the device, partitioned over the ranks, solved in waves
     if not args.no_giant:
         try:
-            line["giant"] = giant_leg(args, api, partition, synth, local_rank, rank, world, flush, reduce_max, reduce_sum, barrier, dist, peak, peak_src)
+            line["giant"] = giant_leg(args, api, partition, synth, local_rank, rank, world, flush, reduce_max, reduce_sum, barrier, dist, peak, peak_src, outputs)
         except Exception as e:   # the headline line must still be printed
             line["giant"] = {"error": repr(e)}
         if line.get("giant", {}).get("roofline_burst"):
             line["roofline_giant"] = line["giant"].pop("roofline_burst")      # the giant-locus kernel timed alone (burst); giant.roofline = over the whole 200-locus job
+
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in outputs.items():
+            fname = f"{name}.npy" if world == 1 else f"{name}.rank{rank}.npy"
+            np.save(os.path.join(args.dump_outputs, fname), np.asarray(a, dtype=np.float64))
 
     if rank == 0:
         if not args.no_cpu_baseline and world == 1:
@@ -402,7 +418,7 @@ GIANT_DRAM_BYTES_PER_NNZ_PASS = {"em_grid_dual_kernel": (10.854, "profiles/r02_g
                                  "em_grid_tma_kernel": (10.34, "profiles/r01_grid_tma_ncu_summary.txt")}
 
 
-def bias_leg(args, api, partition, synth, local_rank, rank, world, flush, reduce_max, reduce_sum, barrier, tpm_exchange):
+def bias_leg(args, api, partition, synth, local_rank, rank, world, flush, reduce_max, reduce_sum, barrier, tpm_exchange, outputs):
     """BASELINE configs[2]: the seed-2 10M-fragment batch with sequencing-bias correction inside the EM (bias_mode = 1), loci
     LPT-partitioned over the ranks. THE REFERENCE HAS NO BIAS IMPLEMENTATION (src/bias.cpp is commented out): the mode is our
     own definition (DESIGN.md section 7) and its only oracle is our CPU restatement - PARITY UNPINNED; no speed-up is quoted."""
@@ -418,16 +434,18 @@ def bias_leg(args, api, partition, synth, local_rank, rank, world, flush, reduce
     qb.set_covariates(X[rows])
     qb.upload()
     ms = []
-    for i in range(1 + 2):                      # one warm-up, two timed solves
+    n_solves = args.warmup + args.steps
+    for i in range(n_solves):
         flush.fill_(1)
         torch.cuda.synchronize()
         qb.solve(one["total_mapped_reads"])
         tpm_exchange(qb)
-        if i:
+        if i >= args.warmup:
             ms.append(qb.stats()["solve_ms"])
     qb.download()
     st, res = qb.stats(), qb.results()
-    _, outer = qb.bias_results()
+    beta, outer = qb.bias_results()
+    outputs.update({"bias_" + k: v for k, v in res.items()}, bias_beta=beta, bias_outer=outer)
     frag = np.add.reduceat(np.asarray(sub["count"], np.int64), np.asarray(sub["loc_row_off"])[:-1]) if len(parts[rank]) else np.zeros(0, np.int64)
     fi_local = float((frag * res["iters"]).sum())
     qb.close()
@@ -440,7 +458,7 @@ def bias_leg(args, api, partition, synth, local_rank, rank, world, flush, reduce
                        f"bias-corrected EM, LPT over {world} GPU(s)",
            "value": fi / (ms_max * 1e-3), "unit": UNIT, "ms_per_step": ms_max, "theta_iters_total": int(it_all), "outer_rounds_total": int(outer_all),
            "kernel": "em_bias_warp_kernel (small loci: one warp per locus, persistent warps) + em_bias_kernel (one cluster of 1 / 2 / 4 / 8 / 16 CTAs per locus by non-zeros, rows streamed from L2, partial sums exchanged through distributed shared memory)",
-           "gpu_launches": int(launches * 3)}
+           "gpu_launches": int(launches * n_solves)}
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         import oracle
         rng = np.random.default_rng(7)
@@ -457,11 +475,12 @@ def bias_leg(args, api, partition, synth, local_rank, rank, world, flush, reduce
     return out
 
 
-def giant_leg(args, api, partition, synth, local_rank, rank, world, flush, reduce_max, reduce_sum, barrier, dist, peak, peak_src):
+def giant_leg(args, api, partition, synth, local_rank, rank, world, flush, reduce_max, reduce_sum, barrier, dist, peak, peak_src, outputs):
     """BASELINE configs[3]: `giant_loci` loci of `giant_rows` single-fragment rows, k ~ 1 + Poisson(47) isoforms per row,
     T ~ U{500..800}, generated ON THE DEVICE from seed 4 (sbq_synth_giant: a locus is a pure function of (seed, global id), so
     the partition does not change the data). Loci are dealt to the ranks by LPT (equal expected cost: round robin) and solved
-    in waves of `giant_wave` resident loci. One pass over all loci = one step; EM time from CUDA events inside libsbq."""
+    in waves of `giant_wave` resident loci. One pass over all loci = one step, `steps` of them timed (times reported per step);
+    EM time from CUDA events inside libsbq."""
     import torch
     n, rows, seed = args.giant_loci, args.giant_rows, 4
     owner = partition.lpt_partition(np.full(n, rows * 48, np.int64), world)
@@ -491,9 +510,7 @@ def giant_leg(args, api, partition, synth, local_rank, rank, world, flush, reduc
         burst = dict(ms=float(np.mean(b_ms)), alg=bst["grid_alg_bytes"], nnz=bst["nnz"], iters=bst["em_iters_total"], n=len(bid), frag_iters=bst["frag_iters"],
                      kernel=next((r["kernel"] for r in qg.launch_stats() if r["kernel"].startswith("em_grid")), "em_grid_kernel"))
     barrier()
-    em_ms = solve_ms = gen_ms = 0.0
-    frag_iters = alg = iters = nnz = launches = 0
-    fpkm_local = 0.0
+    em_ms = solve_ms = gen_ms = 0.0                                  # summed over the steps
     kernel = "em_grid_kernel"
     wave_ms_per_pass = []
     # untimed warm-up at FULL wave size: the first full-size solve allocates the layout buffers of the grid tier (packed chunk stream,
@@ -506,29 +523,38 @@ def giant_leg(args, api, partition, synth, local_rank, rank, world, flush, reduc
     clk = ClockSampler(local_rank)
     clk.__enter__()
     t0 = time.perf_counter()
-    for ids in waves:
-        qg.clear()
-        qg.synth_giant(ids, rows, seed=seed)
-        flush.fill_(1)
-        torch.cuda.synchronize()
-        qg.solve(rows * n)                       # total_mapped_reads of the whole 200-locus job
-        fpkm_local += qg.fpkm_sum()
-        qg.finalize_tpm(1.0)                     # placeholder denominator: TPM of a wave needs the all-reduced sum of ALL waves
-        qg.download()
-        st = qg.stats()
-        em_ms += st["grid_em_ms"]
-        wave_ms_per_pass.append(round(st["grid_em_ms"] / max(st["em_iters_total"] + len(ids), 1), 5))
-        solve_ms += st["solve_ms"]
-        gen_ms += st["upload_ms"]
-        frag_iters += st["frag_iters"]
-        alg += st["grid_alg_bytes"]
-        iters += st["em_iters_total"]
-        nnz += st["nnz"]
-        launches += st["kernel_launches"]
-        kernel = next((r["kernel"] for r in qg.launch_stats() if r["kernel"].startswith("em_grid")), kernel)
+    for _ in range(args.steps):
+        frag_iters = alg = iters = nnz = launches = 0                # one pass: every step does the same work
+        fpkm_local = 0.0
+        step_res = []
+        for ids in waves:
+            qg.clear()
+            qg.synth_giant(ids, rows, seed=seed)
+            flush.fill_(1)
+            torch.cuda.synchronize()
+            qg.solve(rows * n)                       # total_mapped_reads of the whole 200-locus job
+            fpkm_local += qg.fpkm_sum()
+            qg.finalize_tpm(1.0)                     # placeholder denominator: TPM of a wave needs the all-reduced sum of ALL waves
+            qg.download()
+            st = qg.stats()
+            em_ms += st["grid_em_ms"]
+            wave_ms_per_pass.append(round(st["grid_em_ms"] / max(st["em_iters_total"] + len(ids), 1), 5))
+            solve_ms += st["solve_ms"]
+            gen_ms += st["upload_ms"]
+            frag_iters += st["frag_iters"]
+            alg += st["grid_alg_bytes"]
+            iters += st["em_iters_total"]
+            nnz += st["nnz"]
+            launches += st["kernel_launches"]
+            kernel = next((r["kernel"] for r in qg.launch_stats() if r["kernel"].startswith("em_grid")), kernel)
+            if args.dump_outputs:
+                step_res.append(qg.results())
     torch.cuda.synchronize()
-    wall = time.perf_counter() - t0
+    wall = (time.perf_counter() - t0) / args.steps
+    em_ms, solve_ms, gen_ms = em_ms / args.steps, solve_ms / args.steps, gen_ms / args.steps
     clk.__exit__(None, None, None)
+    if step_res:
+        outputs.update({"giant_" + k: np.concatenate([r[k] for r in step_res]) for k in ("theta", "fpkm", "frac", "keep", "iters", "status")})
     barrier()
     # the exchange step of this leg: the TPM denominator over all ranks and waves
     g = torch.tensor([fpkm_local], dtype=torch.float64, device=torch.device("cuda", local_rank))
