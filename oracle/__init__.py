@@ -59,6 +59,7 @@ def oracle_lib():
         _oracle.orc_em_csr.restype = ctypes.c_int
         _oracle.orc_epilogue.restype = ctypes.c_double
         _oracle.orc_quantify_batch.restype = ctypes.c_double
+        _oracle.orc_em_bias_csr.restype = ctypes.c_int
     return _oracle
 
 
@@ -153,10 +154,56 @@ def em_bias_csr(T, row_ptr, col, alpha, count, x, max_out_it=100, max_theta_it=5
     iters, outer = ctypes.c_int32(0), ctypes.c_int32(0)
     p = _BiasParams(max_out_it, max_theta_it, max_bias_it, theta_tol, bias_tol, row_eps)
     L = oracle_lib()
-    L.orc_em_bias_csr.restype = ctypes.c_int
     st = L.orc_em_bias_csr(T, len(count), _p(row_ptr), _p(col), _p(alpha), _p(count), _p(x) if x.size else None, K, ctypes.byref(p),
                            _p(theta), _p(beta), ctypes.byref(iters), ctypes.byref(outer))
     return st, theta, beta[:K], iters.value, outer.value
+
+
+def batch_epilogue(batch, theta, status, total_mapped_reads, min_iso_frac=0.0, effective_len_norm=False, insert_mean=0.0):
+    """FPKM / frac / keep per locus (orc_epilogue; NO_ROWS loci keep nothing) and the batch TPM over the kept isoforms, summed in
+    isoform order - the tail of orc_quantify_batch (sbq_oracle.c) applied to a given theta. -> dict(fpkm, frac, tpm, keep)."""
+    lio = np.asarray(batch["loc_iso_off"], np.int64)
+    il = _c(batch["iso_len"], np.int32)
+    NI = int(lio[-1])
+    fpkm, frac, tpm = np.zeros(NI), np.zeros(NI), np.zeros(NI)
+    keep = np.zeros(NI, np.int32)
+    for l in range(len(lio) - 1):
+        t0, t1 = int(lio[l]), int(lio[l + 1])
+        e = epilogue(theta[t0:t1], il[t0:t1], total_mapped_reads, min_iso_frac, effective_len_norm, insert_mean)
+        fpkm[t0:t1], frac[t0:t1] = e["fpkm"], e["frac"]
+        keep[t0:t1] = 0 if status[l] == ORC_NO_ROWS else e["keep"]
+    kept = np.where(keep != 0, fpkm, 0.0)
+    total_fpkm = float(np.cumsum(kept)[-1]) if NI else 0.0     # sequential, in isoform order, like the C loop
+    with np.errstate(divide="ignore", invalid="ignore"):
+        tpm[:] = 1e6 * fpkm / total_fpkm
+    return dict(fpkm=fpkm, frac=frac, tpm=tpm, keep=keep)
+
+
+def bias_quantify_batch(batch, X, total_mapped_reads, min_iso_frac=0.0, effective_len_norm=False, insert_mean=0.0, n_threads=8,
+                        **limits):
+    """Bias mode over a flat batch: em_bias_csr per locus on a thread pool (ctypes releases the GIL), then batch_epilogue.
+    X: (n_row, K) covariates in row order; limits: em_bias_csr's keywords. -> the keys of quantify_batch plus beta (L x K) and outer."""
+    from concurrent.futures import ThreadPoolExecutor
+    lro, lio, rp = (np.asarray(batch[k], np.int64) for k in ("loc_row_off", "loc_iso_off", "row_ptr"))
+    col, al, cnt = _c(batch["col"], np.int32), _c(batch["alpha"], np.float64), _c(batch["count"], np.int32)
+    X = np.asarray(X, np.float64)
+    L, K = len(lro) - 1, X.shape[1]
+    theta = np.zeros(int(lio[-1]))
+    beta = np.zeros((L, K))
+    status, iters, outer = np.zeros(L, np.int32), np.zeros(L, np.int32), np.zeros(L, np.int32)
+
+    def one(l):
+        r0, r1 = int(lro[l]), int(lro[l + 1])
+        k0, k1 = int(rp[r0]), int(rp[r1])
+        st, th, be, it, out = em_bias_csr(int(lio[l + 1] - lio[l]), rp[r0:r1 + 1] - k0, col[k0:k1], al[k0:k1], cnt[r0:r1], X[r0:r1], **limits)
+        theta[lio[l]:lio[l + 1]], beta[l] = th, be
+        status[l], iters[l], outer[l] = st, it, out
+
+    with ThreadPoolExecutor(max(1, int(n_threads))) as ex:
+        list(ex.map(one, range(L)))
+    out = batch_epilogue(batch, theta, status, total_mapped_reads, min_iso_frac, effective_len_norm, insert_mean)
+    out.update(theta=theta, iters=iters, status=status, beta=beta, outer=outer)
+    return out
 
 
 # ---------------------------------------------------------------- compiled reference (_ref/libsbref.so)

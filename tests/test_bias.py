@@ -47,6 +47,18 @@ def test_restatement_recovers_a_planted_bias_direction(oracle_mod):
     assert abs(th.sum() - L["count"].sum()) < 1e-6 * L["count"].sum()
 
 
+@pytest.mark.parametrize("opts", [{}, dict(min_iso_frac=0.01, effective_len_norm=True, insert_mean=250.0)])
+def test_batch_epilogue_reproduces_quantify_batch(oracle_mod, opts):
+    """The FPKM / frac / keep / TPM tail of oracle.bias_quantify_batch, fed quantify_batch's theta and status, gives
+    quantify_batch's own answers on the golden batch (pins the helper's arithmetic, TPM summation order included)."""
+    import util
+    b, *_ = util.load_golden()
+    ora = oracle_mod.quantify_batch(b, b["total_mapped_reads"], **opts)
+    got = oracle_mod.batch_epilogue(b, ora["theta"], ora["status"], b["total_mapped_reads"], **opts)
+    for k in ("fpkm", "frac", "tpm", "keep"):
+        assert np.array_equal(got[k], ora[k], equal_nan=True), k
+
+
 @pytest.mark.gpu
 def test_bias_kernel_matches_restatement(oracle_mod, sbq_lib_path):
     from strawberry_b200 import api

@@ -38,14 +38,14 @@ def expand_loci(per_locus, batch):
     return np.repeat(per_locus, np.diff(batch["loc_iso_off"]))
 
 
-def assert_matches_oracle(res, ora, batch, what=""):
+def assert_matches_oracle(res, ora, batch, what="", rel=REL_TOL):
     """CUDA results vs oracle results on the same batch: statuses and iteration counts equal,
-    theta / fpkm / frac / tpm within the parity bar, keep flags equal."""
+    theta / fpkm / frac / tpm within the parity bar (rel), keep flags equal."""
     bad_st = np.nonzero(res["status"] != ora["status"])[0]
     assert len(bad_st) == 0, f"{what}: status differs at loci {bad_st[:10]}: {res['status'][bad_st[:10]]} vs {ora['status'][bad_st[:10]]}"
     bad_it = np.nonzero(res["iters"] != ora["iters"])[0]
     assert len(bad_it) == 0, f"{what}: iteration count differs at loci {bad_it[:10]}: {res['iters'][bad_it[:10]]} vs {ora['iters'][bad_it[:10]]}"
-    ok, worst = theta_close(res["theta"], ora["theta"], batch)
+    ok, worst = theta_close(res["theta"], ora["theta"], batch, rel)
     assert ok.all(), f"{what}: theta off at {np.nonzero(~ok)[0][:10]}, worst ratio {worst:.3e}"
     live = expand_loci(ora["status"], batch) != 3
     for k in ("fpkm", "frac", "tpm"):
@@ -54,6 +54,6 @@ def assert_matches_oracle(res, ora, batch, what=""):
         assert np.array_equal(np.isfinite(a), fin), f"{what}: {k} finiteness differs"
         scale = np.maximum(np.abs(b[fin]), 1e-9 * max(float(np.nanmax(np.abs(b[fin]))) if fin.any() else 1.0, 1e-300))
         r = np.abs(a[fin] - b[fin]) / scale
-        assert (r <= 1e-6).all(), f"{what}: {k} worst ratio {r.max():.3e}"
+        assert (r <= rel).all(), f"{what}: {k} worst ratio {r.max():.3e}"
     assert np.array_equal(res["keep"] != 0, ora["keep"] != 0), f"{what}: keep flags differ"
     return worst
