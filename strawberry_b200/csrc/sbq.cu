@@ -37,12 +37,6 @@ namespace {
 
 constexpr size_t SMEM_CAP = CL_SMEM_CAP;   // dynamic shared memory we ask for at most (227 KB usable)
 constexpr int N_SIDE_STREAMS = 12;
-#ifndef SBQ_DEFAULT_WARP_CTAS
-#define SBQ_DEFAULT_WARP_CTAS 0   // 0 = SMs x occupancy
-#endif
-#ifndef SBQ_DEFAULT_ORDER
-#define SBQ_DEFAULT_ORDER 0
-#endif
 
 // ---- pinned host array with geometric growth -------------------------------------------------
 template <typename T>
@@ -113,6 +107,22 @@ struct LaunchTimer {      // CUDA events around one kernel launch, on the stream
    bool used = false;
 };
 
+// One class of giant-tier loci: 0 = the full grid on the main stream, 1 = the "small giants" (below SGRID_MAX_NNZ non-zeros, a
+// few thousand rows) on a SUB-GRID of SGRID_CTAS CTAs, on a stream of its own, so that the cluster and warp tiers keep the other
+// SMs (the full-grid launch of a 400 k-non-zero locus idles most of the GPU for milliseconds: its iterations are barrier latency,
+// not bandwidth). The same kernels run both classes.
+struct GridClass {
+   std::vector<int32_t> list;       // two-slot loci, then TMA ring loci, then register-staged loci (plan() sorts it)
+   std::vector<int64_t> rec_off;    // row-record offset of every two-slot locus (+ total), list order
+   size_t list_off = 0;             // offset into the device list buffer
+   size_t n_dual = 0, n_tma = 0;    // sizes of the two-slot and TMA ring parts of the list
+   int n_cta = 0;
+   int variant = 0;                 // the first kernel the last solve launched (sbq_launch_stat.variant)
+   DevBuf scratch, rowrec, pk;
+   cudaStream_t st = nullptr;
+   LaunchTimer lt;
+};
+
 }  // namespace
 
 struct MultiState;   // n_gpus > 1: one child context per device + the NCCL communicators (defined further down)
@@ -130,9 +140,9 @@ struct sbq_ctx {
    bool grid_ready = false;
    bool upload_pending = false;                         // upload_begin's copies have not been waited for yet
    cudaStream_t side[N_SIDE_STREAMS] = {};
-   cudaEvent_t ev[10] = {};
+   cudaEvent_t ev[9] = {};
    cudaEvent_t ev_fork = nullptr, ev_join[N_SIDE_STREAMS] = {};
-   LaunchTimer lt[N_SIDE_STREAMS + 2];          // [0] warp tier, [1] grid tier, [2+i] cluster class i
+   LaunchTimer lt[1 + N_SIDE_STREAMS];          // [0] warp tier, [1+i] cluster class i
    std::vector<sbq_launch_stat> launch_stats;   // filled by sbq_solve (+ bytes by sbq_download)
    std::vector<int32_t> locus_launch;           // locus -> index into launch_stats
    std::mutex mu;
@@ -197,32 +207,16 @@ struct sbq_ctx {
 
    // plan
    int force_tier = 0, force_cluster = 0;
-   std::vector<int32_t> warp_list, grid_list;
+   std::vector<int32_t> warp_list;
    std::vector<LaunchClass> classes;
+   GridClass grid[2];                           // [0] full grid on the main stream, [1] sub-grid on its own stream
    int warp_max_iso = 1;
    PinnedVec<int32_t> h_lists;
-   size_t warp_list_off = 0, grid_list_off = 0;
+   size_t warp_list_off = 0;
 
    // device
-   DevBuf d_in, d_out, d_lists, d_grid_scratch, d_col16, d_rowrec, d_csc, d_synth, d_pk;
-   bool col16_ready = false, grid_tma_ok = false, grid_dual_ok = false;
-   // "Small giants" (grid-tier loci below SGRID_MAX_NNZ non-zeros, a few thousand rows): the same grid kernels on a SUB-GRID of
-   // SGRID_CTAS CTAs, on a stream of their own, so that the cluster and warp tiers keep the other SMs (the full-grid launch of a
-   // 400 k-non-zero locus idles most of the GPU for milliseconds: its iterations are barrier latency, not bandwidth).
-   std::vector<int32_t> sgrid_list;
-   std::vector<int64_t> sgrid_rec_off;
-   size_t sgrid_list_off = 0, sgrid_n_dual = 0;
-   int sgrid_max_iso = 1, sgrid_max_iso_dual = 1, sgrid_variant = 0;
-   bool sgrid_tma_ok = false;
-   DevBuf d_sgrid_scratch, d_srowrec, d_spk;
-   cudaStream_t sgrid_st = nullptr;
-   cudaEvent_t ev_sgrid_join = nullptr;
-   LaunchTimer lt_sgrid;
-   std::vector<int64_t> grid_rec_off;            // row-record offset of every two-slot-kernel locus (+ total), list order
-   size_t grid_n_dual = 0;                       // the first grid_n_dual entries of grid_list run on the two-slot kernel, the rest on the TMA ring / register-staged kernel
-   int grid_max_iso_dual = 1;
-   int grid_max_iso = 1;
-   int grid_variant = 0;                         // which giant-locus kernel the last solve used (sbq_launch_stat.variant)
+   DevBuf d_in, d_out, d_lists, d_col16, d_csc, d_synth;
+   bool col16_ready = false;
    DevParams dp{};
    double* d_tpm = nullptr;
    double* d_fpkm_sum = nullptr;
@@ -332,32 +326,18 @@ constexpr int N_BUCKETS = 5;
 const int BUCKET_NT[N_BUCKETS] = {64, 128, 512, 512, 512};
 int smem_bucket(size_t bytes) { return bytes <= 12 * 1024 ? 0 : bytes <= 24 * 1024 ? 1 : bytes <= 56 * 1024 ? 2 : bytes <= 112 * 1024 ? 3 : 4; }
 
+constexpr int64_t GRID_MIN_NNZ = 300 * 1000;         // loci of at least this many non-zeros go to the grid tier
 constexpr int64_t SGRID_MAX_NNZ = 1000 * 1000;       // grid-tier loci below this run on a sub-grid (their passes are barrier latency; above, bandwidth starts to count) ...
-constexpr int SGRID_CTAS_DEFAULT = 32;               // ... of this many CTAs (one per SM), beside the other tiers
-inline int sgrid_ctas() {                            // SBQ_SGRID_CTAS overrides (tuning aid; changes the summation order of those loci)
-   static const int v = getenv("SBQ_SGRID_CTAS") ? std::max(1, atoi(getenv("SBQ_SGRID_CTAS"))) : SGRID_CTAS_DEFAULT;
-   return v;
-}
-#define SGRID_CTAS sgrid_ctas()
+constexpr int SGRID_CTAS = 32;                       // ... of this many CTAs (one per SM), beside the other tiers
 
 int cluster_size_for(int64_t nnz) {
    // ~14 B of shared memory per non-zero (row part + CSC index): a CTA's slice stays under ~14k non-zeros, which still
    // fits with its CSC index. Smaller clusters cost latency per iteration (fewer SMs per locus) but less SM time in
    // total; these thresholds were the best of a sweep on the human-shaped workload (profiles/r01_cluster_thresholds.txt).
-   // SBQ_CS_THRESH="a,b,c,d" (thousands of non-zeros) overrides the four thresholds (tuning aid).
-   static int64_t th[4] = {16 * 1024, 32 * 1024, 64 * 1024, 150 * 1024};
-   static bool init = false;
-   if (!init) {
-      init = true;
-      if (const char* e = std::getenv("SBQ_CS_THRESH")) {
-         long long a, b, c2, d;
-         if (std::sscanf(e, "%lld,%lld,%lld,%lld", &a, &b, &c2, &d) == 4) { th[0] = a * 1024; th[1] = b * 1024; th[2] = c2 * 1024; th[3] = d * 1024; }
-      }
-   }
-   if (nnz <= th[0]) return 1;
-   if (nnz <= th[1]) return 2;
-   if (nnz <= th[2]) return 4;
-   if (nnz <= th[3]) return 8;
+   if (nnz <= 16 * 1024) return 1;
+   if (nnz <= 32 * 1024) return 2;
+   if (nnz <= 64 * 1024) return 4;
+   if (nnz <= 150 * 1024) return 8;
    return 16;
 }
 
@@ -374,26 +354,16 @@ void capture_meta_host(sbq_ctx* c) {
 // works from c->meta only, so that batches that exist only on the device (sbq_synth_giant) are planned the same way
 int plan(sbq_ctx* c) {
    c->warp_list.clear();
-   c->grid_list.clear();
-   c->sgrid_list.clear();
-   c->sgrid_max_iso = c->sgrid_max_iso_dual = 1;
-   c->sgrid_tma_ok = true;
+   for (auto& g : c->grid) g.list.clear();
    c->classes.clear();
    c->warp_max_iso = 1;
    c->max_iso_all = 1;
-   c->grid_max_iso = 1;
-   c->grid_max_iso_dual = 1;
-   c->grid_tma_ok = true;
-   c->grid_dual_ok = !getenv("SBQ_GRID_NO_DUAL");   // two-slot layout kernel (sbq_grid_dual.cuh) for the loci that qualify
-   const bool force_dual = getenv("SBQ_GRID_DUAL") != nullptr;
-   static const bool sgrid_enabled = !getenv("SBQ_NO_SGRID");   // tuning aid: every grid-tier locus on the full grid
-   std::vector<char> dual_locus(c->n_loci, 0);
+   enum { DUAL, TMA, REG };
+   std::vector<char> grid_kernel(c->n_loci, 0);   // giant loci: which of the three grid kernels solves the locus
    std::vector<int64_t> nnz_of(c->n_loci);
    LaunchClass* slot[5][N_BUCKETS] = {};
    std::vector<LaunchClass> tmp;
    tmp.reserve(20);
-   // above this a locus goes to the grid tier (SBQ_GRID_MIN_NNZ overrides: tuning aid)
-   static const int64_t grid_min_nnz = getenv("SBQ_GRID_MIN_NNZ") ? atoll(getenv("SBQ_GRID_MIN_NNZ")) : 300 * 1000;
    for (int64_t l = 0; l < c->n_loci; ++l) {
       const int64_t R = c->meta[l].R, T = c->meta[l].T, nnz = c->meta[l].nnz;
       nnz_of[l] = nnz;
@@ -405,7 +375,7 @@ int plan(sbq_ctx* c) {
       // here even though a lane then walks several rows: they are latency-bound either way, and a CTA of the cluster tier would
       // hold 4 - 30 times more of the SM per iteration (plus its one-off sort / transposed-index setup)
       else if (T <= WT_MAX_ISO && R <= WT_MAX_ROWS && nnz <= WT_MAX_NNZ) tier = 1;
-      else if (nnz >= grid_min_nnz) tier = 3;
+      else if (nnz >= GRID_MIN_NNZ) tier = 3;
       else tier = 2;
       if (tier == 1 && T > WT_MAX_ISO) tier = 2;
       // every T <= SBQ_MAX_ISO fits both the cluster tier (streaming accumulators) and the register-staged grid kernel;
@@ -419,22 +389,13 @@ int plan(sbq_ctx* c) {
          c->warp_list.push_back((int32_t)l);
          c->warp_max_iso = std::max(c->warp_max_iso, (int)T);
       } else if (tier == 3) {
-         // sub-grid class: a function of the locus alone (a forced tier - tests, tools - keeps the full grid)
-         const bool small = !c->force_tier && sgrid_enabled && nnz < SGRID_MAX_NNZ;
-         (small ? c->sgrid_list : c->grid_list).push_back((int32_t)l);
-         // bank-aligned two-slot layout: 16-bit slot offsets, 32-bit offsets inside the locus, rows short enough on average
-         const bool dual = c->grid_dual_ok && (grid_dual_supports_iso((int)T) || (force_dual && grid_dual_possible((int)T))) &&
-                           nnz < (1LL << 32) && nnz <= 56 * R;
-         dual_locus[l] = dual;
-         int& mx_dual = small ? c->sgrid_max_iso_dual : c->grid_max_iso_dual;
-         int& mx_rest = small ? c->sgrid_max_iso : c->grid_max_iso;
-         bool& tma_ok = small ? c->sgrid_tma_ok : c->grid_tma_ok;
-         if (dual) {
-            mx_dual = std::max(mx_dual, (int)T);
-         } else {
-            mx_rest = std::max(mx_rest, (int)T);
-            if (!grid_tma_supports((int)T, (long long)R, small ? SGRID_CTAS : c->prop.multiProcessorCount)) tma_ok = false;
-         }
+         // class and kernel are functions of the locus alone (a forced tier - tests, tools - keeps the full grid): the bank-aligned
+         // two-slot layout (16-bit slot offsets, 32-bit offsets inside the locus, rows short enough on average), else the TMA ring,
+         // else the register-staged kernel
+         GridClass& g = c->grid[!c->force_tier && nnz < SGRID_MAX_NNZ];
+         g.list.push_back((int32_t)l);
+         grid_kernel[l] = grid_dual_supports_iso((int)T) && nnz < (1LL << 32) && nnz <= 56 * R ? DUAL :
+                          grid_tma_supports((int)T, (long long)R, g.n_cta) ? TMA : REG;
       } else {
          int cs = c->force_cluster ? c->force_cluster : cluster_size_for(nnz);
          int csi = cs == 1 ? 0 : cs == 2 ? 1 : cs == 4 ? 2 : cs == 8 ? 3 : 4;
@@ -469,24 +430,24 @@ int plan(sbq_ctx* c) {
          std::sort(c->warp_list.begin(), c->warp_list.end(), by_size);
       }
    }
-   // two-slot-kernel loci first, each part by descending size
-   // (within the two-slot part: by the warp count the locus' own T allows, so that every launch group is homogeneous)
-   auto order_grid = [&](std::vector<int32_t>& list, size_t& n_dual, std::vector<int64_t>& rec_off) {
-      std::sort(list.begin(), list.end(), [&](int32_t a, int32_t b) {
-         if (dual_locus[a] != dual_locus[b]) return dual_locus[a] > dual_locus[b];
-         if (dual_locus[a]) {
-            const int na = grid_dual_nc(c->meta[a].T), nb_ = grid_dual_nc(c->meta[b].T);
-            if (na != nb_) return na > nb_;
-         }
+   // two-slot loci, then TMA ring loci, then register-staged loci; inside the first two parts by the warp count the locus' own T
+   // selects, so that every launch is homogeneous; then by descending size
+   auto warps = [&](int32_t l) { return grid_kernel[l] == DUAL ? grid_dual_nc(c->meta[l].T) : grid_kernel[l] == TMA ? grid_tma_nc(c->meta[l].T) : 0; };
+   for (auto& g : c->grid) {
+      std::sort(g.list.begin(), g.list.end(), [&](int32_t a, int32_t b) {
+         if (grid_kernel[a] != grid_kernel[b]) return grid_kernel[a] < grid_kernel[b];
+         const int na = warps(a), nb_ = warps(b);
+         if (na != nb_) return na > nb_;
          return by_size(a, b);
       });
-      n_dual = 0;
-      for (int32_t l : list) n_dual += dual_locus[l];
-      rec_off.assign(n_dual + 1, 0);
-      for (size_t i = 0; i < n_dual; ++i) rec_off[i + 1] = rec_off[i] + c->meta[list[i]].R + 1;
-   };
-   order_grid(c->grid_list, c->grid_n_dual, c->grid_rec_off);
-   order_grid(c->sgrid_list, c->sgrid_n_dual, c->sgrid_rec_off);
+      g.n_dual = g.n_tma = 0;
+      for (int32_t l : g.list) {
+         g.n_dual += grid_kernel[l] == DUAL;
+         g.n_tma += grid_kernel[l] == TMA;
+      }
+      g.rec_off.assign(g.n_dual + 1, 0);
+      for (size_t i = 0; i < g.n_dual; ++i) g.rec_off[i + 1] = g.rec_off[i] + c->meta[g.list[i]].R + 1;
+   }
    for (auto& lc : tmp) {
       std::sort(lc.loci.begin(), lc.loci.end(), by_size);
       if (cluster_stream_groups(lc.max_iso, SMEM_CAP, lc.lpr, 1, 0) <= 0)
@@ -499,16 +460,16 @@ int plan(sbq_ctx* c) {
    c->h_lists.clear();
    c->warp_list_off = 0;
    if (!c->h_lists.append(c->warp_list.data(), c->warp_list.size())) return fail(c, SBQ_ERR_NOMEM, "list staging");
-   c->grid_list_off = c->h_lists.n;
-   if (!c->h_lists.append(c->grid_list.data(), c->grid_list.size())) return fail(c, SBQ_ERR_NOMEM, "list staging");
-   c->sgrid_list_off = c->h_lists.n;
-   if (!c->h_lists.append(c->sgrid_list.data(), c->sgrid_list.size())) return fail(c, SBQ_ERR_NOMEM, "list staging");
+   for (auto& g : c->grid) {
+      g.list_off = c->h_lists.n;
+      if (!c->h_lists.append(g.list.data(), g.list.size())) return fail(c, SBQ_ERR_NOMEM, "list staging");
+   }
    for (auto& lc : c->classes) {
       lc.list_off = c->h_lists.n;
       if (!c->h_lists.append(lc.loci.data(), lc.loci.size())) return fail(c, SBQ_ERR_NOMEM, "list staging");
    }
    c->stats.loci_warp = (int64_t)c->warp_list.size();
-   c->stats.loci_grid = (int64_t)(c->grid_list.size() + c->sgrid_list.size());
+   c->stats.loci_grid = (int64_t)(c->grid[0].list.size() + c->grid[1].list.size());
    c->stats.loci_cta = c->n_loci - c->stats.loci_warp - c->stats.loci_grid;
    return SBQ_SUCCESS;
 }
@@ -583,6 +544,34 @@ int launch_cluster_class_nt(sbq_ctx* c, const LaunchClass& lc, cudaStream_t st) 
    const int32_t* list = c->d_lists_p + lc.list_off;
    CU(cudaLaunchKernelEx(&cfg, kernel, c->dp, list, (int)lc.loci.size(), (unsigned)lc.smem));
    return SBQ_SUCCESS;
+}
+
+// The kernels of one giant-tier class on its stream, each on its part of the list (two-slot, TMA ring, register-staged); the
+// one-off layout passes run on the first solve of an upload. Returns 0 or the launchers' negative code.
+int launch_grid_class(sbq_ctx* c, GridClass& g, int& n_launch) {
+   cudaDeviceProp prop = c->prop;
+   prop.multiProcessorCount = g.n_cta;   // the launchers size their grids by it
+   const int32_t* d_list = c->d_lists_p + g.list_off;
+   const int n_dual = (int)g.n_dual, n_tma = (int)g.n_tma, n_reg = (int)(g.list.size() - g.n_dual - g.n_tma);
+   std::vector<int> h_iso(g.list.size());
+   for (size_t i = 0; i < g.list.size(); ++i) h_iso[i] = c->meta[g.list[i]].T;
+   g.variant = n_dual ? 3 : n_tma ? 2 : 1;
+   int rc = 0, nl = 0;
+   if (n_dual) {
+      GridDualBufs bf{&g.scratch.p, &g.scratch.cap, &c->d_col16.p, &c->d_col16.cap, &g.rowrec.p, &g.rowrec.cap, &g.pk.p, &g.pk.cap};
+      rc = grid_dual_launch(c->dp, c->nnz, d_list, n_dual, h_iso.data(), g.rec_off.data(), prop, bf, c->col16_ready, g.st, &nl);
+      n_launch += nl;
+   }
+   if (rc == 0 && n_tma) {
+      rc = grid_tma_launch(c->dp, c->nnz, d_list + n_dual, n_tma, h_iso.data() + n_dual, prop, &g.scratch.p, &g.scratch.cap, &c->d_col16.p, &c->d_col16.cap,
+                           c->col16_ready, g.st, &nl);
+      n_launch += nl;
+   }
+   if (rc == 0 && n_reg) {
+      rc = grid_tier_launch(c->dp, d_list + n_dual + n_tma, n_reg, prop, &g.scratch.p, &g.scratch.cap, g.st, &nl);
+      n_launch += nl;
+   }
+   return rc;
 }
 
 // Snapshot of the staging sizes, restored when a submit fails half-way (a failed call leaves the queue unchanged).
@@ -728,9 +717,12 @@ int sbq_create(const sbq_config* cfg, sbq_ctx** out) {
       if (cudaEventCreateWithFlags(&e, cudaEventDisableTiming) != cudaSuccess) return bail(SBQ_ERR_CUDA);
    for (auto& t : c->lt)
       if (cudaEventCreate(&t.e0) != cudaSuccess || cudaEventCreate(&t.e1) != cudaSuccess) return bail(SBQ_ERR_CUDA);
-   if (cudaStreamCreateWithFlags(&c->sgrid_st, cudaStreamNonBlocking) != cudaSuccess) return bail(SBQ_ERR_CUDA);
-   if (cudaEventCreateWithFlags(&c->ev_sgrid_join, cudaEventDisableTiming) != cudaSuccess) return bail(SBQ_ERR_CUDA);
-   if (cudaEventCreate(&c->lt_sgrid.e0) != cudaSuccess || cudaEventCreate(&c->lt_sgrid.e1) != cudaSuccess) return bail(SBQ_ERR_CUDA);
+   c->grid[0].st = c->stream;
+   c->grid[0].n_cta = c->prop.multiProcessorCount;
+   if (cudaStreamCreateWithFlags(&c->grid[1].st, cudaStreamNonBlocking) != cudaSuccess) return bail(SBQ_ERR_CUDA);
+   c->grid[1].n_cta = std::min(SGRID_CTAS, c->prop.multiProcessorCount);
+   for (auto& g : c->grid)
+      if (cudaEventCreate(&g.lt.e0) != cudaSuccess || cudaEventCreate(&g.lt.e1) != cudaSuccess) return bail(SBQ_ERR_CUDA);
    if (cfg->n_gpus > 1) {
       const int rc = multi_create(c, ndev);
       if (rc) {
@@ -753,8 +745,13 @@ void sbq_destroy(sbq_ctx* c) {
    c->h_lists.release();
    c->r_theta.release(); c->r_fpkm.release(); c->r_frac.release(); c->r_tpm.release();
    c->r_locus_fpkm.release(); c->r_keep.release(); c->r_iters.release(); c->r_status.release(); c->r_frags.release(); c->d_frags.release();
-   c->d_in.release(); c->d_out.release(); c->d_lists.release(); c->d_grid_scratch.release(); c->d_col16.release(); c->d_rowrec.release(); c->d_csc.release(); c->d_synth.release(); c->d_pk.release(); c->d_raw.release(); c->d_raw2.release(); c->d_bias.release();
-   c->d_sgrid_scratch.release(); c->d_srowrec.release(); c->d_spk.release();
+   c->d_in.release(); c->d_out.release(); c->d_lists.release(); c->d_col16.release(); c->d_csc.release(); c->d_synth.release(); c->d_raw.release(); c->d_raw2.release(); c->d_bias.release();
+   for (auto& g : c->grid) {
+      g.scratch.release(); g.rowrec.release(); g.pk.release();
+      if (g.lt.e0) cudaEventDestroy(g.lt.e0);
+      if (g.lt.e1) cudaEventDestroy(g.lt.e1);
+   }
+   if (c->grid[1].st) cudaStreamSynchronize(c->grid[1].st), cudaStreamDestroy(c->grid[1].st);   // grid[0] runs on c->stream
    c->h_cov.release(); c->r_beta.release(); c->r_outer.release();
    c->h_wseg.release(); c->h_wn.release(); c->h_wmask.release(); c->h_wpool.release(); c->h_wlen.release(); c->h_wpool_off.release(); c->d_weights.release();
    for (auto& e : c->ev) if (e) cudaEventDestroy(e);
@@ -762,10 +759,6 @@ void sbq_destroy(sbq_ctx* c) {
    for (auto& e : c->ev_join) if (e) cudaEventDestroy(e);
    for (auto& t : c->lt) { if (t.e0) cudaEventDestroy(t.e0); if (t.e1) cudaEventDestroy(t.e1); }
    for (auto& s : c->side) if (s) cudaStreamDestroy(s);
-   if (c->lt_sgrid.e0) cudaEventDestroy(c->lt_sgrid.e0);
-   if (c->lt_sgrid.e1) cudaEventDestroy(c->lt_sgrid.e1);
-   if (c->ev_sgrid_join) cudaEventDestroy(c->ev_sgrid_join);
-   if (c->sgrid_st) cudaStreamSynchronize(c->sgrid_st), cudaStreamDestroy(c->sgrid_st);
    if (c->ev_grid_ready) cudaEventDestroy(c->ev_grid_ready);
    for (auto& e : c->ev_class_ready) if (e) cudaEventDestroy(e);
    if (c->copy_st) cudaStreamDestroy(c->copy_st);
@@ -955,11 +948,12 @@ static int upload_begin(sbq_ctx* c) {
    };
    for (auto& r : c->class_ready) r = false;
    c->grid_ready = false;
-   if (!(c->grid_list.empty() && c->sgrid_list.empty()) && c->grid_list.size() + c->sgrid_list.size() <= 16) {
-      int rc = copy_loci(c->grid_list);
-      if (rc) return rc;
-      rc = copy_loci(c->sgrid_list);
-      if (rc) return rc;
+   const size_t n_giant = c->grid[0].list.size() + c->grid[1].list.size();
+   if (n_giant > 0 && n_giant <= 16) {
+      for (auto& g : c->grid) {
+         const int rc = copy_loci(g.list);
+         if (rc) return rc;
+      }
       CU(cudaEventRecord(c->ev_grid_ready, st));
       c->grid_ready = true;
    }
@@ -1204,51 +1198,10 @@ int sbq_solve(sbq_ctx* c, int64_t total_mapped_reads) {
    }
    CU(cudaEventRecord(c->ev[2], st));
    CU(cudaEventRecord(c->ev_fork, st));
-   int used_side = 0;
-   // grid tier on the main stream first (it owns the whole GPU while it runs)
    c->stats.grid_em_ms = 0;
    for (auto& t : c->lt) t.used = false;
    const bool pending = c->upload_pending;   // asynchronous upload in flight: every launch waits for the copies it needs only
-   // one class of grid-tier loci (full grid on the main stream / sub-grid on its own stream): two-slot kernel for the loci that
-   // qualify, TMA ring or register-staged kernel for the rest; the one-off layout passes run on the first solve of an upload
-   auto launch_grid_part = [&](const std::vector<int32_t>& list, size_t list_off, size_t n_dual_, const std::vector<int64_t>& rec_off, int max_iso_rest,
-                               bool tma_ok, const cudaDeviceProp& prop_, DevBuf& scratch, DevBuf& rowrec, DevBuf& pkbuf, cudaStream_t gs_, int& variant,
-                               int& n_launch) -> int {
-      int rc = 0;
-      variant = 0;
-      const int32_t* d_grid = c->d_lists_p + list_off;
-      const int n_dual = (int)n_dual_, n_rest = (int)list.size() - n_dual;
-      if (n_dual) {
-         GridDualBufs bf{&scratch.p, &scratch.cap, &c->d_col16.p, &c->d_col16.cap, &rowrec.p, &rowrec.cap, &pkbuf.p, &pkbuf.cap};
-         int nl = 0;
-         std::vector<int> h_iso((size_t)n_dual);
-         for (int i = 0; i < n_dual; ++i) h_iso[i] = c->meta[list[i]].T;
-         rc = grid_dual_launch(c->dp, c->nnz, d_grid, n_dual, h_iso.data(), rec_off.data(), prop_, bf, c->col16_ready, gs_, &nl);
-         n_launch += nl;
-         variant = 3;
-      }
-      if (rc == 0 && n_rest) {   // loci the two-slot layout does not take (wide, or rows too long on average)
-         int nl = 0;
-         if (tma_ok && !getenv("SBQ_GRID_NO_TMA")) {
-            if (!variant) variant = 2;
-            rc = grid_tma_launch(c->dp, c->nnz, d_grid + n_dual, n_rest, max_iso_rest, prop_, &scratch.p, &scratch.cap,
-                                 &c->d_col16.p, &c->d_col16.cap, c->col16_ready, gs_, &nl);
-         } else {
-            if (!variant) variant = 1;
-            rc = grid_tier_launch(c->dp, d_grid + n_dual, n_rest, prop_, &scratch.p, &scratch.cap, gs_, &nl);
-         }
-         n_launch += nl;
-      }
-      return rc;
-   };
-   auto grid_failed = [&](int rc) -> int {
-      // the one-off layout passes permute alpha inside each giant row IN PLACE: after a failure the resident copy can no
-      // longer be trusted to match the column arrays, so the batch has to be uploaded again
-      c->resident = false;
-      c->col16_ready = false;
-      return fail(c, rc < -6 ? SBQ_ERR_CUDA : rc, "grid tier launch failed: %s", cudaGetErrorString(cudaGetLastError()));
-   };
-   if (!(c->grid_list.empty() && c->sgrid_list.empty())) {
+   if (!(c->grid[0].list.empty() && c->grid[1].list.empty())) {
       // the 16-bit slot array is shared by both classes (indexed by non-zero): sized here, so that neither launch re-allocates it
       // under the other
       const size_t need16 = (size_t)c->nnz * 2 + 256;
@@ -1257,92 +1210,40 @@ int sbq_solve(sbq_ctx* c, int64_t total_mapped_reads) {
          c->col16_ready = false;
       }
    }
-   if (!c->grid_list.empty()) {
-      if (pending) CU(cudaStreamWaitEvent(st, c->grid_ready ? c->ev_grid_ready : c->ev[1], 0));
-      CU(cudaEventRecord(c->ev[6], st));
+   // grid tier first: the full grid on the main stream (it owns the whole GPU while it runs), then the sub-grid on its own stream,
+   // launched before the cluster classes so that it is resident when they fill the other SMs
+   for (int k = 0; k < 2; ++k) {
+      GridClass& g = c->grid[k];
+      g.lt.used = false;
+      if (g.list.empty()) continue;
+      CU(cudaStreamWaitEvent(g.st, c->ev_fork, 0));
+      if (k == 1 && c->grid[0].lt.used) CU(cudaStreamWaitEvent(g.st, c->grid[0].lt.e1, 0));   // the full-grid class owns the GPU first
+      if (pending) CU(cudaStreamWaitEvent(g.st, c->grid_ready ? c->ev_grid_ready : c->ev[1], 0));
+      CU(cudaEventRecord(g.lt.e0, g.st));
       int n_launch = 0;
-      const int rc = launch_grid_part(c->grid_list, c->grid_list_off, c->grid_n_dual, c->grid_rec_off, c->grid_max_iso, c->grid_tma_ok, c->prop,
-                                      c->d_grid_scratch, c->d_rowrec, c->d_pk, st, c->grid_variant, n_launch);
-      if (rc != 0) return grid_failed(rc);
-      launches += n_launch;
-      CU(cudaEventRecord(c->ev[7], st));
-   }
-   c->lt_sgrid.used = false;
-   if (!c->sgrid_list.empty()) {
-      // small giants: same kernels on SGRID_CTAS CTAs (the launchers size their grids by prop.multiProcessorCount), own stream,
-      // launched before the cluster classes so that the sub-grid is resident when they fill the other SMs
-      cudaDeviceProp prop_sg = c->prop;
-      prop_sg.multiProcessorCount = std::min(SGRID_CTAS, c->prop.multiProcessorCount);
-      cudaStream_t gs_ = c->sgrid_st;
-      CU(cudaStreamWaitEvent(gs_, c->ev_fork, 0));
-      if (pending) CU(cudaStreamWaitEvent(gs_, c->grid_ready ? c->ev_grid_ready : c->ev[1], 0));
-      if (!c->grid_list.empty()) {                      // the full-grid class owns the GPU first
-         CU(cudaStreamWaitEvent(gs_, c->ev[7], 0));
+      const int rc = launch_grid_class(c, g, n_launch);
+      if (rc != 0) {
+         // the one-off layout passes permute alpha inside each giant row IN PLACE: after a failure the resident copy can no
+         // longer be trusted to match the column arrays, so the batch has to be uploaded again
+         c->resident = false;
+         c->col16_ready = false;
+         return fail(c, rc < -6 ? SBQ_ERR_CUDA : rc, "grid tier launch failed: %s", cudaGetErrorString(cudaGetLastError()));
       }
-      CU(cudaEventRecord(c->lt_sgrid.e0, gs_));
-      int n_launch = 0;
-      const int rc = launch_grid_part(c->sgrid_list, c->sgrid_list_off, c->sgrid_n_dual, c->sgrid_rec_off, c->sgrid_max_iso, c->sgrid_tma_ok, prop_sg,
-                                      c->d_sgrid_scratch, c->d_srowrec, c->d_spk, gs_, c->sgrid_variant, n_launch);
-      if (rc != 0) return grid_failed(rc);
       launches += n_launch;
-      CU(cudaEventRecord(c->lt_sgrid.e1, gs_));
-      CU(cudaEventRecord(c->ev_sgrid_join, gs_));
-      c->lt_sgrid.used = true;
+      CU(cudaEventRecord(g.lt.e1, g.st));
+      g.lt.used = true;
    }
-   if (!(c->grid_list.empty() && c->sgrid_list.empty())) c->col16_ready = true;
-   const bool serialize = getenv("SBQ_SERIALIZE") != nullptr;   // debugging / profiling: one stream, isolated kernel times
-   // Launch ORDER (class i keeps stream / timer / ready-event i whatever its position). The work distributor serves
+   if (!(c->grid[0].list.empty() && c->grid[1].list.empty())) c->col16_ready = true;
+   // Launch order: the cluster classes (biggest clusters first, see plan()), then the warp tier. The work distributor serves
    // kernels roughly in launch order, 16- and 8-CTA clusters strand a few SMs per GPC that only single CTAs can use, and the
    // many small loci have critical paths of their own (~1 ms): see DESIGN.md section 5 for the measured timelines.
-   static const int order_mode = getenv("SBQ_ORDER") ? atoi(getenv("SBQ_ORDER")) : SBQ_DEFAULT_ORDER;
    const int ncls = (int)c->classes.size();
-   std::vector<int> ord;
-   int warp_pos = ncls;   // position in ord before which the warp tier is launched
-   {
-      std::vector<int> big, small, rest;
-      for (int i = 0; i < ncls; ++i) {
-         const LaunchClass& lc = c->classes[i];
-         if (lc.lpr < CL_NT) small.push_back(i);
-         else if (lc.cs >= (order_mode == 3 ? 16 : 8)) big.push_back(i);
-         else rest.push_back(i);
-      }
-      if (order_mode == 1) { ord = small; ord.insert(ord.end(), big.begin(), big.end()); ord.insert(ord.end(), rest.begin(), rest.end()); warp_pos = 0; }
-      else if (order_mode == 2 || order_mode == 3) { ord = big; warp_pos = (int)ord.size(); ord.insert(ord.end(), small.begin(), small.end()); ord.insert(ord.end(), rest.begin(), rest.end()); }
-      else { for (int i = 0; i < ncls; ++i) ord.push_back(i); }
-   }
-   auto launch_warp = [&]() -> int {
-      if (c->warp_list.empty()) return SBQ_SUCCESS;
-      const size_t smem = warp_tier_smem_bytes(c->warp_max_iso);
-      CU(cudaFuncSetAttribute(em_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      const int n = (int)c->warp_list.size();
-      int per_sm = 1;
-      CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, em_warp_kernel, WT_WARPS * 32, smem));
-      int grid = std::max(1, std::min((n + WT_WARPS - 1) / WT_WARPS, per_sm * c->prop.multiProcessorCount));
-      static const int warp_cta_cap = getenv("SBQ_WARP_CTAS") ? atoi(getenv("SBQ_WARP_CTAS")) : SBQ_DEFAULT_WARP_CTAS;   // persistent warps: the grid only sets the parallelism
-      if (warp_cta_cap > 0) grid = std::min(grid, warp_cta_cap);
-      int* queue = (int*)((char*)c->d_fpkm_sum + 64);
-      if (pending) CU(cudaStreamWaitEvent(st, c->ev[1], 0));   // many small loci all over the batch: they need everything
-      CU(cudaMemsetAsync(queue, 0, sizeof(int), st));
-      CU(cudaEventRecord(c->lt[0].e0, st));
-      em_warp_kernel<<<grid, WT_WARPS * 32, smem, st>>>(c->dp, c->d_lists_p + c->warp_list_off, n, c->warp_max_iso, queue);
-      CU(cudaGetLastError());
-      CU(cudaEventRecord(c->lt[0].e1, st));
-      c->lt[0].used = true;
-      ++launches;
-      return SBQ_SUCCESS;
-   };
-   for (int pos = 0; pos <= ncls; ++pos) {
-      if (pos == warp_pos) {
-         const int rcw = launch_warp();
-         if (rcw) return rcw;
-      }
-      if (pos == ncls) break;
-      const int i = ord[pos];
+   for (int i = 0; i < ncls; ++i) {
       const LaunchClass& lc = c->classes[i];
-      cudaStream_t ss = serialize ? st : c->side[i % N_SIDE_STREAMS];
-      if (!serialize && i < N_SIDE_STREAMS) CU(cudaStreamWaitEvent(ss, c->ev_fork, 0));
+      cudaStream_t ss = c->side[i % N_SIDE_STREAMS];
+      if (i < N_SIDE_STREAMS) CU(cudaStreamWaitEvent(ss, c->ev_fork, 0));
       if (pending) CU(cudaStreamWaitEvent(ss, (i < N_SIDE_STREAMS && c->class_ready[i]) ? c->ev_class_ready[i] : c->ev[1], 0));
-      LaunchTimer& t = c->lt[2 + i % N_SIDE_STREAMS];
+      LaunchTimer& t = c->lt[1 + i % N_SIDE_STREAMS];
       CU(cudaEventRecord(t.e0, ss));
       // register caps (launch bounds) follow the CTAs-per-SM targets of the buckets
       int rc = lc.lpr == 64 ? launch_cluster_class_nt<64, 0, 8>(c, lc, ss) : lc.lpr == 128 ? launch_cluster_class_nt<128, 0, 4>(c, lc, ss) :
@@ -1352,12 +1253,28 @@ int sbq_solve(sbq_ctx* c, int64_t total_mapped_reads) {
       t.used = true;
       ++launches;
    }
-   used_side = ncls;
-   for (int i = 0; i < std::min(used_side, N_SIDE_STREAMS) && !serialize; ++i) {
+   if (!c->warp_list.empty()) {
+      const size_t smem = warp_tier_smem_bytes(c->warp_max_iso);
+      CU(cudaFuncSetAttribute(em_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      const int n = (int)c->warp_list.size();
+      int per_sm = 1;
+      CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, em_warp_kernel, WT_WARPS * 32, smem));
+      const int grid = std::max(1, std::min((n + WT_WARPS - 1) / WT_WARPS, per_sm * c->prop.multiProcessorCount));   // persistent warps: the grid only sets the parallelism
+      int* queue = (int*)((char*)c->d_fpkm_sum + 64);
+      if (pending) CU(cudaStreamWaitEvent(st, c->ev[1], 0));   // many small loci all over the batch: they need everything
+      CU(cudaMemsetAsync(queue, 0, sizeof(int), st));
+      CU(cudaEventRecord(c->lt[0].e0, st));
+      em_warp_kernel<<<grid, WT_WARPS * 32, smem, st>>>(c->dp, c->d_lists_p + c->warp_list_off, n, c->warp_max_iso, queue);
+      CU(cudaGetLastError());
+      CU(cudaEventRecord(c->lt[0].e1, st));
+      c->lt[0].used = true;
+      ++launches;
+   }
+   for (int i = 0; i < std::min(ncls, N_SIDE_STREAMS); ++i) {
       CU(cudaEventRecord(c->ev_join[i], c->side[i]));
       CU(cudaStreamWaitEvent(st, c->ev_join[i], 0));
    }
-   if (c->lt_sgrid.used) CU(cudaStreamWaitEvent(st, c->ev_sgrid_join, 0));
+   if (c->grid[1].lt.used) CU(cudaStreamWaitEvent(st, c->grid[1].lt.e1, 0));
    CU(cudaEventRecord(c->ev[3], st));
    fpkm_sum_kernel<<<1, 1024, 0, st>>>(dp.locus_fpkm, c->n_loci, c->d_fpkm_sum);
    CU(cudaGetLastError());
@@ -1373,11 +1290,7 @@ int sbq_solve(sbq_ctx* c, int64_t total_mapped_reads) {
    c->stats.solve_ms = ms;
    CU(cudaEventElapsedTime(&ms, c->ev[2], c->ev[3]));
    c->stats.em_ms = ms;
-   if (!c->grid_list.empty()) {
-      CU(cudaEventElapsedTime(&ms, c->ev[6], c->ev[7]));
-      c->stats.grid_em_ms = ms;
-   }
-   // per-launch records: [warp] [grid] [cluster classes...]
+   // per-launch records: [warp] [grid classes...] [cluster classes...]
    c->launch_stats.clear();
    c->locus_launch.assign(c->n_loci, -1);
    auto add_stat = [&](int kind, int cs, int lpr, const std::vector<int32_t>& loci, double ms_, cudaEvent_t e0 = nullptr) {
@@ -1389,14 +1302,16 @@ int sbq_solve(sbq_ctx* c, int64_t total_mapped_reads) {
       c->launch_stats.push_back(ls);
    };
    if (c->lt[0].used) { CU(cudaEventElapsedTime(&ms, c->lt[0].e0, c->lt[0].e1)); add_stat(1, 1, 1, c->warp_list, ms, c->lt[0].e0); }
-   if (!c->grid_list.empty()) { add_stat(3, 0, 32, c->grid_list, c->stats.grid_em_ms, c->ev[6]); c->launch_stats.back().variant = c->grid_variant; }
-   if (c->lt_sgrid.used) {      // sub-grid class: cluster_size field = its CTA count
-      CU(cudaEventElapsedTime(&ms, c->lt_sgrid.e0, c->lt_sgrid.e1));
-      add_stat(3, std::min(SGRID_CTAS, c->prop.multiProcessorCount), 32, c->sgrid_list, ms, c->lt_sgrid.e0);
-      c->launch_stats.back().variant = c->sgrid_variant;
+   for (int k = 0; k < 2; ++k) {
+      const GridClass& g = c->grid[k];
+      if (!g.lt.used) continue;
+      CU(cudaEventElapsedTime(&ms, g.lt.e0, g.lt.e1));
+      if (k == 0) c->stats.grid_em_ms = ms;                        // grid_em_ms: the full grid only
+      add_stat(3, k == 0 ? 0 : g.n_cta, 32, g.list, ms, g.lt.e0);   // cluster_size: 0 for the full grid, the CTA count of the sub-grid
+      c->launch_stats.back().variant = g.variant;
    }
    for (size_t i = 0; i < c->classes.size(); ++i) {
-      LaunchTimer& t = c->lt[2 + i % N_SIDE_STREAMS];
+      LaunchTimer& t = c->lt[1 + i % N_SIDE_STREAMS];
       CU(cudaEventElapsedTime(&ms, t.e0, t.e1));
       add_stat(2, c->classes[i].cs, c->classes[i].lpr, c->classes[i].loci, ms, t.e0);
    }
@@ -1466,7 +1381,7 @@ int sbq_download(sbq_ctx* c) {
              c->r_keep.reserve(ni) && c->r_iters.reserve(nl) && c->r_status.reserve(nl) && c->r_locus_fpkm.reserve(nl);
    if (!ok) return fail(c, SBQ_ERR_NOMEM, "pinned result buffers");
    cudaStream_t st = c->stream;
-   CU(cudaEventRecord(c->ev[8], st));
+   CU(cudaEventRecord(c->ev[7], st));
    CU(cudaMemcpyAsync(c->r_theta.p, c->dp.theta, ni * 8, cudaMemcpyDeviceToHost, st));
    CU(cudaMemcpyAsync(c->r_fpkm.p, c->dp.fpkm, ni * 8, cudaMemcpyDeviceToHost, st));
    CU(cudaMemcpyAsync(c->r_frac.p, c->dp.frac, ni * 8, cudaMemcpyDeviceToHost, st));
@@ -1475,10 +1390,10 @@ int sbq_download(sbq_ctx* c) {
    CU(cudaMemcpyAsync(c->r_iters.p, c->dp.iters, nl * 4, cudaMemcpyDeviceToHost, st));
    CU(cudaMemcpyAsync(c->r_status.p, c->dp.status, nl * 4, cudaMemcpyDeviceToHost, st));
    CU(cudaMemcpyAsync(&c->r_fpkm_sum, c->d_fpkm_sum, 8, cudaMemcpyDeviceToHost, st));
-   CU(cudaEventRecord(c->ev[9], st));
+   CU(cudaEventRecord(c->ev[8], st));
    CU(cudaStreamSynchronize(st));
    float ms = 0;
-   CU(cudaEventElapsedTime(&ms, c->ev[8], c->ev[9]));
+   CU(cudaEventElapsedTime(&ms, c->ev[7], c->ev[8]));
    c->stats.download_ms = ms;
    c->stats.d2h_bytes = (int64_t)ni * 36 + (int64_t)nl * 8 + 8;
 
@@ -1509,7 +1424,7 @@ static void account(sbq_ctx* c) {
    if (!c->stats_stale || !c->downloaded) return;
    const size_t nl = (size_t)c->n_loci;
    std::vector<char> is_grid(nl, 0);
-   for (int32_t l : c->grid_list) is_grid[l] = 1;
+   for (int32_t l : c->grid[0].list) is_grid[l] = 1;   // grid_alg_bytes goes with grid_em_ms: the full grid only
    int64_t it_total = 0, frag_iters = 0, alg = 0, galg = 0;
    for (auto& ls : c->launch_stats) ls.nnz = ls.alg_bytes = ls.frag_iters = ls.max_iters = 0;
    for (size_t l = 0; l < nl && l < c->meta.size(); ++l) {   // shapes captured at upload: the host arrays may be gone by now

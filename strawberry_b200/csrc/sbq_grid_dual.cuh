@@ -895,13 +895,11 @@ em_grid_dual_kernel(DevParams p, const unsigned short* __restrict__ col16, RowRe
 // default wherever the kernel can run: measured on 1 M rows x 48 non-zeros, even its 4-warp configuration (T = 2000: 0.32 of the HBM
 // peak, T = 1400 with 6 warps: 0.43) beats the TMA ring kernel (0.27 / 0.37), which remains for T > G6_MAX_ISO and dense rows
 inline bool grid_dual_supports_iso(int T) { return T <= G6_MAX_ISO && G6Cfg<4>::fits(T, 1); }
-inline bool grid_dual_possible(int T) { return T <= G6_MAX_ISO && G6Cfg<4>::fits(T, 1); }   // SBQ_GRID_DUAL=1 forces the kernel wherever it can run
 
 // warps per CTA for a locus of T isoforms: a function of the LOCUS alone (the launcher groups loci by it), so that neither the
 // speed nor the summation order of a locus depends on which other loci share its batch
 inline int grid_dual_nc(int T) {
-   static const int force_nc = getenv("SBQ_DUAL_NC") ? atoi(getenv("SBQ_DUAL_NC")) : 0;   // tuning: force the number of warps
-#define SBQ_NC6(NC) if (force_nc ? (force_nc == NC && G6Cfg<NC>::fits(T, 1)) : G6Cfg<NC>::fits(T, 1)) return NC;
+#define SBQ_NC6(NC) if (G6Cfg<NC>::fits(T, 1)) return NC;
    // (14 warps fit up to T = 624 but force 128 registers per thread: measured 0.1427 ms per pass against 0.1433 with 12 - not worth a variant)
    SBQ_NC6(12) SBQ_NC6(10) SBQ_NC6(8) SBQ_NC6(6) SBQ_NC6(4)
 #undef SBQ_NC6

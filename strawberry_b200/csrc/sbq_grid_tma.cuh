@@ -8,7 +8,7 @@
 //    CTA are contiguous in CSR, so each slab is one contiguous, 16-byte aligned piece of HBM;
 //  * full/empty mbarriers per stage; consumers wait (try_wait.parity), take two rows of the chunk per warp,
 //    and release the stage. HBM latency is covered by the ring depth instead of by registers;
-//  * columns are pre-narrowed to u16 by cols_to_u16_kernel at upload (10 B of HBM traffic per non-zero and
+//  * columns are pre-narrowed to u16 by grid_prepare_kernel once per upload (10 B of HBM traffic per non-zero and
 //    iteration instead of 12; the algorithmic-byte accounting of SURVEY 8d stays 12).
 // Reductions (warp-private accumulators -> per-CTA partial -> column owners -> theta') are unchanged and
 // deterministic. Chunks whose non-zeros exceed the stage capacity are processed straight from global memory
@@ -24,7 +24,7 @@ constexpr int G4_CHUNK_BYTES = (((G4_MAX_CHUNKS + 1) * 4 + 127) / 128) * 128;
 
 // Geometry of one kernel instantiation: NC consumer warps (one warp-private accumulator row each) and a ring of
 // NS stages. More consumer warps hide more shared-memory / shuffle latency but cost NC * T * 8 B of accumulators,
-// so the launcher picks the largest NC whose shared memory fits for the widest giant locus of the batch.
+// so every locus takes the largest NC whose shared memory fits its own T (grid_tma_nc).
 template <int NC, int NSTAGE>
 struct G4Cfg {
    static constexpr int CONSUMERS = NC;
@@ -48,12 +48,21 @@ struct G4Cfg {
    }
 };
 
-inline bool grid_tma_supports(int T, long long rows, int n_cta) {
-   return G4Cfg<8, 4>::smem_bytes(T) <= 225 * 1024 && T <= 65535 && rows / n_cta + 64 < (long long)G4_MAX_CHUNKS * 16;
+// consumer warps for a locus of T isoforms: the most whose shared memory fits, 0 if none does. A function of the LOCUS alone
+// (the launcher groups loci by it), so that neither the speed nor the summation order of a locus depends on which other loci
+// share its batch
+inline int grid_tma_nc(int T) {
+   const size_t cap = 225 * 1024;
+   if (G4Cfg<24, 3>::smem_bytes(T) <= cap) return 24;
+   if (G4Cfg<20, 3>::smem_bytes(T) <= cap) return 20;
+   if (G4Cfg<16, 4>::smem_bytes(T) <= cap) return 16;
+   if (G4Cfg<12, 4>::smem_bytes(T) <= cap) return 12;
+   if (G4Cfg<8, 4>::smem_bytes(T) <= cap) return 8;
+   return 0;
 }
 
-__global__ void cols_to_u16_kernel(const int32_t* __restrict__ col, unsigned short* __restrict__ out, int64_t n) {
-   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) out[i] = (unsigned short)col[i];
+inline bool grid_tma_supports(int T, long long rows, int n_cta) {
+   return grid_tma_nc(T) > 0 && T <= 65535 && rows / n_cta + 64 < (long long)G4_MAX_CHUNKS * 16;
 }
 
 // One-off prepare pass for giant loci (run once per upload): reorder the non-zeros INSIDE every row (<= 64 entries) so
@@ -524,11 +533,10 @@ em_grid_tma_kernel(DevParams p, const unsigned short* __restrict__ col16, const 
    }
 }
 
-// Host launcher of the TMA path. col16_scratch: device buffer for the u16 columns of the whole batch (grown here).
+// One cooperative launch of the TMA path for loci of up to max_iso isoforms (the u16 columns are in place).
 template <typename C>
-inline int grid_tma_launch_cfg(const DevParams& dp, int64_t nnz_total, const int32_t* d_list, int n_list, int max_iso, const cudaDeviceProp& prop,
-                               void** scratch, size_t* scratch_cap, void** col16_scratch, size_t* col16_cap, bool cols_ready, cudaStream_t st,
-                               int* n_launch) {
+inline int grid_tma_launch_cfg(const DevParams& dp, const int32_t* d_list, int n_list, int max_iso, const cudaDeviceProp& prop, void** scratch,
+                               size_t* scratch_cap, const unsigned short* c16, cudaStream_t st, int* n_launch) {
    const size_t smem = C::smem_bytes(max_iso);
    auto kernel = em_grid_tma_kernel<C>;
    if (cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return -3;
@@ -544,20 +552,6 @@ inline int grid_tma_launch_cfg(const DevParams& dp, int64_t nnz_total, const int
       if (cudaMalloc(scratch, need) != cudaSuccess) return -4;
       *scratch_cap = need;
    }
-   const size_t need16 = (size_t)nnz_total * 2 + 256;
-   if (need16 > *col16_cap) {
-      if (*col16_scratch) cudaFree(*col16_scratch);
-      *col16_scratch = nullptr;
-      *col16_cap = 0;
-      if (cudaMalloc(col16_scratch, need16) != cudaSuccess) return -4;
-      *col16_cap = need16;
-      cols_ready = false;
-   }
-   if (!cols_ready) {
-      if (getenv("SBQ_GRID_NO_REORDER")) cols_to_u16_kernel<<<prop.multiProcessorCount * 8, 256, 0, st>>>(dp.col, (unsigned short*)*col16_scratch, nnz_total);
-      else grid_prepare_kernel<<<prop.multiProcessorCount * 8, 256, 0, st>>>(dp, d_list, n_list, (unsigned short*)*col16_scratch);
-      ++*n_launch;
-   }
    GridScratch gs;
    char* q = (char*)*scratch;
    gs.partial = (double*)q; q += (size_t)nb * tstride * sizeof(double);
@@ -568,30 +562,51 @@ inline int grid_tma_launch_cfg(const DevParams& dp, int64_t nnz_total, const int
    gs.tstride = tstride;
    if (cudaMemsetAsync(gs.ctr, 0, (size_t)n_list * (2 * sizeof(long long) + sizeof(int)), st) != cudaSuccess) return -3;
    DevParams dpc = dp;
-   const unsigned short* c16 = (const unsigned short*)*col16_scratch;
    void* args[] = {(void*)&dpc, (void*)&c16, (void*)&d_list, (void*)&n_list, (void*)&gs, (void*)&cur_glob};
    if (cudaLaunchCooperativeKernel((void*)kernel, dim3(nb), dim3(C::NT), args, smem, st) != cudaSuccess) return -3;
    ++*n_launch;
    return 0;
 }
 
-inline int grid_tma_launch(const DevParams& dp, int64_t nnz_total, const int32_t* d_list, int n_list, int max_iso, const cudaDeviceProp& prop,
+// Host launcher of the TMA path. h_iso: T of every list entry (host); the planner sorts the list by grid_tma_nc. col16_scratch:
+// device buffer for the u16 columns of the whole batch (grown here). cols_ready: the prepare pass of this upload already ran.
+inline int grid_tma_launch(const DevParams& dp, int64_t nnz_total, const int32_t* d_list, int n_list, const int* h_iso, const cudaDeviceProp& prop,
                            void** scratch, size_t* scratch_cap, void** col16_scratch, size_t* col16_cap, bool cols_ready, cudaStream_t st,
                            int* n_launch) {
    *n_launch = 0;
    if (n_list == 0) return 0;
-   const size_t cap = 225 * 1024;
-#define SBQ_TRY(NC, NSTAGE)                                                                                                              \
-   if (G4Cfg<NC, NSTAGE>::smem_bytes(max_iso) <= cap)                                                                                    \
-      return grid_tma_launch_cfg<G4Cfg<NC, NSTAGE>>(dp, nnz_total, d_list, n_list, max_iso, prop, scratch, scratch_cap, col16_scratch,   \
-                                                    col16_cap, cols_ready, st, n_launch);
-   SBQ_TRY(24, 3)
-   SBQ_TRY(20, 3)
-   SBQ_TRY(16, 4)
-   SBQ_TRY(12, 4)
-   SBQ_TRY(8, 4)
-#undef SBQ_TRY
-   return -6;
+   const size_t need16 = (size_t)nnz_total * 2 + 256;
+   if (need16 > *col16_cap) {
+      if (*col16_scratch) cudaFree(*col16_scratch);
+      *col16_scratch = nullptr;
+      *col16_cap = 0;
+      if (cudaMalloc(col16_scratch, need16) != cudaSuccess) return -4;
+      *col16_cap = need16;
+      cols_ready = false;
+   }
+   const unsigned short* c16 = (const unsigned short*)*col16_scratch;
+   if (!cols_ready) {
+      grid_prepare_kernel<<<prop.multiProcessorCount * 8, 256, 0, st>>>(dp, d_list, n_list, (unsigned short*)c16);
+      ++*n_launch;
+   }
+   // one cooperative launch per run of loci with the same warp count
+   for (int i0 = 0; i0 < n_list;) {
+      const int nc = grid_tma_nc(h_iso[i0]);
+      int i1 = i0, mx = 1;
+      while (i1 < n_list && grid_tma_nc(h_iso[i1]) == nc) { mx = mx > h_iso[i1] ? mx : h_iso[i1]; ++i1; }
+      int rc = -6;
+      switch (nc) {
+         case 24: rc = grid_tma_launch_cfg<G4Cfg<24, 3>>(dp, d_list + i0, i1 - i0, mx, prop, scratch, scratch_cap, c16, st, n_launch); break;
+         case 20: rc = grid_tma_launch_cfg<G4Cfg<20, 3>>(dp, d_list + i0, i1 - i0, mx, prop, scratch, scratch_cap, c16, st, n_launch); break;
+         case 16: rc = grid_tma_launch_cfg<G4Cfg<16, 4>>(dp, d_list + i0, i1 - i0, mx, prop, scratch, scratch_cap, c16, st, n_launch); break;
+         case 12: rc = grid_tma_launch_cfg<G4Cfg<12, 4>>(dp, d_list + i0, i1 - i0, mx, prop, scratch, scratch_cap, c16, st, n_launch); break;
+         case 8: rc = grid_tma_launch_cfg<G4Cfg<8, 4>>(dp, d_list + i0, i1 - i0, mx, prop, scratch, scratch_cap, c16, st, n_launch); break;
+         default: break;
+      }
+      if (rc) return rc;
+      i0 = i1;
+   }
+   return 0;
 }
 
 }  // namespace sbq

@@ -268,7 +268,6 @@ def test_golden_vectors_through_the_two_slot_grid_kernel(q, monkeypatch):
     """The reference's golden vectors (all four locus outcomes) through the grid tier: 135 of the 136 loci qualify for the
     two-slot kernel, the one whose rows average more than 56 non-zeros runs on the TMA ring kernel in the same solve."""
     b, theta_ref, rc_ref, iters, status = load_golden()
-    monkeypatch.setenv("SBQ_GRID_DUAL", "1")
     monkeypatch.setenv("SBQ_DUAL_VERIFY", "1")
     res = run_gpu(q, b, 3, 0)
     assert res["stats"]["loci_grid"] == len(status)
@@ -308,7 +307,6 @@ def test_grid_tier_two_slot_layout_edge_shapes(q, oracle_mod, monkeypatch):
     giant-shaped locus; bit-reproducible when the resident batch is solved again."""
     b = synth.concat([_two_slot_edge_locus(40001, 733, 11), synth.giant(n_loci=1, rows_per_locus=4503, seed=4), _two_slot_edge_locus(3001, 90, 12)])   # 40001 rows: > 12 chunks per CTA, the stage refill path runs
     ora = oracle_mod.quantify_batch(b, b["total_mapped_reads"], n_threads=2)
-    monkeypatch.setenv("SBQ_GRID_DUAL", "1")   # read by the planner when the batch is submitted
     monkeypatch.setenv("SBQ_DUAL_VERIFY", "1")   # libsbq checks the prepared layout: distinct banks per step, disjoint slots of rows r, r + 4
     res = run_gpu(q, b, 3, 0)
     assert res["stats"]["loci_grid"] == 3
@@ -368,7 +366,6 @@ def test_grid_tier_two_slot_rows_with_unsorted_columns(q, oracle_mod, monkeypatc
         b["col"][k0:k1] = b["col"][k0:k1][perm]
         b["alpha"][k0:k1] = b["alpha"][k0:k1][perm]
     ora = oracle_mod.quantify_batch(b, b["total_mapped_reads"])
-    monkeypatch.setenv("SBQ_GRID_DUAL", "1")
     monkeypatch.setenv("SBQ_DUAL_VERIFY", "1")
     q.clear()                                        # (sbq_validate rejects such input; callers may skip validation)
     q.set_plan(3, 0)
@@ -410,6 +407,29 @@ def _shape_locus(rng, T, R, k_mean, empty_rows=0, dropped_rows=0):
                 col=np.concatenate([c for c, _ in rows]).astype(np.int32), alpha=np.concatenate([a for _, a in rows]),
                 count=rng.integers(1, 100, n).astype(np.int32), iso_len=rng.integers(300, 5000, T).astype(np.int32),
                 total_mapped_reads=1_000_000)
+
+
+def test_giant_loci_are_solved_the_same_whatever_shares_their_batch(q, oracle_mod):
+    """The grid kernel and its warp count are chosen from the locus' own shape: four giant-tier loci that take four different
+    launches - TMA ring with 24 warps, TMA ring with 12 warps, register-staged, two-slot - solved in one batch give the same bits as
+    each solved alone."""
+    rng = np.random.default_rng(29)
+    loci = [_shape_locus(rng, 300, 3000, 80),     # dense rows (> 56 non-zeros on average): TMA ring, 24 warps
+            _shape_locus(rng, 1200, 3000, 80),    # dense rows: TMA ring, 12 warps
+            _shape_locus(rng, 2700, 3000, 30),    # too wide for the two-slot and TMA ring kernels: register-staged
+            _shape_locus(rng, 600, 3000, 30)]     # two-slot kernel
+    b = synth.concat(loci)
+    b["total_mapped_reads"] = 1_000_000
+    ora = oracle_mod.quantify_batch(b, b["total_mapped_reads"], n_threads=2)
+    res = run_gpu(q, b, 3, 0)
+    assert [r["kernel"] for r in q.launch_stats() if r["n_loci"]] == ["em_grid_dual_kernel"]
+    assert_matches_oracle(res, ora, b, "mixed giant-tier batch")
+    iso = b["loc_iso_off"]
+    for l, one in enumerate(loci):
+        alone = run_gpu(q, one, 3, 0)
+        sl = slice(iso[l], iso[l + 1])
+        assert np.array_equal(res["theta"][sl].view(np.uint64), alone["theta"].view(np.uint64)), l
+        assert res["iters"][l] == alone["iters"][0] and res["status"][l] == alone["status"][0], l
 
 
 @pytest.mark.parametrize("cluster", [1, 2, 16])

@@ -8,7 +8,6 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-os.environ.setdefault("SBQ_GRID_DUAL", "1")
 os.environ.setdefault("SBQ_DUAL_VERIFY", "1")
 import oracle  # noqa: E402
 from strawberry_b200 import api, synth  # noqa: E402

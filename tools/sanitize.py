@@ -43,15 +43,20 @@ q.set_covariates(synth.covariates(bb, seed=3))
 q.run(bb["total_mapped_reads"])
 print("bias ok", np.isfinite(q.results()["theta"]).all(), q.stats()["kernel_launches"])
 q.close()
-os.environ["SBQ_GRID_NO_DUAL"] = "1"                      # the TMA ring kernel
+rng = np.random.default_rng(8)                            # forced grid tier, rows of 60 - 99 non-zeros (the two-slot layout takes <= 56 on average): TMA ring kernel
+T, R = 200, 600
+k = rng.integers(60, 100, R)
+rp = np.concatenate([[0], np.cumsum(k)]).astype(np.int64)
+bd = dict(loc_row_off=np.array([0, R], np.int64), loc_iso_off=np.array([0, T], np.int64), row_ptr=rp,
+          col=np.concatenate([np.sort(rng.choice(T, kk, replace=False)) for kk in k]).astype(np.int32), alpha=10.0 ** rng.uniform(-4, -1.5, int(rp[-1])),
+          count=rng.integers(1, 100, R).astype(np.int32), iso_len=rng.integers(300, 5000, T).astype(np.int32), total_mapped_reads=1_000_000)
 q = api.Quantifier(max_iter=4)
 q.set_plan(3, 0)
-q.submit_flat(b)
-q.run(b["total_mapped_reads"])
-print("tma ring ok", np.isfinite(q.results()["theta"]).all())
+q.submit_flat(bd)
+q.run(bd["total_mapped_reads"])
+print("tma ring ok", np.isfinite(q.results()["theta"]).all(), [r["kernel"] for r in q.launch_stats() if r["n_loci"]])
 q.close()
-del os.environ["SBQ_GRID_NO_DUAL"]
-q = api.Quantifier(max_iter=5)                            # device generator -> two-slot kernel (layout + packing passes)
+q = api.Quantifier(max_iter=5)                           # device generator -> two-slot kernel (layout + packing passes)
 q.synth_giant([0, 3], 7000)
 q.solve(14000)
 q.finalize_tpm(q.fpkm_sum())
