@@ -68,26 +68,6 @@ struct PinnedVec {
    }
 };
 
-struct DevBuf {
-   void* p = nullptr;
-   size_t cap = 0;
-   bool reserve(size_t bytes) {
-      if (bytes <= cap) return true;
-      if (p) cudaFree(p);
-      p = nullptr;
-      cap = 0;
-      size_t want = bytes + bytes / 8 + 4096;
-      if (cudaMalloc(&p, want) != cudaSuccess) return false;
-      cap = want;
-      return true;
-   }
-   void release() {
-      if (p) cudaFree(p);
-      p = nullptr;
-      cap = 0;
-   }
-};
-
 struct LaunchClass {      // one kernel launch of the cluster tier
    int cs, lpr;           // lpr doubles as the thread count of the launch (CL_NT or CL_NT_SMALL)
    std::vector<int32_t> loci;
@@ -557,18 +537,17 @@ int launch_grid_class(sbq_ctx* c, GridClass& g, int& n_launch) {
    for (size_t i = 0; i < g.list.size(); ++i) h_iso[i] = c->meta[g.list[i]].T;
    g.variant = n_dual ? 3 : n_tma ? 2 : 1;
    int rc = 0, nl = 0;
+   unsigned short* c16 = (unsigned short*)c->d_col16.p;   // sized by sbq_solve before any giant class launches
    if (n_dual) {
-      GridDualBufs bf{&g.scratch.p, &g.scratch.cap, &c->d_col16.p, &c->d_col16.cap, &g.rowrec.p, &g.rowrec.cap, &g.pk.p, &g.pk.cap};
-      rc = grid_dual_launch(c->dp, c->nnz, d_list, n_dual, h_iso.data(), g.rec_off.data(), prop, bf, c->col16_ready, g.st, &nl);
+      rc = grid_dual_launch(c->dp, d_list, n_dual, h_iso.data(), g.rec_off.data(), prop, g.scratch, c16, g.rowrec, g.pk, c->col16_ready, g.st, &nl);
       n_launch += nl;
    }
    if (rc == 0 && n_tma) {
-      rc = grid_tma_launch(c->dp, c->nnz, d_list + n_dual, n_tma, h_iso.data() + n_dual, prop, &g.scratch.p, &g.scratch.cap, &c->d_col16.p, &c->d_col16.cap,
-                           c->col16_ready, g.st, &nl);
+      rc = grid_tma_launch(c->dp, d_list + n_dual, n_tma, h_iso.data() + n_dual, prop, g.scratch, c16, c->col16_ready, g.st, &nl);
       n_launch += nl;
    }
    if (rc == 0 && n_reg) {
-      rc = grid_tier_launch(c->dp, d_list + n_dual + n_tma, n_reg, prop, &g.scratch.p, &g.scratch.cap, g.st, &nl);
+      rc = grid_tier_launch(c->dp, d_list + n_dual + n_tma, n_reg, prop, g.scratch, g.st, &nl);
       n_launch += nl;
    }
    return rc;

@@ -328,38 +328,8 @@ em_bias_kernel(DevParams p, BiasParams bp, const int32_t* __restrict__ list, int
    }
 
    // ---- outputs + epilogue (same tail as the other tiers, src/estimate.cpp:310-356)
-   const bool uniform = status == LOCUS_ZERO_DENOM || status == LOCUS_NO_ROWS;
-   double fsum = 0.0;
-   for (int j = tid; j < T; j += BI_NT) {
-      const double tj = uniform ? theta0 : cur[j];
-      bool na = false;
-      double f = 0.0;
-      if (status != LOCUS_NO_ROWS) f = iso_fpkm(p, tj, p.iso_len[t0 + j], na);
-      p.theta[t0 + j] = tj;
-      p.fpkm[t0 + j] = f;
-      th[j] = na ? -1.0 : 0.0;
-      fsum += f;
-   }
-   fsum = block_sum<BI_NT>(fsum, red);
-   double ksum = 0.0;
-   for (int j = tid; j < T; j += BI_NT) {
-      const bool na = th[j] < 0;
-      const double f = p.fpkm[t0 + j];
-      double fr = 0.0;
-      int kp = 0;
-      if (status != LOCUS_NO_ROWS) {
-         if (!na) fr = f / fsum;
-         kp = !(fr < p.min_frac) ? (na ? -1 : 1) : 0;
-      }
-      p.frac[t0 + j] = fr;
-      p.keep[t0 + j] = kp;
-      if (kp != 0) ksum += f;
-   }
-   ksum = block_sum<BI_NT>(ksum, red);
+   locus_epilogue_block<BI_NT>(p, l, t0, T, status, iters, theta0, cur, th, red);
    if (tid == 0) {
-      p.iters[l] = iters;
-      p.status[l] = status;
-      p.locus_fpkm[l] = ksum;
       bp.outer[l] = outer;
       for (int a = 0; a < K; ++a) bp.beta[(size_t)l * K + a] = s_beta[a];
    }
@@ -628,30 +598,8 @@ em_bias_warp_kernel(DevParams p, BiasParams bp, const int32_t* __restrict__ list
       }
 
       // ---- outputs + epilogue (same tail as the EM warp tier, src/estimate.cpp:310-356)
-      const double theta_out = (status == LOCUS_ZERO_DENOM || status == LOCUS_NO_ROWS) ? theta0 : cur;
-      bool na = false;
-      double f = 0.0;
-      if (lane < T && status != LOCUS_NO_ROWS) f = iso_fpkm(p, theta_out, p.iso_len[t0 + lane], na);
-      const double sum = warp_sum(f);
-      double fr = 0.0;
-      int kp = 0;
-      if (lane < T && status != LOCUS_NO_ROWS) {
-         if (!na) fr = f / sum;
-         kp = !(fr < p.min_frac) ? (na ? -1 : 1) : 0;
-      }
-      const double kept_sum = warp_sum(kp != 0 ? f : 0.0);
-      if (lane < T) {
-         p.theta[t0 + lane] = theta_out;
-         p.fpkm[t0 + lane] = f;
-         p.frac[t0 + lane] = fr;
-         p.keep[t0 + lane] = kp;
-      }
-      if (lane == 0) {
-         p.iters[l] = iters;
-         p.status[l] = status;
-         p.locus_fpkm[l] = kept_sum;
-         bp.outer[l] = outer;
-      }
+      locus_epilogue_warp(p, l, t0, T, lane, status, iters, theta0, cur);
+      if (lane == 0) bp.outer[l] = outer;
 #pragma unroll
       for (int a = 0; a < BI_MAX_COV; ++a)
          if (lane == 0 && a < K) bp.beta[(size_t)l * K + a] = beta[a];

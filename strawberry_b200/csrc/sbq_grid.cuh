@@ -39,6 +39,65 @@ struct GridScratch {
    int tstride;
 };
 
+// ---- per-locus frame shared by the three giant-tier kernels (em_grid_kernel, em_grid_tma_kernel, em_grid_dual_kernel)
+
+// Rows [s_rows[0], s_rows[1]) of CTA b of nb: the locus's R rows split over the grid by non-zero count, inner boundaries rounded to
+// the nearest multiple of `chunk` rows (1: not rounded). Threads 0 and 1 write s_rows; the caller synchronises before reading it.
+__device__ __forceinline__ void grid_row_range(const int64_t* rp, int R, int chunk, int b, int nb, int* s_rows) {
+   const int tid = threadIdx.x;
+   if (tid < 2) {
+      const int64_t base = rp[0], nnz = rp[R] - base;
+      const int64_t target = base + (nnz * (int64_t)(b + tid)) / nb;
+      int lo = 0, hi = R;
+      if (b + tid >= nb) lo = R;
+      else if (b + tid == 0) hi = 0;
+      while (lo < hi) {
+         const int mid = (lo + hi) >> 1;
+         if (rp[mid] < target) lo = mid + 1; else hi = mid;
+      }
+      if (b + tid < nb) lo = min(R, (lo + chunk / 2) / chunk * chunk);
+      s_rows[tid] = lo;
+   }
+}
+
+// Adds the total / kept row counts of this warp's setup pass into the counters of list entry `item`.
+__device__ __forceinline__ void grid_publish_counts(const GridScratch& gs, int item, long long tot, long long kept) {
+   tot = warp_sum_ll(tot);
+   kept = warp_sum_ll(kept);
+   if ((threadIdx.x & 31) == 0 && (tot | kept)) {
+      atomicAdd((unsigned long long*)&gs.ctr[2 * item], (unsigned long long)tot);
+      atomicAdd((unsigned long long*)&gs.ctr[2 * item + 1], (unsigned long long)kept);
+   }
+}
+
+// Called by every CTA once it has written its partial[cta][0, T): column owners sum the partials over the CTAs, in CTA order,
+// into theta_next. Returns when theta_next is complete, on every CTA.
+template <int NT>
+__device__ __forceinline__ void grid_owner_reduce(cg::grid_group& grid, const GridScratch& gs, int T) {
+   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nb = gridDim.x;
+   grid.sync();
+   for (int j = blockIdx.x * (NT / 32) + warp; j < T; j += nb * (NT / 32)) {
+      double sj = 0.0;
+      for (int cta = lane; cta < nb; cta += 32) sj += __ldcg(gs.partial + (size_t)cta * gs.tstride + j);
+      sj = warp_sum(sj);
+      if (lane == 0) gs.theta_next[j] = sj;
+   }
+   grid.sync();
+}
+
+// Copies theta' (theta_next) into th[0, T) and returns ||theta' - cur||^2, the same value on every thread of every CTA.
+template <int NT>
+__device__ __forceinline__ double grid_read_next(const GridScratch& gs, const double* cur, double* th, int T, double* red) {
+   double d2 = 0.0;
+   for (int j = threadIdx.x; j < T; j += NT) {
+      const double nj = __ldcg(gs.theta_next + j);
+      const double diff = nj - cur[j];
+      d2 += diff * diff;
+      th[j] = nj;
+   }
+   return block_sum<NT>(d2, red);
+}
+
 __device__ __forceinline__ double ld_stream_f64(const double* p) {
    double v;
    asm volatile("ld.global.nc.L1::no_allocate.f64 %0, [%1];" : "=d"(v) : "l"(p));
@@ -172,7 +231,7 @@ em_grid_kernel(DevParams p, const int32_t* __restrict__ list, int n_list, GridSc
    extern __shared__ double smem[];
    __shared__ double red[GT_NT / 32];
    __shared__ int s_rows[2];
-   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+   const int tid = threadIdx.x;
    const int nb = gridDim.x, b = blockIdx.x;
 
    for (int item = 0; item < n_list; ++item) {
@@ -191,18 +250,7 @@ em_grid_kernel(DevParams p, const int32_t* __restrict__ list, int n_list, GridSc
       const int32_t* cnt = p.count + r0;
       double* my_partial = gs.partial + (size_t)b * gs.tstride;
 
-      if (tid < 2) {
-         const int64_t base = rp[0], nnz = rp[R] - base;
-         const int64_t target = base + (nnz * (int64_t)(b + tid)) / nb;
-         int lo = 0, hi = R;
-         if (b + tid >= nb) lo = R;
-         else if (b + tid == 0) hi = 0;
-         while (lo < hi) {
-            const int mid = (lo + hi) >> 1;
-            if (rp[mid] < target) lo = mid + 1; else hi = mid;
-         }
-         s_rows[tid] = lo;
-      }
+      grid_row_range(rp, R, 1, b, nb, s_rows);
       for (int x = tid; x < W * T; x += GT_NT) acc[x] = 0.0;
       __syncthreads();
       const int ra = s_rows[0], rb = s_rows[1];
@@ -211,26 +259,14 @@ em_grid_kernel(DevParams p, const int32_t* __restrict__ list, int n_list, GridSc
       long long tot = 0, kept = 0;
       int zero = 0;
       grid_row_pass<true>(p, rp, neff, cnt, ra, rb, W, th, acc, T, tot, kept, zero);
-      tot = warp_sum_ll(tot);
-      kept = warp_sum_ll(kept);
-      if (lane == 0 && (tot | kept)) {
-         atomicAdd((unsigned long long*)&gs.ctr[2 * item], (unsigned long long)tot);
-         atomicAdd((unsigned long long*)&gs.ctr[2 * item + 1], (unsigned long long)kept);
-      }
+      grid_publish_counts(gs, item, tot, kept);
       __syncthreads();
       for (int j = tid; j < T; j += GT_NT) {
          double sj = 0.0;
          for (int w = 0; w < W; ++w) { sj += acc[(size_t)w * T + j]; acc[(size_t)w * T + j] = 0.0; }
          my_partial[j] = sj;
       }
-      grid.sync();
-      for (int j = b * (GT_NT / 32) + warp; j < T; j += nb * (GT_NT / 32)) {
-         double sj = 0.0;
-         for (int cta = lane; cta < nb; cta += 32) sj += __ldcg(gs.partial + (size_t)cta * gs.tstride + j);
-         sj = warp_sum(sj);
-         if (lane == 0) gs.theta_next[j] = sj;
-      }
-      grid.sync();
+      grid_owner_reduce<GT_NT>(grid, gs, T);
       const double total = (double)__ldcg(gs.ctr + 2 * item);
       const long long kept_all = __ldcg(gs.ctr + 2 * item + 1);
       const double theta0 = total / (double)T;
@@ -257,24 +293,12 @@ em_grid_kernel(DevParams p, const int32_t* __restrict__ list, int n_list, GridSc
                for (int w = 0; w < W; ++w) { sj += acc[(size_t)w * T + j]; acc[(size_t)w * T + j] = 0.0; }
                my_partial[j] = sj;
             }
-            grid.sync();
-            for (int j = b * (GT_NT / 32) + warp; j < T; j += nb * (GT_NT / 32)) {
-               double sj = 0.0;
-               for (int cta = lane; cta < nb; cta += 32) sj += __ldcg(gs.partial + (size_t)cta * gs.tstride + j);
-               sj = warp_sum(sj);
-               if (lane == 0) gs.theta_next[j] = sj;
-            }
-            grid.sync();
+            grid_owner_reduce<GT_NT>(grid, gs, T);
             const int zf = *(volatile int*)&gs.zero_flag[item];
-            double d2 = 0.0;
-            for (int j = tid; j < T; j += GT_NT) {
-               const double nj = __ldcg(gs.theta_next + j);
-               const double diff = nj - cur[j];
-               d2 += diff * diff;
-               th[j] = nj;
-            }
-            d2 = block_sum<GT_NT>(d2, red);
+            const double d2 = grid_read_next<GT_NT>(gs, cur, th, T, red);
             if (zf) { status = LOCUS_ZERO_DENOM; break; }
+            // (the TMA and two-slot kernels test d2 < tol^2: the two tests can disagree in the last bit, so unifying them could
+            // change an iteration count)
             if (sqrt(d2) < p.tol) { status = LOCUS_OK; break; }
             for (int j = tid; j < T; j += GT_NT) {
                const double nj = th[j];
@@ -288,48 +312,69 @@ em_grid_kernel(DevParams p, const int32_t* __restrict__ list, int n_list, GridSc
 
       // ---- outputs + epilogue by CTA 0 (src/estimate.cpp:310-356)
       if (b == 0) {
-         const bool uniform = status == LOCUS_ZERO_DENOM || status == LOCUS_NO_ROWS;
-         double fsum = 0.0;
-         for (int j = tid; j < T; j += GT_NT) {
-            const double tj = uniform ? theta0 : cur[j];
-            bool na = false;
-            double f = 0.0;
-            if (status != LOCUS_NO_ROWS) f = iso_fpkm(p, tj, p.iso_len[t0 + j], na);
-            p.theta[t0 + j] = tj;
-            p.fpkm[t0 + j] = f;
-            th[j] = na ? -1.0 : 0.0;
-            fsum += f;
-         }
-         fsum = block_sum<GT_NT>(fsum, red);
-         double ksum = 0.0;
-         for (int j = tid; j < T; j += GT_NT) {
-            const bool na = th[j] < 0;
-            const double f = p.fpkm[t0 + j];
-            double fr = 0.0;
-            int kp = 0;
-            if (status != LOCUS_NO_ROWS) {
-               if (!na) fr = f / fsum;
-               kp = !(fr < p.min_frac) ? (na ? -1 : 1) : 0;
-            }
-            p.frac[t0 + j] = fr;
-            p.keep[t0 + j] = kp;
-            if (kp != 0) ksum += f;
-         }
-         ksum = block_sum<GT_NT>(ksum, red);
-         if (tid == 0) {
-            p.iters[l] = iters;
-            p.status[l] = status;
-            p.locus_fpkm[l] = ksum;
-         }
+         locus_epilogue_block<GT_NT>(p, l, t0, T, status, iters, theta0, cur, th, red);
       }
       grid.sync();   // scratch (partial, theta_next) is reused by the next locus
    }
 }
 
-// Host launcher. Returns 0 or an sbq_error code (<0). scratch/scratch_cap: a device buffer the caller
-// owns and this function may grow.
-inline int grid_tier_launch(const DevParams& dp, const int32_t* d_list, int n_list, const cudaDeviceProp& prop, void** scratch,
-                            size_t* scratch_cap, cudaStream_t st, int* n_launch) {
+// ---- host side
+
+// Device buffer that grows on demand (it allocates 1/8 more than asked).
+struct DevBuf {
+   void* p = nullptr;
+   size_t cap = 0;
+   bool reserve(size_t bytes) {
+      if (bytes <= cap) return true;
+      if (p) cudaFree(p);
+      p = nullptr;
+      cap = 0;
+      size_t want = bytes + bytes / 8 + 4096;
+      if (cudaMalloc(&p, want) != cudaSuccess) return false;
+      cap = want;
+      return true;
+   }
+   void release() {
+      if (p) cudaFree(p);
+      p = nullptr;
+      cap = 0;
+   }
+};
+
+// Global scratch of one giant-tier launch, carved out of buf (grown if needed): partial[nb][tstride], then (cur_glob != nullptr)
+// the per-CTA theta copies [nb][tstride], theta_next[tstride] and the per-entry counters, which are cleared on st.
+// Returns 0 or an sbq_error code (<0).
+inline int grid_scratch(DevBuf& buf, int nb, int tstride, int n_list, double** cur_glob, cudaStream_t st, GridScratch* gs) {
+   const size_t arr = (size_t)nb * tstride * sizeof(double);
+   const size_t ctr_bytes = (size_t)n_list * (2 * sizeof(long long) + sizeof(int));
+   if (!buf.reserve(arr * (cur_glob ? 2 : 1) + (size_t)tstride * sizeof(double) + ctr_bytes + 1024)) return -4;
+   char* q = (char*)buf.p;
+   gs->partial = (double*)q; q += arr;
+   if (cur_glob) { *cur_glob = (double*)q; q += arr; }
+   gs->theta_next = (double*)q; q += (size_t)tstride * sizeof(double);
+   gs->ctr = (long long*)q; q += (size_t)n_list * 2 * sizeof(long long);
+   gs->zero_flag = (int*)q;
+   gs->tstride = tstride;
+   return cudaMemsetAsync(gs->ctr, 0, ctr_bytes, st) == cudaSuccess ? 0 : -3;
+}
+
+// Calls launch(i0, i1, nc, max_iso) for every run [i0, i1) of list entries with the same warp count nc = nc_of(T) (the planner
+// sorts the list by it; max_iso: the largest T of the run), one cooperative launch each. Returns the first non-zero result.
+template <typename NcOf, typename Launch>
+inline int grid_for_each_run(const int* h_iso, int n_list, NcOf nc_of, Launch launch) {
+   for (int i0 = 0; i0 < n_list;) {
+      const int nc = nc_of(h_iso[i0]);
+      int i1 = i0, mx = 1;
+      while (i1 < n_list && nc_of(h_iso[i1]) == nc) { mx = mx > h_iso[i1] ? mx : h_iso[i1]; ++i1; }
+      if (const int rc = launch(i0, i1, nc, mx)) return rc;
+      i0 = i1;
+   }
+   return 0;
+}
+
+// Host launcher. Returns 0 or an sbq_error code (<0). scratch: a device buffer the caller owns and this function may grow.
+inline int grid_tier_launch(const DevParams& dp, const int32_t* d_list, int n_list, const cudaDeviceProp& prop, DevBuf& scratch, cudaStream_t st,
+                            int* n_launch) {
    *n_launch = 0;
    if (n_list == 0) return 0;
    const size_t smem = GT_SMEM_CAP;
@@ -337,23 +382,9 @@ inline int grid_tier_launch(const DevParams& dp, const int32_t* d_list, int n_li
    int per_sm = 0;
    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, em_grid_kernel, GT_NT, smem) != cudaSuccess || per_sm < 1) return -3;
    const int nb = prop.multiProcessorCount;   // one CTA per SM
-   const int tstride = 4096;                   // >= T for every locus grid_tier_supports() accepts
-   const size_t need = ((size_t)nb * tstride + tstride) * sizeof(double) + (size_t)n_list * (2 * sizeof(long long) + sizeof(int)) + 1024;
-   if (need > *scratch_cap) {
-      if (*scratch) cudaFree(*scratch);
-      *scratch = nullptr;
-      *scratch_cap = 0;
-      if (cudaMalloc(scratch, need) != cudaSuccess) return -4;
-      *scratch_cap = need;
-   }
    GridScratch gs;
-   char* q = (char*)*scratch;
-   gs.partial = (double*)q; q += (size_t)nb * tstride * sizeof(double);
-   gs.theta_next = (double*)q; q += (size_t)tstride * sizeof(double);
-   gs.ctr = (long long*)q; q += (size_t)n_list * 2 * sizeof(long long);
-   gs.zero_flag = (int*)q;
-   gs.tstride = tstride;
-   if (cudaMemsetAsync(gs.ctr, 0, (size_t)n_list * (2 * sizeof(long long) + sizeof(int)), st) != cudaSuccess) return -3;
+   // tstride 4096: >= T for every locus grid_tier_supports() accepts
+   if (const int rc = grid_scratch(scratch, nb, 4096, n_list, nullptr, st, &gs)) return rc;
    DevParams dpc = dp;
    void* args[] = {(void*)&dpc, (void*)&d_list, (void*)&n_list, (void*)&gs};
    if (cudaLaunchCooperativeKernel((void*)em_grid_kernel, dim3(nb), dim3(GT_NT), args, smem, st) != cudaSuccess) return -3;

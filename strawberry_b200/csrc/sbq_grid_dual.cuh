@@ -695,7 +695,7 @@ em_grid_dual_kernel(DevParams p, const unsigned short* __restrict__ col16, RowRe
    __shared__ double red[C::NT / 32];
    __shared__ int s_rows[2];
    __shared__ __align__(8) uint64_t s_bar[G6_MAX_WARPS * G6_MAX_SPW];
-   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+   const int tid = threadIdx.x, warp = tid >> 5;
    const int nb = gridDim.x, b = blockIdx.x;
    const int ns = spw * C::CONSUMERS;   // stages of the CTA
 
@@ -726,20 +726,7 @@ em_grid_dual_kernel(DevParams p, const unsigned short* __restrict__ col16, RowRe
       double* my_partial = gs.partial + (size_t)b * gs.tstride;
       RowRec* rec_l = recs + rec_off[item];
 
-      if (tid < 2) {
-         // split rows over CTAs by non-zeros, boundaries rounded to whole chunks
-         const int64_t base = rp[0], nnz = rp[R] - base;
-         const int64_t target = base + (nnz * (int64_t)(b + tid)) / nb;
-         int lo = 0, hi = R;
-         if (b + tid >= nb) lo = R;
-         else if (b + tid == 0) hi = 0;
-         while (lo < hi) {
-            const int mid = (lo + hi) >> 1;
-            if (rp[mid] < target) lo = mid + 1; else hi = mid;
-         }
-         if (b + tid < nb) lo = min(R, (lo + C::CROWS / 2) / C::CROWS * C::CROWS);
-         s_rows[tid] = lo;
-      }
+      grid_row_range(rp, R, C::CROWS, b, nb, s_rows);
       for (int x = tid; x < C::CONSUMERS * T2; x += C::NT) acc[x] = 0.0;
       if (tid < 64) th2[2 * Tp + tid] = 0.0;   // dummy slots read as theta = 0
       __syncthreads();
@@ -766,24 +753,12 @@ em_grid_dual_kernel(DevParams p, const unsigned short* __restrict__ col16, RowRe
       long long tot = 0, kept = 0;
       int zero = 0;
       g6_pass<C, true>(p, col16, pk_cta, rec_cta, rp + ra, kbase, r0 + ra, rb - ra, n_chunk, ring, 16 * Tp, th2, my_acc, tot, kept, zero);
-      tot = warp_sum_ll(tot);
-      kept = warp_sum_ll(kept);
-      if (lane == 0 && (tot | kept)) {
-         atomicAdd((unsigned long long*)&gs.ctr[2 * item], (unsigned long long)tot);
-         atomicAdd((unsigned long long*)&gs.ctr[2 * item + 1], (unsigned long long)kept);
-      }
+      grid_publish_counts(gs, item, tot, kept);
       __threadfence();
       asm volatile("fence.proxy.async;" ::: "memory");
       __syncthreads();
       for (int j = tid; j < T; j += C::NT) my_partial[j] = fold(j);
-      grid.sync();
-      for (int j = b * (C::NT / 32) + warp; j < T; j += nb * (C::NT / 32)) {
-         double sj = 0.0;
-         for (int cta = lane; cta < nb; cta += 32) sj += __ldcg(gs.partial + (size_t)cta * gs.tstride + j);
-         sj = warp_sum(sj);
-         if (lane == 0) gs.theta_next[j] = sj;
-      }
-      grid.sync();
+      grid_owner_reduce<C::NT>(grid, gs, T);
       const double total = (double)__ldcg(gs.ctr + 2 * item);
       const long long kept_all = __ldcg(gs.ctr + 2 * item + 1);
       const double theta0 = total / (double)T;
@@ -809,23 +784,9 @@ em_grid_dual_kernel(DevParams p, const unsigned short* __restrict__ col16, RowRe
             zero = __syncthreads_or(zero);
             if (zero && tid == 0) atomicOr(&gs.zero_flag[item], 1);
             for (int j = tid; j < T; j += C::NT) my_partial[j] = fold(j);
-            grid.sync();
-            for (int j = b * (C::NT / 32) + warp; j < T; j += nb * (C::NT / 32)) {
-               double sj = 0.0;
-               for (int cta = lane; cta < nb; cta += 32) sj += __ldcg(gs.partial + (size_t)cta * gs.tstride + j);
-               sj = warp_sum(sj);
-               if (lane == 0) gs.theta_next[j] = sj;
-            }
-            grid.sync();
+            grid_owner_reduce<C::NT>(grid, gs, T);
             const int zf = *(volatile int*)&gs.zero_flag[item];
-            double d2 = 0.0;
-            for (int j = tid; j < T; j += C::NT) {
-               const double nj = __ldcg(gs.theta_next + j);
-               const double diff = nj - my_cur[j];
-               d2 += diff * diff;
-               th2[j] = nj;
-            }
-            d2 = block_sum<C::NT>(d2, red);
+            const double d2 = grid_read_next<C::NT>(gs, my_cur, th2, T, red);
             if (zf) { status = LOCUS_ZERO_DENOM; break; }
             if (d2 < tol2) { status = LOCUS_OK; break; }
             for (int j = tid; j < T; j += C::NT) {
@@ -842,39 +803,7 @@ em_grid_dual_kernel(DevParams p, const unsigned short* __restrict__ col16, RowRe
 
       // ---- outputs + epilogue by CTA 0 (src/estimate.cpp:310-356)
       if (b == 0) {
-         const bool uniform = status == LOCUS_ZERO_DENOM || status == LOCUS_NO_ROWS;
-         double fsum = 0.0;
-         for (int j = tid; j < T; j += C::NT) {
-            const double tj = uniform ? theta0 : my_cur[j];
-            bool na = false;
-            double f = 0.0;
-            if (status != LOCUS_NO_ROWS) f = iso_fpkm(p, tj, p.iso_len[t0 + j], na);
-            p.theta[t0 + j] = tj;
-            p.fpkm[t0 + j] = f;
-            th2[j] = na ? -1.0 : 0.0;
-            fsum += f;
-         }
-         fsum = block_sum<C::NT>(fsum, red);
-         double ksum = 0.0;
-         for (int j = tid; j < T; j += C::NT) {
-            const bool na = th2[j] < 0;
-            const double f = p.fpkm[t0 + j];
-            double fr = 0.0;
-            int kp = 0;
-            if (status != LOCUS_NO_ROWS) {
-               if (!na) fr = f / fsum;
-               kp = !(fr < p.min_frac) ? (na ? -1 : 1) : 0;
-            }
-            p.frac[t0 + j] = fr;
-            p.keep[t0 + j] = kp;
-            if (kp != 0) ksum += f;
-         }
-         ksum = block_sum<C::NT>(ksum, red);
-         if (tid == 0) {
-            p.iters[l] = iters;
-            p.status[l] = status;
-            p.locus_fpkm[l] = ksum;
-         }
+         locus_epilogue_block<C::NT>(p, l, t0, T, status, iters, theta0, my_cur, th2, red);
       }
       grid.sync();   // scratch (partial, theta_next) is reused by the next locus
    }
@@ -906,16 +835,10 @@ inline int grid_dual_nc(int T) {
    return 0;
 }
 
-struct GridDualBufs {
-   void** scratch; size_t* scratch_cap;      // partial / theta copies / counters
-   void** col16; size_t* col16_cap;          // u16 slots of the whole batch
-   void** recs; size_t* recs_cap;            // per-locus record offsets and first packed chunks (int64 each, at the front) + row records of the giant loci
-   void** pk; size_t* pk_cap;                // packed chunk stream of the giant loci (G6_PK_STRIDE bytes per 8-row chunk)
-};
-
 template <typename C>
-inline int grid_dual_launch_cfg(const DevParams& dp, const int32_t* d_list, int n_list, int max_iso, const cudaDeviceProp& prop, const GridDualBufs& bf,
-                                const int64_t* d_rec_off, RowRec* d_recs, const int64_t* d_pk_off, cudaStream_t st, int* n_launch) {
+inline int grid_dual_launch_cfg(const DevParams& dp, const int32_t* d_list, int n_list, int max_iso, const cudaDeviceProp& prop, DevBuf& scratch,
+                                const unsigned short* c16, const int64_t* d_rec_off, RowRec* d_recs, unsigned char* pk, const int64_t* d_pk_off,
+                                cudaStream_t st, int* n_launch) {
    const int spw = C::stages_per_warp(max_iso);
    const size_t smem = (size_t)spw * C::CONSUMERS * C::STAGE_BYTES + C::fixed_bytes(max_iso);
    auto kernel = em_grid_dual_kernel<C>;
@@ -923,28 +846,12 @@ inline int grid_dual_launch_cfg(const DevParams& dp, const int32_t* d_list, int 
    int per_sm = 0;
    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, C::NT, smem) != cudaSuccess || per_sm < 1) return -3;
    const int nb = prop.multiProcessorCount;
-   const int tstride = 2 * (((max_iso + 255) / 256) * 256);   // theta copy in the lower half, s_j in the upper half
-   const size_t need = ((size_t)nb * tstride * 2 + tstride) * sizeof(double) + (size_t)n_list * (2 * sizeof(long long) + sizeof(int)) + 1024;
-   if (need > *bf.scratch_cap) {
-      if (*bf.scratch) cudaFree(*bf.scratch);
-      *bf.scratch = nullptr;
-      *bf.scratch_cap = 0;
-      if (cudaMalloc(bf.scratch, need) != cudaSuccess) return -4;
-      *bf.scratch_cap = need;
-   }
    GridScratch gs;
-   char* q = (char*)*bf.scratch;
-   gs.partial = (double*)q; q += (size_t)nb * tstride * sizeof(double);
-   double* cur_glob = (double*)q; q += (size_t)nb * tstride * sizeof(double);
-   gs.theta_next = (double*)q; q += (size_t)tstride * sizeof(double);
-   gs.ctr = (long long*)q; q += (size_t)n_list * 2 * sizeof(long long);
-   gs.zero_flag = (int*)q;
-   gs.tstride = tstride;
-   if (cudaMemsetAsync(gs.ctr, 0, (size_t)n_list * (2 * sizeof(long long) + sizeof(int)), st) != cudaSuccess) return -3;
+   double* cur_glob = nullptr;
+   // theta copy in the lower half of tstride, s_j in the upper half
+   if (const int rc = grid_scratch(scratch, nb, 2 * (((max_iso + 255) / 256) * 256), n_list, &cur_glob, st, &gs)) return rc;
    DevParams dpc = dp;
-   const unsigned short* c16 = (const unsigned short*)*bf.col16;
    int ns_arg = spw;
-   unsigned char* pk = (unsigned char*)*bf.pk;
    void* args[] = {(void*)&dpc, (void*)&c16, (void*)&d_recs, (void*)&d_rec_off, (void*)&d_list, (void*)&n_list, (void*)&gs, (void*)&cur_glob, (void*)&ns_arg,
                    (void*)&pk, (void*)&d_pk_off};
    if (cudaLaunchCooperativeKernel((void*)kernel, dim3(nb), dim3(C::NT), args, smem, st) != cudaSuccess) return -3;
@@ -952,20 +859,15 @@ inline int grid_dual_launch_cfg(const DevParams& dp, const int32_t* d_list, int 
    return 0;
 }
 
-// h_rec_off: n_list + 1 record offsets (host; a locus of R rows owns R + 1 records). prepared: the sorted layout of this upload is already in place.
-inline int grid_dual_launch(const DevParams& dp, int64_t nnz_total, const int32_t* d_list, int n_list, const int* h_iso /* T of every list entry */, const int64_t* h_rec_off,
-                            const cudaDeviceProp& prop, const GridDualBufs& bf, bool prepared, cudaStream_t st, int* n_launch) {
+// h_rec_off: n_list + 1 record offsets (host; a locus of R rows owns R + 1 records). c16: the u16 slots of the whole batch (the
+// caller sizes the buffer). recs: per-locus record offsets and first packed chunks (int64 each, at the front) + row records of
+// the giant loci; pk: their packed chunk stream (G6_PK_STRIDE bytes per 8-row chunk). prepared: the sorted layout of this upload
+// is already in place.
+inline int grid_dual_launch(const DevParams& dp, const int32_t* d_list, int n_list, const int* h_iso /* T of every list entry */, const int64_t* h_rec_off,
+                            const cudaDeviceProp& prop, DevBuf& scratch, unsigned short* c16, DevBuf& recs, DevBuf& pk, bool prepared, cudaStream_t st,
+                            int* n_launch) {
    *n_launch = 0;
    if (n_list == 0) return 0;
-   const size_t need16 = (size_t)nnz_total * 2 + 256;
-   if (need16 > *bf.col16_cap) {
-      if (*bf.col16) cudaFree(*bf.col16);
-      *bf.col16 = nullptr;
-      *bf.col16_cap = 0;
-      if (cudaMalloc(bf.col16, need16) != cudaSuccess) return -4;
-      *bf.col16_cap = need16;
-      prepared = false;
-   }
    const size_t off_bytes = (((size_t)(n_list + 1) * 2 * sizeof(int64_t) + 255) / 256) * 256;   // record offsets | first packed chunks
    const size_t need_rec = off_bytes + (size_t)(h_rec_off[n_list] + 64) * sizeof(RowRec);
    std::vector<int64_t> h_off(2 * (size_t)(n_list + 1));
@@ -976,65 +878,46 @@ inline int grid_dual_launch(const DevParams& dp, int64_t nnz_total, const int32_
       h_off[n_list + 1 + i + 1] = h_off[n_list + 1 + i] + (R + G6_PK_ROWS - 1) / G6_PK_ROWS;
    }
    const size_t need_pk = (size_t)h_off[2 * n_list + 1] * G6_PK_STRIDE + 256;
-   if (need_pk > *bf.pk_cap) {
-      if (*bf.pk) cudaFree(*bf.pk);
-      *bf.pk = nullptr;
-      *bf.pk_cap = 0;
-      if (cudaMalloc(bf.pk, need_pk) != cudaSuccess) return -4;
-      *bf.pk_cap = need_pk;
+   if (need_pk > pk.cap || need_rec > recs.cap) {
+      if (!pk.reserve(need_pk) || !recs.reserve(need_rec)) return -4;
       prepared = false;
    }
-   if (need_rec > *bf.recs_cap) {
-      if (*bf.recs) cudaFree(*bf.recs);
-      *bf.recs = nullptr;
-      *bf.recs_cap = 0;
-      if (cudaMalloc(bf.recs, need_rec) != cudaSuccess) return -4;
-      *bf.recs_cap = need_rec;
-      prepared = false;
-   }
-   const int64_t* d_rec_off = (const int64_t*)*bf.recs;
+   const int64_t* d_rec_off = (const int64_t*)recs.p;
    const int64_t* d_pk_off = d_rec_off + (n_list + 1);
-   RowRec* d_recs = (RowRec*)((char*)*bf.recs + off_bytes);
+   RowRec* d_recs = (RowRec*)((char*)recs.p + off_bytes);
    if (!prepared) {
       // (pageable host vector: the copy is staged by the runtime before the call returns)
-      if (cudaMemcpyAsync(*bf.recs, h_off.data(), h_off.size() * sizeof(int64_t), cudaMemcpyHostToDevice, st) != cudaSuccess) return -3;
+      if (cudaMemcpyAsync(recs.p, h_off.data(), h_off.size() * sizeof(int64_t), cudaMemcpyHostToDevice, st) != cudaSuccess) return -3;
       const size_t psmem = (size_t)G6_PREP_WARPS * sizeof(G6PrepTile);
       if (cudaFuncSetAttribute(dual_prepare_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)psmem) != cudaSuccess) return -3;
-      dual_prepare_kernel<<<prop.multiProcessorCount * 2, G6_PREP_WARPS * 32, psmem, st>>>(dp, d_list, n_list, d_rec_off, d_recs, (unsigned short*)*bf.col16);
+      dual_prepare_kernel<<<prop.multiProcessorCount * 2, G6_PREP_WARPS * 32, psmem, st>>>(dp, d_list, n_list, d_rec_off, d_recs, c16);
       ++*n_launch;
       if (getenv("SBQ_DUAL_VERIFY")) {   // tests: the prepared layout must satisfy the kernel's conflict-freedom assumptions
          int* d_viol = nullptr;
          int h_viol = -1;
          if (cudaMalloc(&d_viol, sizeof(int)) != cudaSuccess) return -4;
          cudaMemsetAsync(d_viol, 0, sizeof(int), st);
-         dual_verify_kernel<<<prop.multiProcessorCount * 4, 256, 0, st>>>(dp, d_list, n_list, d_rec_off, d_recs, (const unsigned short*)*bf.col16, d_viol);
+         dual_verify_kernel<<<prop.multiProcessorCount * 4, 256, 0, st>>>(dp, d_list, n_list, d_rec_off, d_recs, c16, d_viol);
          cudaMemcpyAsync(&h_viol, d_viol, sizeof(int), cudaMemcpyDeviceToHost, st);
          cudaStreamSynchronize(st);
          cudaFree(d_viol);
          if (h_viol != 0) { fprintf(stderr, "sbq: two-slot layout check failed: %d groups violate it\n", h_viol); return -7; }
       }
-      dual_pack_kernel<<<prop.multiProcessorCount * 8, 256, 0, st>>>(dp, d_list, n_list, d_rec_off, d_recs, (const unsigned short*)*bf.col16, d_pk_off,
-                                                                   (unsigned char*)*bf.pk);
+      dual_pack_kernel<<<prop.multiProcessorCount * 8, 256, 0, st>>>(dp, d_list, n_list, d_rec_off, d_recs, c16, d_pk_off, (unsigned char*)pk.p);
       ++*n_launch;
    }
-   // one cooperative launch per run of loci with the same warp count (the planner sorts the list by it)
-   for (int i0 = 0; i0 < n_list;) {
-      const int nc = grid_dual_nc(h_iso[i0]);
-      int i1 = i0, mx = 1;
-      while (i1 < n_list && grid_dual_nc(h_iso[i1]) == nc) { mx = mx > h_iso[i1] ? mx : h_iso[i1]; ++i1; }
-      int rc = -6;
+   return grid_for_each_run(h_iso, n_list, grid_dual_nc, [&](int i0, int i1, int nc, int mx) {
+      const int32_t* li = d_list + i0;
+      unsigned char* pkp = (unsigned char*)pk.p;
       switch (nc) {
-         case 12: rc = grid_dual_launch_cfg<G6Cfg<12>>(dp, d_list + i0, i1 - i0, mx, prop, bf, d_rec_off + i0, d_recs, d_pk_off + i0, st, n_launch); break;
-         case 10: rc = grid_dual_launch_cfg<G6Cfg<10>>(dp, d_list + i0, i1 - i0, mx, prop, bf, d_rec_off + i0, d_recs, d_pk_off + i0, st, n_launch); break;
-         case 8: rc = grid_dual_launch_cfg<G6Cfg<8>>(dp, d_list + i0, i1 - i0, mx, prop, bf, d_rec_off + i0, d_recs, d_pk_off + i0, st, n_launch); break;
-         case 6: rc = grid_dual_launch_cfg<G6Cfg<6>>(dp, d_list + i0, i1 - i0, mx, prop, bf, d_rec_off + i0, d_recs, d_pk_off + i0, st, n_launch); break;
-         case 4: rc = grid_dual_launch_cfg<G6Cfg<4>>(dp, d_list + i0, i1 - i0, mx, prop, bf, d_rec_off + i0, d_recs, d_pk_off + i0, st, n_launch); break;
-         default: break;
+         case 12: return grid_dual_launch_cfg<G6Cfg<12>>(dp, li, i1 - i0, mx, prop, scratch, c16, d_rec_off + i0, d_recs, pkp, d_pk_off + i0, st, n_launch);
+         case 10: return grid_dual_launch_cfg<G6Cfg<10>>(dp, li, i1 - i0, mx, prop, scratch, c16, d_rec_off + i0, d_recs, pkp, d_pk_off + i0, st, n_launch);
+         case 8: return grid_dual_launch_cfg<G6Cfg<8>>(dp, li, i1 - i0, mx, prop, scratch, c16, d_rec_off + i0, d_recs, pkp, d_pk_off + i0, st, n_launch);
+         case 6: return grid_dual_launch_cfg<G6Cfg<6>>(dp, li, i1 - i0, mx, prop, scratch, c16, d_rec_off + i0, d_recs, pkp, d_pk_off + i0, st, n_launch);
+         case 4: return grid_dual_launch_cfg<G6Cfg<4>>(dp, li, i1 - i0, mx, prop, scratch, c16, d_rec_off + i0, d_recs, pkp, d_pk_off + i0, st, n_launch);
+         default: return -6;
       }
-      if (rc) return rc;
-      i0 = i1;
-   }
-   return 0;
+   });
 }
 
 }  // namespace sbq

@@ -378,18 +378,7 @@ em_grid_tma_kernel(DevParams p, const unsigned short* __restrict__ col16, const 
       const int32_t* cnt = p.count + r0;
       double* my_partial = gs.partial + (size_t)b * gs.tstride;
 
-      if (tid < 2) {
-         const int64_t base = rp[0], nnz = rp[R] - base;
-         const int64_t target = base + (nnz * (int64_t)(b + tid)) / nb;
-         int lo = 0, hi = R;
-         if (b + tid >= nb) lo = R;
-         else if (b + tid == 0) hi = 0;
-         while (lo < hi) {
-            const int mid = (lo + hi) >> 1;
-            if (rp[mid] < target) lo = mid + 1; else hi = mid;
-         }
-         s_rows[tid] = lo;
-      }
+      grid_row_range(rp, R, 1, b, nb, s_rows);
       for (int x = tid; x < C::ACC * T; x += C::NT) acc[x] = 0.0;
       __syncthreads();
       const int ra = s_rows[0], rb = s_rows[1];
@@ -408,12 +397,7 @@ em_grid_tma_kernel(DevParams p, const unsigned short* __restrict__ col16, const 
       } else {
          g4_consume<C, true>(p, col16, neff, cnt, rp, r0, kb, s_chunk, ra, rb, n_chunk, ring, use, th, my_acc, T, tot, kept, zero);
       }
-      tot = warp_sum_ll(tot);
-      kept = warp_sum_ll(kept);
-      if (lane == 0 && (tot | kept)) {
-         atomicAdd((unsigned long long*)&gs.ctr[2 * item], (unsigned long long)tot);
-         atomicAdd((unsigned long long*)&gs.ctr[2 * item + 1], (unsigned long long)kept);
-      }
+      grid_publish_counts(gs, item, tot, kept);
       __threadfence();
       asm volatile("fence.proxy.async;" ::: "memory");
       __syncthreads();
@@ -422,14 +406,7 @@ em_grid_tma_kernel(DevParams p, const unsigned short* __restrict__ col16, const 
          for (int w = 0; w < C::ACC; ++w) { sj += acc[(size_t)w * T + j]; acc[(size_t)w * T + j] = 0.0; }
          my_partial[j] = sj;
       }
-      grid.sync();
-      for (int j = b * (C::NT / 32) + warp; j < T; j += nb * (C::NT / 32)) {
-         double sj = 0.0;
-         for (int cta = lane; cta < nb; cta += 32) sj += __ldcg(gs.partial + (size_t)cta * gs.tstride + j);
-         sj = warp_sum(sj);
-         if (lane == 0) gs.theta_next[j] = sj;
-      }
-      grid.sync();
+      grid_owner_reduce<C::NT>(grid, gs, T);
       const double total = (double)__ldcg(gs.ctr + 2 * item);
       const long long kept_all = __ldcg(gs.ctr + 2 * item + 1);
       const double theta0 = total / (double)T;
@@ -464,23 +441,9 @@ em_grid_tma_kernel(DevParams p, const unsigned short* __restrict__ col16, const 
                for (int w = 0; w < C::ACC; ++w) { sj += acc[(size_t)w * T + j]; acc[(size_t)w * T + j] = 0.0; }
                my_partial[j] = sj;
             }
-            grid.sync();
-            for (int j = b * (C::NT / 32) + warp; j < T; j += nb * (C::NT / 32)) {
-               double sj = 0.0;
-               for (int cta = lane; cta < nb; cta += 32) sj += __ldcg(gs.partial + (size_t)cta * gs.tstride + j);
-               sj = warp_sum(sj);
-               if (lane == 0) gs.theta_next[j] = sj;
-            }
-            grid.sync();
+            grid_owner_reduce<C::NT>(grid, gs, T);
             const int zf = *(volatile int*)&gs.zero_flag[item];
-            double d2 = 0.0;
-            for (int j = tid; j < T; j += C::NT) {
-               const double nj = __ldcg(gs.theta_next + j);
-               const double diff = nj - my_cur[j];
-               d2 += diff * diff;
-               th[j] = nj;
-            }
-            d2 = block_sum<C::NT>(d2, red);
+            const double d2 = grid_read_next<C::NT>(gs, my_cur, th, T, red);
             if (zf) { status = LOCUS_ZERO_DENOM; break; }
             if (d2 < tol2) { status = LOCUS_OK; break; }
             for (int j = tid; j < T; j += C::NT) {
@@ -495,39 +458,7 @@ em_grid_tma_kernel(DevParams p, const unsigned short* __restrict__ col16, const 
 
       // ---- outputs + epilogue by CTA 0 (src/estimate.cpp:310-356)
       if (b == 0) {
-         const bool uniform = status == LOCUS_ZERO_DENOM || status == LOCUS_NO_ROWS;
-         double fsum = 0.0;
-         for (int j = tid; j < T; j += C::NT) {
-            const double tj = uniform ? theta0 : my_cur[j];
-            bool na = false;
-            double f = 0.0;
-            if (status != LOCUS_NO_ROWS) f = iso_fpkm(p, tj, p.iso_len[t0 + j], na);
-            p.theta[t0 + j] = tj;
-            p.fpkm[t0 + j] = f;
-            th[j] = na ? -1.0 : 0.0;
-            fsum += f;
-         }
-         fsum = block_sum<C::NT>(fsum, red);
-         double ksum = 0.0;
-         for (int j = tid; j < T; j += C::NT) {
-            const bool na = th[j] < 0;
-            const double f = p.fpkm[t0 + j];
-            double fr = 0.0;
-            int kp = 0;
-            if (status != LOCUS_NO_ROWS) {
-               if (!na) fr = f / fsum;
-               kp = !(fr < p.min_frac) ? (na ? -1 : 1) : 0;
-            }
-            p.frac[t0 + j] = fr;
-            p.keep[t0 + j] = kp;
-            if (kp != 0) ksum += f;
-         }
-         ksum = block_sum<C::NT>(ksum, red);
-         if (tid == 0) {
-            p.iters[l] = iters;
-            p.status[l] = status;
-            p.locus_fpkm[l] = ksum;
-         }
+         locus_epilogue_block<C::NT>(p, l, t0, T, status, iters, theta0, my_cur, th, red);
       }
       grid.sync();   // scratch (partial, theta_next) is reused by the next locus
    }
@@ -535,32 +466,18 @@ em_grid_tma_kernel(DevParams p, const unsigned short* __restrict__ col16, const 
 
 // One cooperative launch of the TMA path for loci of up to max_iso isoforms (the u16 columns are in place).
 template <typename C>
-inline int grid_tma_launch_cfg(const DevParams& dp, const int32_t* d_list, int n_list, int max_iso, const cudaDeviceProp& prop, void** scratch,
-                               size_t* scratch_cap, const unsigned short* c16, cudaStream_t st, int* n_launch) {
+inline int grid_tma_launch_cfg(const DevParams& dp, const int32_t* d_list, int n_list, int max_iso, const cudaDeviceProp& prop, DevBuf& scratch,
+                               const unsigned short* c16, cudaStream_t st, int* n_launch) {
    const size_t smem = C::smem_bytes(max_iso);
    auto kernel = em_grid_tma_kernel<C>;
    if (cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return -3;
    int per_sm = 0;
    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, C::NT, smem) != cudaSuccess || per_sm < 1) return -3;
    const int nb = prop.multiProcessorCount;
-   const int tstride = 8192;   // theta copy in the lower half, s_j in the upper half
-   const size_t need = ((size_t)nb * tstride * 2 + tstride) * sizeof(double) + (size_t)n_list * (2 * sizeof(long long) + sizeof(int)) + 1024;
-   if (need > *scratch_cap) {
-      if (*scratch) cudaFree(*scratch);
-      *scratch = nullptr;
-      *scratch_cap = 0;
-      if (cudaMalloc(scratch, need) != cudaSuccess) return -4;
-      *scratch_cap = need;
-   }
    GridScratch gs;
-   char* q = (char*)*scratch;
-   gs.partial = (double*)q; q += (size_t)nb * tstride * sizeof(double);
-   double* cur_glob = (double*)q; q += (size_t)nb * tstride * sizeof(double);
-   gs.theta_next = (double*)q; q += (size_t)tstride * sizeof(double);
-   gs.ctr = (long long*)q; q += (size_t)n_list * 2 * sizeof(long long);
-   gs.zero_flag = (int*)q;
-   gs.tstride = tstride;
-   if (cudaMemsetAsync(gs.ctr, 0, (size_t)n_list * (2 * sizeof(long long) + sizeof(int)), st) != cudaSuccess) return -3;
+   double* cur_glob = nullptr;
+   // tstride 8192: theta copy in the lower half, s_j in the upper half
+   if (const int rc = grid_scratch(scratch, nb, 8192, n_list, &cur_glob, st, &gs)) return rc;
    DevParams dpc = dp;
    void* args[] = {(void*)&dpc, (void*)&c16, (void*)&d_list, (void*)&n_list, (void*)&gs, (void*)&cur_glob};
    if (cudaLaunchCooperativeKernel((void*)kernel, dim3(nb), dim3(C::NT), args, smem, st) != cudaSuccess) return -3;
@@ -568,45 +485,27 @@ inline int grid_tma_launch_cfg(const DevParams& dp, const int32_t* d_list, int n
    return 0;
 }
 
-// Host launcher of the TMA path. h_iso: T of every list entry (host); the planner sorts the list by grid_tma_nc. col16_scratch:
-// device buffer for the u16 columns of the whole batch (grown here). cols_ready: the prepare pass of this upload already ran.
-inline int grid_tma_launch(const DevParams& dp, int64_t nnz_total, const int32_t* d_list, int n_list, const int* h_iso, const cudaDeviceProp& prop,
-                           void** scratch, size_t* scratch_cap, void** col16_scratch, size_t* col16_cap, bool cols_ready, cudaStream_t st,
-                           int* n_launch) {
+// Host launcher of the TMA path. h_iso: T of every list entry (host); the planner sorts the list by grid_tma_nc. c16: the u16
+// columns of the whole batch (the caller sizes the buffer); cols_ready: the prepare pass of this upload already filled it.
+inline int grid_tma_launch(const DevParams& dp, const int32_t* d_list, int n_list, const int* h_iso, const cudaDeviceProp& prop, DevBuf& scratch,
+                           unsigned short* c16, bool cols_ready, cudaStream_t st, int* n_launch) {
    *n_launch = 0;
    if (n_list == 0) return 0;
-   const size_t need16 = (size_t)nnz_total * 2 + 256;
-   if (need16 > *col16_cap) {
-      if (*col16_scratch) cudaFree(*col16_scratch);
-      *col16_scratch = nullptr;
-      *col16_cap = 0;
-      if (cudaMalloc(col16_scratch, need16) != cudaSuccess) return -4;
-      *col16_cap = need16;
-      cols_ready = false;
-   }
-   const unsigned short* c16 = (const unsigned short*)*col16_scratch;
    if (!cols_ready) {
-      grid_prepare_kernel<<<prop.multiProcessorCount * 8, 256, 0, st>>>(dp, d_list, n_list, (unsigned short*)c16);
+      grid_prepare_kernel<<<prop.multiProcessorCount * 8, 256, 0, st>>>(dp, d_list, n_list, c16);
       ++*n_launch;
    }
-   // one cooperative launch per run of loci with the same warp count
-   for (int i0 = 0; i0 < n_list;) {
-      const int nc = grid_tma_nc(h_iso[i0]);
-      int i1 = i0, mx = 1;
-      while (i1 < n_list && grid_tma_nc(h_iso[i1]) == nc) { mx = mx > h_iso[i1] ? mx : h_iso[i1]; ++i1; }
-      int rc = -6;
+   return grid_for_each_run(h_iso, n_list, grid_tma_nc, [&](int i0, int i1, int nc, int mx) {
+      const int32_t* li = d_list + i0;
       switch (nc) {
-         case 24: rc = grid_tma_launch_cfg<G4Cfg<24, 3>>(dp, d_list + i0, i1 - i0, mx, prop, scratch, scratch_cap, c16, st, n_launch); break;
-         case 20: rc = grid_tma_launch_cfg<G4Cfg<20, 3>>(dp, d_list + i0, i1 - i0, mx, prop, scratch, scratch_cap, c16, st, n_launch); break;
-         case 16: rc = grid_tma_launch_cfg<G4Cfg<16, 4>>(dp, d_list + i0, i1 - i0, mx, prop, scratch, scratch_cap, c16, st, n_launch); break;
-         case 12: rc = grid_tma_launch_cfg<G4Cfg<12, 4>>(dp, d_list + i0, i1 - i0, mx, prop, scratch, scratch_cap, c16, st, n_launch); break;
-         case 8: rc = grid_tma_launch_cfg<G4Cfg<8, 4>>(dp, d_list + i0, i1 - i0, mx, prop, scratch, scratch_cap, c16, st, n_launch); break;
-         default: break;
+         case 24: return grid_tma_launch_cfg<G4Cfg<24, 3>>(dp, li, i1 - i0, mx, prop, scratch, c16, st, n_launch);
+         case 20: return grid_tma_launch_cfg<G4Cfg<20, 3>>(dp, li, i1 - i0, mx, prop, scratch, c16, st, n_launch);
+         case 16: return grid_tma_launch_cfg<G4Cfg<16, 4>>(dp, li, i1 - i0, mx, prop, scratch, c16, st, n_launch);
+         case 12: return grid_tma_launch_cfg<G4Cfg<12, 4>>(dp, li, i1 - i0, mx, prop, scratch, c16, st, n_launch);
+         case 8: return grid_tma_launch_cfg<G4Cfg<8, 4>>(dp, li, i1 - i0, mx, prop, scratch, c16, st, n_launch);
+         default: return -6;
       }
-      if (rc) return rc;
-      i0 = i1;
-   }
-   return 0;
+   });
 }
 
 }  // namespace sbq

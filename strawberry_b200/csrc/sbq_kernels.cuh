@@ -96,6 +96,87 @@ __device__ __forceinline__ double iso_fpkm(const DevParams& p, double theta, int
    return theta * p.rpm * kb;
 }
 
+template <int NT>
+__device__ __forceinline__ double block_sum(double v, double* red) {
+   // fixed shape: warp butterfly, then every thread adds the warp totals in warp order
+   v = warp_sum(v);
+   if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
+   __syncthreads();
+   double t = 0.0;
+#pragma unroll
+   for (int w = 0; w < NT / 32; ++w) t += red[w];
+   __syncthreads();
+   return t;
+}
+
+// FPKM / frac / keep tail of one locus (src/estimate.cpp:310-356), written by the NT threads of one CTA. cur: theta of the
+// locus (ignored when the status resets it to theta0); na_scratch: T doubles of shared memory; red: block_sum's NT / 32 doubles.
+template <int NT>
+__device__ __forceinline__ void locus_epilogue_block(const DevParams& p, int l, int64_t t0, int T, int status, int iters, double theta0,
+                                                     const double* cur, double* na_scratch, double* red) {
+   const bool uniform = status == LOCUS_ZERO_DENOM || status == LOCUS_NO_ROWS;
+   double fsum = 0.0;
+   for (int j = threadIdx.x; j < T; j += NT) {
+      const double tj = uniform ? theta0 : cur[j];
+      bool na = false;
+      double f = 0.0;
+      if (status != LOCUS_NO_ROWS) f = iso_fpkm(p, tj, p.iso_len[t0 + j], na);
+      p.theta[t0 + j] = tj;
+      p.fpkm[t0 + j] = f;
+      na_scratch[j] = na ? -1.0 : 0.0;   // remember NA
+      fsum += f;
+   }
+   fsum = block_sum<NT>(fsum, red);
+   double ksum = 0.0;
+   for (int j = threadIdx.x; j < T; j += NT) {
+      const bool na = na_scratch[j] < 0;
+      const double f = p.fpkm[t0 + j];
+      double fr = 0.0;
+      int kp = 0;
+      if (status != LOCUS_NO_ROWS) {
+         if (!na) fr = f / fsum;
+         kp = !(fr < p.min_frac) ? (na ? -1 : 1) : 0;
+      }
+      p.frac[t0 + j] = fr;
+      p.keep[t0 + j] = kp;
+      if (kp != 0) ksum += f;
+   }
+   ksum = block_sum<NT>(ksum, red);
+   if (threadIdx.x == 0) {
+      p.iters[l] = iters;
+      p.status[l] = status;
+      p.locus_fpkm[l] = ksum;
+   }
+}
+
+// The same tail for a locus whose T <= 32 isoforms are owned one per lane of a warp; cur: this lane's theta.
+__device__ __forceinline__ void locus_epilogue_warp(const DevParams& p, int l, int64_t t0, int T, int lane, int status, int iters, double theta0,
+                                                    double cur) {
+   const double theta_out = (status == LOCUS_ZERO_DENOM || status == LOCUS_NO_ROWS) ? theta0 : cur;
+   bool na = false;
+   double f = 0.0;
+   if (lane < T && status != LOCUS_NO_ROWS) f = iso_fpkm(p, theta_out, p.iso_len[t0 + lane], na);
+   const double sum = warp_sum(f);
+   double fr = 0.0;
+   int kp = 0;
+   if (lane < T && status != LOCUS_NO_ROWS) {
+      if (!na) fr = f / sum;
+      kp = !(fr < p.min_frac) ? (na ? -1 : 1) : 0;
+   }
+   const double kept_sum = warp_sum(kp != 0 ? f : 0.0);
+   if (lane < T) {
+      p.theta[t0 + lane] = theta_out;
+      p.fpkm[t0 + lane] = f;
+      p.frac[t0 + lane] = fr;
+      p.keep[t0 + lane] = kp;
+   }
+   if (lane == 0) {
+      p.iters[l] = iters;
+      p.status[l] = status;
+      p.locus_fpkm[l] = kept_sum;
+   }
+}
+
 // --------------------------------------------------------------------------------------------
 // Tier 1: one warp per small locus (T <= 32). Lane i owns rows i, i+32, ...; lane j owns theta_j.
 // Accumulators acc[j][lane] are lane-private (stride 33 doubles per column: conflict-free both for
@@ -272,29 +353,7 @@ em_warp_kernel(DevParams p, const int32_t* __restrict__ list, int n_list, int ma
       }
 
       // ---- outputs + epilogue (src/estimate.cpp:310-356)
-      const double theta_out = (status == LOCUS_ZERO_DENOM || status == LOCUS_NO_ROWS) ? theta0 : cur;
-      bool na = false;
-      double f = 0.0;
-      if (lane < T && status != LOCUS_NO_ROWS) f = iso_fpkm(p, theta_out, p.iso_len[t0 + lane], na);
-      const double sum = warp_sum(f);
-      double fr = 0.0;
-      int kp = 0;
-      if (lane < T && status != LOCUS_NO_ROWS) {
-         if (!na) fr = f / sum;
-         kp = !(fr < p.min_frac) ? (na ? -1 : 1) : 0;
-      }
-      const double kept_sum = warp_sum(kp != 0 ? f : 0.0);
-      if (lane < T) {
-         p.theta[t0 + lane] = theta_out;
-         p.fpkm[t0 + lane] = f;
-         p.frac[t0 + lane] = fr;
-         p.keep[t0 + lane] = kp;
-      }
-      if (lane == 0) {
-         p.iters[l] = iters;
-         p.status[l] = status;
-         p.locus_fpkm[l] = kept_sum;
-      }
+      locus_epilogue_warp(p, l, t0, T, lane, status, iters, theta0, cur);
       __syncwarp();
    }
 }
@@ -358,19 +417,6 @@ __host__ __device__ inline size_t cluster_class_smem(int max_iso, size_t slice_b
 // per-CTA resident slice estimate with 12 % slack for the row-granular split
 __host__ __device__ inline size_t cluster_slice_estimate(long long nnz, long long R, int T, int cs) {
    return (size_t)(1.12 * (double)cluster_resident_bytes((size_t)(nnz / cs + 1), (size_t)(R / cs + 1), T)) + 512;
-}
-
-template <int NT>
-__device__ __forceinline__ double block_sum(double v, double* red) {
-   // fixed shape: warp butterfly, then every thread adds the warp totals in warp order
-   v = warp_sum(v);
-   if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
-   __syncthreads();
-   double t = 0.0;
-#pragma unroll
-   for (int w = 0; w < NT / 32; ++w) t += red[w];
-   __syncthreads();
-   return t;
 }
 
 // Row accessor of one CTA's slice streamed from global/L2 (fallback when the slice does not fit shared memory).
@@ -1388,39 +1434,7 @@ em_cluster_kernel(DevParams p, const int32_t* __restrict__ list, int n_list, uns
 
    if (rank != 0) return;
    // ---- outputs + epilogue (src/estimate.cpp:310-356), CTA 0 of the cluster
-   const bool uniform = status == LOCUS_ZERO_DENOM || status == LOCUS_NO_ROWS;
-   double fsum = 0.0;
-   for (int j = tid; j < T; j += NT) {
-      const double tj = uniform ? theta0 : cur[j];
-      bool na = false;
-      double f = 0.0;
-      if (status != LOCUS_NO_ROWS) f = iso_fpkm(p, tj, p.iso_len[t0 + j], na);
-      p.theta[t0 + j] = tj;
-      p.fpkm[t0 + j] = f;
-      th[j] = na ? -1.0 : 0.0;   // remember NA
-      fsum += f;
-   }
-   fsum = block_sum<NT>(fsum, red);
-   double ksum = 0.0;
-   for (int j = tid; j < T; j += NT) {
-      const bool na = th[j] < 0;
-      const double f = p.fpkm[t0 + j];
-      double fr = 0.0;
-      int kp = 0;
-      if (status != LOCUS_NO_ROWS) {
-         if (!na) fr = f / fsum;
-         kp = !(fr < p.min_frac) ? (na ? -1 : 1) : 0;
-      }
-      p.frac[t0 + j] = fr;
-      p.keep[t0 + j] = kp;
-      if (kp != 0) ksum += f;
-   }
-   ksum = block_sum<NT>(ksum, red);
-   if (tid == 0) {
-      p.iters[l] = iters;
-      p.status[l] = status;
-      p.locus_fpkm[l] = ksum;
-   }
+   locus_epilogue_block<NT>(p, l, t0, T, status, iters, theta0, cur, th, red);
 }
 
 // --------------------------------------------------------------------------------------------

@@ -432,6 +432,33 @@ def test_giant_loci_are_solved_the_same_whatever_shares_their_batch(q, oracle_mo
         assert res["iters"][l] == alone["iters"][0] and res["status"][l] == alone["status"][0], l
 
 
+@pytest.mark.parametrize("min_iso_frac", [0.01, 0.0])
+def test_epilogue_options_through_every_em_kernel(oracle_mod, min_iso_frac):
+    """The low-fraction filter and the effective-length "NA" branch (iso_len < insert_mean) through kernels the planner would
+    not send such loci to: the four giant-tier launches of the batch above (two-slot, TMA ring at 24 and 12 warps,
+    register-staged), and the warp and cluster tiers on the golden batch (all four locus outcomes). Every solve against the
+    oracle, keep flags signed: -1 for a kept NA isoform, which only happens without the filter (it has frac 0)."""
+    rng = np.random.default_rng(29)
+    giant = synth.concat([_shape_locus(rng, 300, 3000, 80), _shape_locus(rng, 1200, 3000, 80), _shape_locus(rng, 2700, 3000, 30),
+                          _shape_locus(rng, 600, 3000, 30)])
+    giant["total_mapped_reads"] = 1_000_000
+    golden, *_ = load_golden()
+    kw = dict(min_iso_frac=min_iso_frac, effective_len_norm=1, insert_mean=200.0)
+    for b, tier, cluster, counter in ((giant, 3, 0, "loci_grid"), (golden, 1, 0, "loci_warp"), (golden, 2, 2, "loci_cta")):
+        b["iso_len"] = b["iso_len"].copy()
+        b["iso_len"][::13] = 150
+        ora = oracle_mod.quantify_batch(b, b["total_mapped_reads"], min_iso_frac=min_iso_frac, effective_len_norm=True, insert_mean=200.0,
+                                        n_threads=4)
+        res = run_gpu(None, b, tier, cluster, **kw)
+        what = f"epilogue options, tier {tier} cluster {cluster}, min_iso_frac {min_iso_frac}"
+        assert res["stats"][counter] > 0, what
+        assert_matches_oracle(res, ora, b, what)
+        na = b["iso_len"] < 200
+        assert np.array_equal(res["keep"], np.where(na & (ora["keep"] != 0), -1, ora["keep"])), what
+        want = [0, 1] if min_iso_frac > 0 else [-1, 1]
+        assert all((res["keep"] == k).any() for k in want), what
+
+
 @pytest.mark.parametrize("cluster", [1, 2, 16])
 def test_cluster_tier_edge_shapes(q, oracle_mod, cluster):
     """Shapes that take the less common branches of the cluster kernel: more isoforms than threads (generic M-step),
