@@ -122,16 +122,24 @@ int  sbq_fetch_alpha(sbq_ctx*, double* alpha);
  * insert model come from sbq_set_insert_model; defer_weights is ignored) - and sbq_upload then builds the whole class table of
  * the batch on the GPU: compatibility (Contig::is_compatible), class coordinates (overlap_exons), first-seen class ids,
  * code-blind set semantics of ExonBin::_frags, float class masses, the class x isoform CSR and the weight descriptors that
- * weights_kernel turns into alpha. Integer results are bit-identical to sbq_build_locus (tests/test_gpu_rawbuild.py). A batch
- * is either all raw loci or none. In a multi-GPU context (n_gpus > 1) every raw locus is dealt to a device when it is submitted -
- * the device with the least hits x isoforms so far; its non-zeros are not known before the table exists - and the devices build
- * their tables concurrently; results come back in submit order. What the kernels cannot reproduce bit-exactly - fragment
- * masses that are not multiples of 1/2 (--allow-multimapped-hits), a hit touching more than 16 exon segments, a class spanning
- * more than 32 segments of an isoform - makes sbq_upload return SBQ_ERR_UNSUPPORTED: use sbq_build_locus for such a batch.
- * sbq_fetch_raw_classes (tests, single-device contexts) copies the device-built table out; the CSR comes from sbq_fetch_batch. */
+ * weights_kernel turns into alpha. Integer results are bit-identical to sbq_build_locus (tests/test_gpu_rawbuild.py,
+ * tests/test_gpu_rawbuild_long.py). A batch is either all raw loci or none. In a multi-GPU context (n_gpus > 1) every raw locus
+ * is dealt to a device when it is submitted - the device with the least hits x isoforms so far; its non-zeros are not known
+ * before the table exists - and the devices build their tables concurrently; results come back in submit order. A hit may
+ * touch any number of exon segments and a class may span any number of an isoform's segments (long reads, exon-dense loci),
+ * as in sbq_build_locus; a locus may have at most 65535 segments (sbq_submit_raw refuses more). What the kernels cannot
+ * reproduce bit-exactly - fragment masses that are not multiples of 1/2 (--allow-multimapped-hits), a 64-bit hash collision
+ * of two coordinate lists - and a class coordinate outside the isoform's segments (the reference asserts) make sbq_upload
+ * return SBQ_ERR_UNSUPPORTED: use sbq_build_locus for such a batch.
+ * sbq_fetch_raw_classes (tests, single-device contexts) copies the device-built table out; the CSR comes from sbq_fetch_batch.
+ * Its hit_coords[n_hit][16] holds the first 16 segments a hit touches (zeros after the last) and hit_ncoord[n_hit] their
+ * number, saturated at 255; for hits of at most 16 segments that is the whole list. sbq_fetch_raw_coords (tests,
+ * single-device contexts) copies the full lists: hit h touches hit_coords[hit_coord_off[h] .. hit_coord_off[h + 1]), and
+ * hit_coord_off[n_hit] is the length of hit_coords (fetch the offsets first, with hit_coords = NULL, to size it). */
 int  sbq_submit_raw(sbq_ctx*, const sbq_locus_input* in, int64_t* locus_index /* may be NULL: position of the locus in the batch (submit order) */);
 int  sbq_fetch_raw_classes(sbq_ctx*, int32_t* hit_class, uint8_t* hit_ncoord, uint16_t* hit_coords, int64_t* class_rep, float* class_mass,
                            int32_t* class_nfrag);
+int  sbq_fetch_raw_coords(sbq_ctx*, int64_t* hit_coord_off /* [n_hit + 1] */, uint16_t* hit_coords);
 
 /* hit_class[n_hit]: class id of every input hit (the ExonBin whose _frags set it was offered to), -1 for hits
  * that were dropped (ref_id -1) or are compatible with no isoform. */

@@ -16,7 +16,7 @@ CIG_M, CIG_I, CIG_D, CIG_N, CIG_S = 0, 1, 2, 3, 4
 BUILDER_SYMBOLS = ["sbq_build_locus", "sbq_table_free", "sbq_table_locus", "sbq_table_get_dims", "sbq_table_segments",
                    "sbq_table_iso_segments", "sbq_table_classes", "sbq_table_hit_classes", "sbq_table_weight_desc",
                    "sbq_set_insert_model", "sbq_submit_deferred", "sbq_fetch_alpha", "sbq_pair_features", "sbq_effective_len", "sbq_insert_pdf",
-                   "sbq_submit_raw", "sbq_fetch_raw_classes"]
+                   "sbq_submit_raw", "sbq_fetch_raw_classes", "sbq_fetch_raw_coords"]
 
 
 class InsertModel(ctypes.Structure):
@@ -56,6 +56,7 @@ def _lib():
                                         ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int32]
         L.sbq_submit_raw.argtypes = [ctypes.c_void_p, ctypes.POINTER(LocusInput), ctypes.c_void_p]
         L.sbq_fetch_raw_classes.argtypes = [ctypes.c_void_p] * 7
+        L.sbq_fetch_raw_coords.argtypes = [ctypes.c_void_p] * 3
         L.sbq_effective_len.restype = ctypes.c_int32
         L.sbq_effective_len.argtypes = [ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32]
         L.sbq_insert_pdf.restype = ctypes.c_double
@@ -204,8 +205,8 @@ def submit_raw(q, transcripts, hits, *, read_len, long_read=False, ref_ids=None)
 
 
 def fetch_raw_classes(q, n_hit):
-    """Device-built class table of the last raw upload (tests): per hit class id / touched segments, per class representative
-    hit, float mass and member count."""
+    """Device-built class table of the last raw upload (tests): per hit class id / touched segments (the first 16; ncoord
+    saturates at 255, fetch_raw_coords has the full lists), per class representative hit, float mass and member count."""
     L = _lib()
     st = q.stats()
     R = st["n_row"]
@@ -214,3 +215,13 @@ def fetch_raw_classes(q, n_hit):
     rep, mass, nfrag = np.zeros(max(R, 1), np.int64), np.zeros(max(R, 1), np.float32), np.zeros(max(R, 1), np.int32)
     q._chk(L.sbq_fetch_raw_classes(q._h, hit_class.ctypes.data, ncoord.ctypes.data, coords.ctypes.data, rep.ctypes.data, mass.ctypes.data, nfrag.ctypes.data))
     return dict(hit_class=hit_class[:n_hit], ncoord=ncoord[:n_hit], coords=coords[:n_hit], class_rep=rep[:R], class_mass=mass[:R], class_nfrag=nfrag[:R])
+
+
+def fetch_raw_coords(q, n_hit):
+    """Full coordinate lists of the last raw upload (tests): list h of the result is the segments hit h touches."""
+    L = _lib()
+    off = np.zeros(n_hit + 1, np.int64)
+    q._chk(L.sbq_fetch_raw_coords(q._h, off.ctypes.data, None))
+    pool = np.zeros(max(int(off[-1]), 1), np.uint16)
+    q._chk(L.sbq_fetch_raw_coords(q._h, None, pool.ctypes.data))
+    return [pool[off[h]:off[h + 1]] for h in range(n_hit)]

@@ -1028,7 +1028,7 @@ int sbq_upload(sbq_ctx* c) {
       if (!c->model_emp.empty()) CU(cudaMemcpyAsync(d_emp, c->model_emp.data(), c->model_emp.size() * 8, cudaMemcpyHostToDevice, st));
       WeightModel wm{c->model.use_emp, c->model.start_offset, c->model.end_offset, c->model.total_reads, d_emp, c->model.mean, c->model.sd, c->model_read_len};
       const int blocks = std::max(1, std::min<int>((int)((c->nnz + 7) / 8), c->prop.multiProcessorCount * 16));
-      weights_kernel<<<blocks, 256, 0, st>>>(c->nnz, d_seg, d_n, d_m, d_l, d_pool, wm, const_cast<double*>(c->dp.alpha));
+      weights_kernel<uint8_t><<<blocks, 256, 0, st>>>(c->nnz, d_seg, d_n, d_m, d_l, d_pool, wm, const_cast<double*>(c->dp.alpha));
       CU(cudaGetLastError());
       CU(cudaEventRecord(c->ev[6], st));
       CU(cudaStreamSynchronize(st));
@@ -1614,7 +1614,7 @@ static int raw_upload(sbq_ctx* c) {
    const size_t o_hm = sz(H * 4), o_hr = sz(H * 4), o_lho = sz((L + 1) * 8), o_lio = sz((L + 1) * 8), o_lso = sz((L + 1) * 8);
    const size_t o_ifp = sz((T + 1) * 8), o_ifo = sz(r.if_off.size() * 4), o_ifl = sz(r.if_len.size() * 4), o_ifc = sz(r.if_code.size());
    const size_t o_sl = sz(S * 4), o_sr = sz(S * 4), o_isp = sz((T + 1) * 8), o_isg = sz(r.iso_seg.size() * 4), o_il = sz(T * 4);
-   const size_t o_co = sz(H * RB_MAXC * 2), o_nc = sz(H), o_va = sz(H), o_ch = sz(H * 8), o_fh = sz(H * 8), o_cmo = sz((L + 1) * 8), o_cm = sz(CM * 4);
+   const size_t o_nc = sz(H * 4), o_co = sz((H + 1) * 8), o_va = sz(H), o_ch = sz(H * 8), o_fh = sz(H * 8), o_cmo = sz((L + 1) * 8), o_cm = sz(CM * 4);
    const size_t o_to = sz((L + 1) * 8), o_k1 = sz(TAB * 8), o_m1 = sz(TAB * 4), o_s1 = sz(H * 4), o_k2 = sz(TAB * 8), o_m2 = sz(TAB * 4), o_s2 = sz(H * 4);
    const size_t o_ir = sz(H * 4), o_cp = sz((H + 1) * 8), o_hc = sz(H * 4), o_fl = sz(64), o_bs = sz((size_t)n_scan * 8 + 8), o_g = sz((L + 1) * 8);
    if (!c->d_raw.reserve(need)) return fail(c, SBQ_ERR_NOMEM, "device allocation failed (raw batch, %zu MB)", need >> 20);
@@ -1644,7 +1644,7 @@ static int raw_upload(sbq_ctx* c) {
    b.if_len = (const uint32_t*)(base + o_ifl); b.if_code = (const uint8_t*)(base + o_ifc); b.seg_left = (const uint32_t*)(base + o_sl);
    b.seg_right = (const uint32_t*)(base + o_sr); b.iso_seg_ptr = (const int64_t*)(base + o_isp); b.iso_seg = (const int32_t*)(base + o_isg);
    b.iso_len = (const int32_t*)(base + o_il);
-   b.coords = (uint16_t*)(base + o_co); b.ncoord = (uint8_t*)(base + o_nc); b.valid = (uint8_t*)(base + o_va); b.chash = (unsigned long long*)(base + o_ch);
+   b.ncoord = (int32_t*)(base + o_nc); b.coord_off = (int64_t*)(base + o_co); b.valid = (uint8_t*)(base + o_va); b.chash = (unsigned long long*)(base + o_ch);
    b.fhash = (unsigned long long*)(base + o_fh); b.loc_cm_off = (const int64_t*)(base + o_cmo); b.cm = (uint32_t*)(base + o_cm);
    b.loc_tab_off = (const int64_t*)(base + o_to); b.keys1 = (unsigned long long*)(base + o_k1); b.min1 = (uint32_t*)(base + o_m1); b.slot1 = (uint32_t*)(base + o_s1);
    b.keys2 = (unsigned long long*)(base + o_k2); b.min2 = (uint32_t*)(base + o_m2); b.slot2 = (uint32_t*)(base + o_s2);
@@ -1661,10 +1661,10 @@ static int raw_upload(sbq_ctx* c) {
       int f = 0;
       CU(cudaMemcpyAsync(&f, b.flags, sizeof f, cudaMemcpyDeviceToHost, st));
       CU(cudaStreamSynchronize(st));
-      if (f) return fail(c, SBQ_ERR_UNSUPPORTED, "device class assignment refused the batch (%s):%s%s%s%s - use the host builder (sbq_build_locus) for it", where,
-                         f & RB_FLAG_COORDS ? " a hit touches more than 16 exon segments;" : "", f & RB_FLAG_COLLISION ? " 64-bit hash collision;" : "",
+      if (f) return fail(c, SBQ_ERR_UNSUPPORTED, "device class assignment refused the batch (%s):%s%s%s - use the host builder (sbq_build_locus) for it", where,
+                         f & RB_FLAG_COLLISION ? " 64-bit hash collision;" : "",
                          f & RB_FLAG_MASS ? " fragment masses are not multiples of 1/2 (or a class holds >= 2^23): the float sum would depend on the set order;" : "",
-                         f & RB_FLAG_NSEG ? " a class spans more than 32 segments of an isoform;" : "");
+                         f & RB_FLAG_NSEG ? " a class coordinate lies outside the isoform's segments (the reference asserts);" : "");
       return 0;
    };
    if (H) {
@@ -1674,10 +1674,12 @@ static int raw_upload(sbq_ctx* c) {
       CU(cudaGetLastError());
    }
    if (rb_scan(st, b.is_rep, H, d_bs, b.cls_prefix)) return fail(c, SBQ_ERR_CUDA, "scan failed");
-   // ---- round trip 1: classes per locus
+   if (rb_scan(st, b.ncoord, H, d_bs, b.coord_off)) return fail(c, SBQ_ERR_CUDA, "scan failed");
+   // ---- round trip 1: classes per locus, length of the coordinate pool
    rb_gather_kernel<<<(unsigned)((L + 1 + 255) / 256), 256, 0, st>>>(b.cls_prefix, b.loc_hit_off, L + 1, d_gather);
    std::vector<int64_t> cls_off(L + 1);
    CU(cudaMemcpyAsync(cls_off.data(), d_gather, (L + 1) * 8, cudaMemcpyDeviceToHost, st));
+   CU(cudaMemcpyAsync(&b.n_coord, b.coord_off + H, 8, cudaMemcpyDeviceToHost, st));
    if ((rc = check_flags("hits"))) return rc;
    const int64_t R = cls_off[L];
    std::vector<int64_t> cmask_off(L + 1, 0);
@@ -1691,7 +1693,8 @@ static int raw_upload(sbq_ctx* c) {
    auto sz2 = [&](size_t bytes) { const size_t o = need2; need2 += align_up(bytes + 16); return o; };
    const int n_scan2 = (int)((std::max<int64_t>(R, 1) + RB_SCAN_BLOCK - 1) / RB_SCAN_BLOCK);
    const size_t p_co = sz2((L + 1) * 8), p_mo = sz2((L + 1) * 8), p_cl = sz2(R * 4), p_rep = sz2(R * 8), p_ms = sz2(R * 4), p_nf = sz2(R * 4), p_cmk = sz2(cmask_off[L] * 4),
-                p_nz = sz2(R * 4), p_rp = sz2((R + 1) * 8), p_bs = sz2((size_t)n_scan2 * 8 + 8), p_g = sz2((L + 1) * 8);
+                p_nz = sz2(R * 4), p_rp = sz2((R + 1) * 8), p_bs = sz2((size_t)n_scan2 * 8 + 8), p_g = sz2((L + 1) * 8), p_hc = sz2(b.n_coord * 2),
+                p_ns = sz2(R * 4), p_po = sz2((R + 1) * 8);
    if (!c->d_raw2.reserve(need2)) return fail(c, SBQ_ERR_NOMEM, "device allocation failed (class arrays)");
    char* base2 = (char*)c->d_raw2.p;
    CU(cudaMemcpyAsync(base2 + p_co, cls_off.data(), (L + 1) * 8, cudaMemcpyHostToDevice, st));
@@ -1702,20 +1705,26 @@ static int raw_upload(sbq_ctx* c) {
    CU(cudaMemsetAsync(base2 + p_cmk, 0, align_up(cmask_off[L] * 4 + 16), st));
    b.loc_cls_off = (const int64_t*)(base2 + p_co); b.loc_cmask_off = (const int64_t*)(base2 + p_mo); b.class_rep = (int64_t*)(base2 + p_rep);
    b.class_mass = (float*)(base2 + p_ms); b.class_nfrag = (int32_t*)(base2 + p_nf); b.cmask = (uint32_t*)(base2 + p_cmk); b.class_nnz = (int32_t*)(base2 + p_nz);
+   b.coords = (uint16_t*)(base2 + p_hc); b.class_nseg = (int32_t*)(base2 + p_ns);
+   int64_t* d_pool_off = (int64_t*)(base2 + p_po);
    const int32_t* d_class_locus = (const int32_t*)(base2 + p_cl);
    int64_t* d_rp_tmp = (int64_t*)(base2 + p_rp);
    const int nbc = std::max(1, std::min<int>((int)((R + 127) / 128), c->prop.multiProcessorCount * 16));
    if (H) {
+      raw_coord_kernel<<<nbk, 128, 0, st>>>(b);
       raw_member_kernel<<<nbk, 256, 0, st>>>(b);
       raw_mass_kernel<<<nbk, 256, 0, st>>>(b);
    }
    if (R) raw_nnz_kernel<<<nbc, 256, 0, st>>>(b, R, d_class_locus);
    CU(cudaGetLastError());
    if (rb_scan(st, b.class_nnz, R, (long long*)(base2 + p_bs), d_rp_tmp)) return fail(c, SBQ_ERR_CUDA, "scan failed");
-   // ---- round trip 2: non-zeros per locus
+   if (rb_scan(st, b.class_nseg, R, (long long*)(base2 + p_bs), d_pool_off)) return fail(c, SBQ_ERR_CUDA, "scan failed");
+   // ---- round trip 2: non-zeros per locus, length of the descriptor pool
    rb_gather_kernel<<<(unsigned)((L + 1 + 255) / 256), 256, 0, st>>>(d_rp_tmp, b.loc_cls_off, L + 1, (int64_t*)(base2 + p_g));
    std::vector<int64_t> nz_off(L + 1);
+   int64_t n_pool = 0;
    CU(cudaMemcpyAsync(nz_off.data(), base2 + p_g, (L + 1) * 8, cudaMemcpyDeviceToHost, st));
+   CU(cudaMemcpyAsync(&n_pool, d_pool_off + R, 8, cudaMemcpyDeviceToHost, st));
    if ((rc = check_flags("classes"))) return rc;
    c->n_row = R;
    c->nnz = nz_off[L];
@@ -1727,18 +1736,18 @@ static int raw_upload(sbq_ctx* c) {
    CU(cudaMemcpyAsync(const_cast<int32_t*>(dp.iso_len), c->h_iso_len.p, T * 4, cudaMemcpyHostToDevice, st));
    // ---- CSR rows, counts, weight descriptors; alpha by weights_kernel (the same kernel the deferred host tables use)
    const int64_t nnz = c->nnz;
-   const size_t b_seg = align_up(nnz * 8 + 8), b_n = align_up(nnz + 8), b_m = align_up(nnz * 4 + 8), b_l = align_up(nnz * 4 + 8), b_pool = align_up((size_t)nnz * RB_POOL * 4 + 8),
+   const size_t b_seg = align_up(nnz * 8 + 8), b_n = align_up(nnz * 2 + 8), b_m = align_up(nnz * 4 + 8), b_l = align_up(nnz * 4 + 8), b_pool = align_up((size_t)n_pool * 4 + 8),
                 b_emp = align_up(c->model_emp.size() * 8 + 8);
    if (!c->d_weights.reserve(b_seg + b_n + b_m + b_l + b_pool + b_emp)) return fail(c, SBQ_ERR_NOMEM, "device allocation failed (weight descriptors)");
    char* q = (char*)c->d_weights.p;
    int64_t* d_seg = (int64_t*)q; q += b_seg;
-   uint8_t* d_n = (uint8_t*)q; q += b_n;
+   uint16_t* d_n = (uint16_t*)q; q += b_n;
    uint32_t* d_m = (uint32_t*)q; q += b_m;
    int32_t* d_l = (int32_t*)q; q += b_l;
    uint32_t* d_pool = (uint32_t*)q; q += b_pool;
    double* d_emp = (double*)q;
-   if (R) raw_fill_kernel<<<nbc, 128, 0, st>>>(b, R, d_class_locus, dp.row_ptr, const_cast<int32_t*>(dp.col), const_cast<double*>(dp.alpha), const_cast<int32_t*>(dp.count),
-                                               d_seg, d_n, d_m, d_l, d_pool);
+   if (R) raw_fill_kernel<<<nbc, 128, 0, st>>>(b, R, d_class_locus, dp.row_ptr, d_pool_off, const_cast<int32_t*>(dp.col), const_cast<double*>(dp.alpha),
+                                               const_cast<int32_t*>(dp.count), d_seg, d_n, d_m, d_l, d_pool);
    CU(cudaGetLastError());
    if ((rc = check_flags("weights"))) return rc;
    CU(cudaEventRecord(c->ev[5], st));
@@ -1746,7 +1755,7 @@ static int raw_upload(sbq_ctx* c) {
       if (!c->model_emp.empty()) CU(cudaMemcpyAsync(d_emp, c->model_emp.data(), c->model_emp.size() * 8, cudaMemcpyHostToDevice, st));
       WeightModel wm{c->model.use_emp, c->model.start_offset, c->model.end_offset, c->model.total_reads, d_emp, c->model.mean, c->model.sd, c->model_read_len};
       const int blocks = std::max(1, std::min<int>((int)((nnz + 7) / 8), c->prop.multiProcessorCount * 16));
-      weights_kernel<<<blocks, 256, 0, st>>>(nnz, d_seg, d_n, d_m, d_l, d_pool, wm, const_cast<double*>(dp.alpha));
+      weights_kernel<uint16_t><<<blocks, 256, 0, st>>>(nnz, d_seg, d_n, d_m, d_l, d_pool, wm, const_cast<double*>(dp.alpha));
       CU(cudaGetLastError());
    }
    CU(cudaEventRecord(c->ev[6], st));
@@ -1782,8 +1791,9 @@ static int raw_upload(sbq_ctx* c) {
 extern "C" {
 
 // Tests: the device-built class table of the last raw upload. hit_class[n_hit] (local class id or -1), hit_ncoord[n_hit] and
-// hit_coords[n_hit][16] (segment indices a hit touches), class_rep[n_row] (representative hit, batch-wide index),
-// class_mass[n_row], class_nfrag[n_row]; the CSR itself comes from sbq_fetch_batch. Any pointer may be NULL.
+// hit_coords[n_hit][16] (segment indices a hit touches: the first 16 of them, zeros after the last; the count saturates at 255 -
+// sbq_fetch_raw_coords has the full lists), class_rep[n_row] (representative hit, batch-wide index), class_mass[n_row],
+// class_nfrag[n_row]; the CSR itself comes from sbq_fetch_batch. Any pointer may be NULL.
 int sbq_fetch_raw_classes(sbq_ctx* c, int32_t* hit_class, uint8_t* hit_ncoord, uint16_t* hit_coords, int64_t* class_rep, float* class_mass, int32_t* class_nfrag) {
    if (!c) return SBQ_ERR_INVALID;
    std::lock_guard<std::mutex> lk(c->mu);
@@ -1792,12 +1802,40 @@ int sbq_fetch_raw_classes(sbq_ctx* c, int32_t* hit_class, uint8_t* hit_ncoord, u
    if (!c->resident || !c->raw_mode) return fail(c, SBQ_ERR_STATE, "sbq_fetch_raw_classes needs an uploaded raw batch");
    const RawBatch& b = c->rb;
    cudaStream_t st = c->stream;
+   std::vector<int64_t> off;
+   std::vector<uint16_t> pool;
+   if ((hit_ncoord || hit_coords) && b.n_hit) {
+      off.resize(b.n_hit + 1);
+      pool.resize(b.n_coord);
+      CU(cudaMemcpyAsync(off.data(), b.coord_off, (b.n_hit + 1) * 8, cudaMemcpyDeviceToHost, st));
+      if (b.n_coord) CU(cudaMemcpyAsync(pool.data(), b.coords, b.n_coord * 2, cudaMemcpyDeviceToHost, st));
+   }
    if (hit_class && b.n_hit) CU(cudaMemcpyAsync(hit_class, b.hit_class, b.n_hit * 4, cudaMemcpyDeviceToHost, st));
-   if (hit_ncoord && b.n_hit) CU(cudaMemcpyAsync(hit_ncoord, b.ncoord, b.n_hit, cudaMemcpyDeviceToHost, st));
-   if (hit_coords && b.n_hit) CU(cudaMemcpyAsync(hit_coords, b.coords, b.n_hit * RB_MAXC * 2, cudaMemcpyDeviceToHost, st));
    if (class_rep && c->n_row) CU(cudaMemcpyAsync(class_rep, b.class_rep, c->n_row * 8, cudaMemcpyDeviceToHost, st));
    if (class_mass && c->n_row) CU(cudaMemcpyAsync(class_mass, b.class_mass, c->n_row * 4, cudaMemcpyDeviceToHost, st));
    if (class_nfrag && c->n_row) CU(cudaMemcpyAsync(class_nfrag, b.class_nfrag, c->n_row * 4, cudaMemcpyDeviceToHost, st));
+   CU(cudaStreamSynchronize(st));
+   for (int64_t h = 0; h < (int64_t)off.size() - 1; ++h) {
+      const int64_t n = off[h + 1] - off[h];
+      if (hit_ncoord) hit_ncoord[h] = (uint8_t)std::min<int64_t>(n, 255);
+      if (hit_coords)
+         for (int64_t i = 0; i < 16; ++i) hit_coords[h * 16 + i] = i < n ? pool[off[h] + i] : 0;
+   }
+   return SBQ_SUCCESS;
+}
+
+// Tests: the full coordinate lists of the last raw upload. Hit h touches segments hit_coords[hit_coord_off[h] .. hit_coord_off[h + 1]);
+// hit_coord_off[n_hit] is the length of hit_coords. Either pointer may be NULL.
+int sbq_fetch_raw_coords(sbq_ctx* c, int64_t* hit_coord_off, uint16_t* hit_coords) {
+   if (!c) return SBQ_ERR_INVALID;
+   std::lock_guard<std::mutex> lk(c->mu);
+   if (c->multi) return fail(c, SBQ_ERR_UNSUPPORTED, "sbq_fetch_raw_coords is single-device (a test aid)");
+   CU(cudaSetDevice(c->device));
+   if (!c->resident || !c->raw_mode) return fail(c, SBQ_ERR_STATE, "sbq_fetch_raw_coords needs an uploaded raw batch");
+   const RawBatch& b = c->rb;
+   cudaStream_t st = c->stream;
+   if (hit_coord_off) CU(cudaMemcpyAsync(hit_coord_off, b.coord_off, (b.n_hit + 1) * 8, cudaMemcpyDeviceToHost, st));
+   if (hit_coords && b.n_coord) CU(cudaMemcpyAsync(hit_coords, b.coords, b.n_coord * 2, cudaMemcpyDeviceToHost, st));
    CU(cudaStreamSynchronize(st));
    return SBQ_SUCCESS;
 }

@@ -31,7 +31,8 @@ __device__ __forceinline__ int w_gap_ef(int l_left, int l_right, int l_int, int 
    return max(0, end - start);
 }
 
-// s: the entry's segment lengths (global memory, n <= 32), mask: implicit segments
+// s: the entry's segment lengths (global memory), mask: implicit segments, bit i & 31 for span index i (the reference's 32-bit
+// masks alias the same way)
 __device__ int w_effective_len(const uint32_t* __restrict__ s, int n, unsigned mask, int fl, int rl) {
    const int gap = fl - 2 * rl;
    if (n == 1) return (int)(s[0] - (uint32_t)fl + 1u);
@@ -55,7 +56,10 @@ __device__ int w_effective_len(const uint32_t* __restrict__ s, int n, unsigned m
    }
    const unsigned num_inners = (unsigned)n - 2;
    unsigned num_pos = 0;
-   const unsigned target = (n >= 32 ? 0xffffffffu : ((1u << n) - 1u)) & ~mask;
+   // the reference's target (uint32_t)(uint64_t)(pow(2, n) - 1) is all ones for 32 <= n <= 53 and 0 from n = 54 on, where
+   // 2^n - 1 rounds to 2^n in a double
+   const unsigned target = (n < 32 ? (1u << n) - 1u : n < 54 ? 0xffffffffu : 0u) & ~mask;
+   if (target == 0) return 0;   // every hit mask has bit 0 set: no start offset can match
    int inner_sum = 0;
    for (int k = 1; k < n - 1; ++k) inner_sum += (int)s[k];
    const unsigned last = s[n - 1];
@@ -95,8 +99,11 @@ __device__ __forceinline__ double w_insert_pdf(const WeightModel& m, unsigned fl
    return p > 0 ? p : 0.0;
 }
 
+// NSeg: uint8_t for descriptors built on the host (sbq_weight_desc, spans of at most 32 segments), uint16_t for those the device
+// class builder writes (a span may cover every segment of a locus, at most 65 535)
+template <typename NSeg>
 __global__ void __launch_bounds__(256)
-weights_kernel(int64_t n_entry, const int64_t* __restrict__ seg_ptr, const uint8_t* __restrict__ n_seg, const uint32_t* __restrict__ mask,
+weights_kernel(int64_t n_entry, const int64_t* __restrict__ seg_ptr, const NSeg* __restrict__ n_seg, const uint32_t* __restrict__ mask,
                const int32_t* __restrict__ iso_len, const uint32_t* __restrict__ pool, WeightModel m, double* __restrict__ alpha) {
    const int lane = threadIdx.x & 31;
    const int64_t wid = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5, nw = ((int64_t)gridDim.x * blockDim.x) >> 5;
