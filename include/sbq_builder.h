@@ -128,9 +128,9 @@ int  sbq_fetch_alpha(sbq_ctx*, double* alpha);
  * before the table exists - and the devices build their tables concurrently; results come back in submit order. A hit may
  * touch any number of exon segments and a class may span any number of an isoform's segments (long reads, exon-dense loci),
  * as in sbq_build_locus; a locus may have at most 65535 segments (sbq_submit_raw refuses more). What the kernels cannot
- * reproduce bit-exactly - fragment masses that are not multiples of 1/2 (--allow-multimapped-hits), a 64-bit hash collision
+ * reproduce bit-exactly - in the default mass mode fragment masses that are not multiples of 1/2, a 64-bit hash collision
  * of two coordinate lists - and a class coordinate outside the isoform's segments (the reference asserts) make sbq_upload
- * return SBQ_ERR_UNSUPPORTED: use sbq_build_locus for such a batch.
+ * return SBQ_ERR_UNSUPPORTED: use sbq_build_locus for such a batch. Fractional masses are accepted in SBQ_RAW_MASS_ANY mode (below).
  * sbq_fetch_raw_classes (tests, single-device contexts) copies the device-built table out; the CSR comes from sbq_fetch_batch.
  * Its hit_coords[n_hit][16] holds the first 16 segments a hit touches (zeros after the last) and hit_ncoord[n_hit] their
  * number, saturated at 255; for hits of at most 16 segments that is the whole list. sbq_fetch_raw_coords (tests,
@@ -140,6 +140,20 @@ int  sbq_submit_raw(sbq_ctx*, const sbq_locus_input* in, int64_t* locus_index /*
 int  sbq_fetch_raw_classes(sbq_ctx*, int32_t* hit_class, uint8_t* hit_ncoord, uint16_t* hit_coords, int64_t* class_rep, float* class_mass,
                            int32_t* class_nfrag);
 int  sbq_fetch_raw_coords(sbq_ctx*, int64_t* hit_coord_off /* [n_hit + 1] */, uint16_t* hit_coords);
+
+/* How the device adds the masses of a raw batch's classes (n_c = (int) sum of float masses over ExonBin::_frags,
+ * include/isoform.h:285-296; the sum runs in std::set<Contig> order: ref_id, then the feature lists lexicographically by
+ * (offset, len), op codes ignored, a proper prefix first).
+ *   SBQ_RAW_MASS_HALVES (default)  order-free atomic sum; exact, hence equal to the set-order sum, because every mass must be a
+ *                                  multiple of 1/2 and every class sum below 2^23 (collapse masses without
+ *                                  --allow-multimapped-hits); any other mass makes sbq_upload return SBQ_ERR_UNSUPPORTED.
+ *   SBQ_RAW_MASS_ANY               any finite, non-negative mass (1/NH fractions of multimapped hits): the surviving members of
+ *                                  every class are sorted in set order on the device and added in float in that order, bit for
+ *                                  bit the reference's sum. A class sum of 2^31 or more is refused ((int) is undefined there).
+ * The mode is per context, takes effect at the next sbq_upload and is forwarded to the devices of a multi-GPU context.
+ * An unknown mode returns SBQ_ERR_INVALID. */
+enum { SBQ_RAW_MASS_HALVES = 0, SBQ_RAW_MASS_ANY = 1 };
+int  sbq_set_raw_mass_mode(sbq_ctx*, int32_t mode);
 
 /* hit_class[n_hit]: class id of every input hit (the ExonBin whose _frags set it was offered to), -1 for hits
  * that were dropped (ref_id -1) or are compatible with no isoform. */

@@ -55,14 +55,14 @@ vector<int32_t> g_keep, g_status;
 
 struct Timers {   // SBQ_TIMING=1: where quantification time goes (printed at exit)
    atomic<long long> table_ns{0}, stage_ns{0}, run_ns{0}, finish_ns{0};
-   atomic<long long> loci{0};
+   atomic<long long> loci{0}, device_class_loci{0};
    bool on = getenv("SBQ_TIMING") != nullptr;
    ~Timers() {
       if (!on) return;
       sbq_stats st{};
       if (g_ctx) sbq_get_stats(g_ctx, &st);
-      fprintf(stderr, "SBQ_TIMING sbq loci %lld class_table_ms %.3f stage_ms %.3f run_ms %.3f (upload %.3f solve %.3f download %.3f) finish_ms %.3f\n", loci.load(),
-              table_ns / 1e6, stage_ns / 1e6, run_ns / 1e6, st.upload_ms, st.solve_ms, st.download_ms, finish_ns / 1e6);
+      fprintf(stderr, "SBQ_TIMING sbq loci %lld class_table_ms %.3f stage_ms %.3f run_ms %.3f (upload %.3f solve %.3f download %.3f) finish_ms %.3f device_class_loci %lld\n",
+              loci.load(), table_ns / 1e6, stage_ns / 1e6, run_ns / 1e6, st.upload_ms, st.solve_ms, st.download_ms, finish_ns / 1e6, device_class_loci.load());
    }
 } g_tm;
 long long now_ns() { return chrono::duration_cast<chrono::nanoseconds>(chrono::steady_clock::now().time_since_epoch()).count(); }
@@ -136,15 +136,20 @@ void LocusContext::assign_exon_bin(const vector<Contig>& hits, const vector<Geno
                       _read_len, long_read_sample ? 1 : 0, defer};
    tl_deferred = defer != 0;
    // Class assignment on the device as well (sbq_submit_raw): the locus is queued as it is - flattened hits and isoforms - and
-   // the whole class table of the sample is built by CUDA kernels during sbq_upload. Fragment masses must be multiples of 1/2
-   // (true unless --allow-multimapped-hits), -f needs the table on the host; SBQ_HOST_CLASSES=1 keeps the host builder.
-   tl_raw = defer && use_only_unique_hits && !getenv("SBQ_HOST_CLASSES");   // (on N GPUs libsbq deals every raw locus to a device at submit time)
-   if (defer && !g_model_set.load()) {      // the context's insert model and read length (once per sample)
+   // the whole class table of the sample is built by CUDA kernels during sbq_upload. With --allow-multimapped-hits the masses
+   // are 1/NH fractions, so the device adds them in the reference's set order (SBQ_RAW_MASS_ANY). -f needs the table on the
+   // host; SBQ_HOST_CLASSES=1 keeps the host builder.
+   tl_raw = defer && !getenv("SBQ_HOST_CLASSES");   // (on N GPUs libsbq deals every raw locus to a device at submit time)
+   if (defer && !g_model_set.load()) {      // the context's insert model, read length and mass mode (once per sample)
       lock_guard<mutex> lk(g_ctx_mu);
       if (!g_model_set.load()) {
          if (!g_ctx) g_insert_mean = ins._mean;
          const int rcm = sbq_set_insert_model(context(), &model, _read_len);
          if (rcm != SBQ_SUCCESS) { fprintf(stderr, "libsbq: sbq_set_insert_model: %s\n", sbq_error_string(rcm)); exit(1); }
+         if (!use_only_unique_hits) {
+            const int rcx = sbq_set_raw_mass_mode(context(), SBQ_RAW_MASS_ANY);
+            if (rcx != SBQ_SUCCESS) { fprintf(stderr, "libsbq: sbq_set_raw_mass_mode: %s\n", sbq_error_string(rcx)); exit(1); }
+         }
          g_model_set = true;
       }
    }
@@ -168,6 +173,7 @@ void LocusContext::assign_exon_bin(const vector<Contig>& hits, const vector<Geno
       }
       g_tm.table_ns += now_ns() - t_raw;
       g_tm.loci += 1;
+      g_tm.device_class_loci += 1;
       return;                                  // exon_bins stay empty: nothing on the host needs them without -f
    }
    sbq_table* tb = nullptr;

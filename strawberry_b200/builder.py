@@ -16,7 +16,8 @@ CIG_M, CIG_I, CIG_D, CIG_N, CIG_S = 0, 1, 2, 3, 4
 BUILDER_SYMBOLS = ["sbq_build_locus", "sbq_table_free", "sbq_table_locus", "sbq_table_get_dims", "sbq_table_segments",
                    "sbq_table_iso_segments", "sbq_table_classes", "sbq_table_hit_classes", "sbq_table_weight_desc",
                    "sbq_set_insert_model", "sbq_submit_deferred", "sbq_fetch_alpha", "sbq_pair_features", "sbq_effective_len", "sbq_insert_pdf",
-                   "sbq_submit_raw", "sbq_fetch_raw_classes", "sbq_fetch_raw_coords"]
+                   "sbq_submit_raw", "sbq_fetch_raw_classes", "sbq_fetch_raw_coords", "sbq_set_raw_mass_mode"]
+RAW_MASS_HALVES, RAW_MASS_ANY = 0, 1
 
 
 class InsertModel(ctypes.Structure):
@@ -57,6 +58,7 @@ def _lib():
         L.sbq_submit_raw.argtypes = [ctypes.c_void_p, ctypes.POINTER(LocusInput), ctypes.c_void_p]
         L.sbq_fetch_raw_classes.argtypes = [ctypes.c_void_p] * 7
         L.sbq_fetch_raw_coords.argtypes = [ctypes.c_void_p] * 3
+        L.sbq_set_raw_mass_mode.argtypes = [ctypes.c_void_p, ctypes.c_int32]
         L.sbq_effective_len.restype = ctypes.c_int32
         L.sbq_effective_len.argtypes = [ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32]
         L.sbq_insert_pdf.restype = ctypes.c_double
@@ -202,6 +204,13 @@ def submit_raw(q, transcripts, hits, *, read_len, long_read=False, ref_ids=None)
     inp = LocusInput(len(transcripts), _p(ip), _p(io), _p(il), _p(ic), len(hits), hp.ctypes.data, _p(ho), _p(hl), _p(hc),
                      _p(mass), _p(rid) if rid is not None else None, int(read_len), int(long_read), 1)
     q._chk(L.sbq_submit_raw(q._h, ctypes.byref(inp), None))
+
+
+def set_raw_mass_mode(q, mode):
+    """How q.upload() adds the class masses of raw loci (sbq_set_raw_mass_mode): RAW_MASS_HALVES (default; masses must be
+    multiples of 1/2, the atomic sum is exact) or RAW_MASS_ANY (any finite non-negative mass, e.g. the 1/NH fractions of
+    multimapped hits, added in the reference's std::set order)."""
+    q._chk(_lib().sbq_set_raw_mass_mode(q._h, int(mode)))
 
 
 def fetch_raw_classes(q, n_hit):

@@ -182,6 +182,7 @@ struct sbq_ctx {
       void clear() { *this = RawStage(); }
    } raw;
    bool raw_mode = false;
+   int32_t raw_mass_mode = SBQ_RAW_MASS_HALVES;   // sbq_set_raw_mass_mode
    DevBuf d_raw, d_raw2;
    RawBatch rb{};                    // device view of the last raw upload (tests fetch the class table through it)
 
@@ -1475,6 +1476,14 @@ int sbq_set_insert_model(sbq_ctx* c, const sbq_insert_model* model, int32_t read
    return SBQ_SUCCESS;
 }
 
+int sbq_set_raw_mass_mode(sbq_ctx* c, int32_t mode) {
+   if (!c || (mode != SBQ_RAW_MASS_HALVES && mode != SBQ_RAW_MASS_ANY)) return SBQ_ERR_INVALID;
+   std::lock_guard<std::mutex> lk(c->mu);
+   c->raw_mass_mode = mode;
+   c->resident = c->solved = c->downloaded = false;
+   return SBQ_SUCCESS;
+}
+
 int sbq_submit_deferred(sbq_ctx* c, const sbq_table* const* tables, int64_t n_tables) {
    if (!c || (!tables && n_tables > 0) || n_tables < 0) return SBQ_ERR_INVALID;
    for (int64_t t = 0; t < n_tables; ++t) {
@@ -1637,6 +1646,8 @@ static int raw_upload(sbq_ctx* c) {
    RawBatch& b = c->rb;
    b = RawBatch{};
    b.n_hit = H; b.n_loci = (int32_t)L; b.long_read = r.long_read;
+   const bool ordered = c->raw_mass_mode == SBQ_RAW_MASS_ANY;
+   b.mass_mode = ordered ? RB_MASS_ANY : RB_MASS_HALVES;
    b.hit_locus = (const int32_t*)(base + o_hl); b.hit_feat_ptr = (const int64_t*)(base + o_hfp); b.hf_off = (const uint32_t*)(base + o_hfo);
    b.hf_len = (const uint32_t*)(base + o_hfl); b.hf_code = (const uint8_t*)(base + o_hfc); b.hit_mass = (const float*)(base + o_hm);
    b.hit_ref = (const int32_t*)(base + o_hr); b.loc_hit_off = (const int64_t*)(base + o_lho); b.loc_iso_off = (const int64_t*)(base + o_lio);
@@ -1661,9 +1672,11 @@ static int raw_upload(sbq_ctx* c) {
       int f = 0;
       CU(cudaMemcpyAsync(&f, b.flags, sizeof f, cudaMemcpyDeviceToHost, st));
       CU(cudaStreamSynchronize(st));
-      if (f) return fail(c, SBQ_ERR_UNSUPPORTED, "device class assignment refused the batch (%s):%s%s%s - use the host builder (sbq_build_locus) for it", where,
-                         f & RB_FLAG_COLLISION ? " 64-bit hash collision;" : "",
-                         f & RB_FLAG_MASS ? " fragment masses are not multiples of 1/2 (or a class holds >= 2^23): the float sum would depend on the set order;" : "",
+      if (f) return fail(c, SBQ_ERR_UNSUPPORTED, "device class assignment refused the batch (%s, mass mode %s):%s%s%s - use the host builder (sbq_build_locus) for it", where,
+                         ordered ? "SBQ_RAW_MASS_ANY" : "SBQ_RAW_MASS_HALVES", f & RB_FLAG_COLLISION ? " 64-bit hash collision;" : "",
+                         !(f & RB_FLAG_MASS) ? ""
+                         : ordered ? " a fragment mass is NaN, infinite or negative (or a class holds >= 2^31, where (int) is undefined);"
+                                   : " fragment masses are not multiples of 1/2 (or a class holds >= 2^23): the float sum would depend on the set order (SBQ_RAW_MASS_ANY sums in set order);",
                          f & RB_FLAG_NSEG ? " a class coordinate lies outside the isoform's segments (the reference asserts);" : "");
       return 0;
    };
@@ -1695,6 +1708,10 @@ static int raw_upload(sbq_ctx* c) {
    const size_t p_co = sz2((L + 1) * 8), p_mo = sz2((L + 1) * 8), p_cl = sz2(R * 4), p_rep = sz2(R * 8), p_ms = sz2(R * 4), p_nf = sz2(R * 4), p_cmk = sz2(cmask_off[L] * 4),
                 p_nz = sz2(R * 4), p_rp = sz2((R + 1) * 8), p_bs = sz2((size_t)n_scan2 * 8 + 8), p_g = sz2((L + 1) * 8), p_hc = sz2(b.n_coord * 2),
                 p_ns = sz2(R * 4), p_po = sz2((R + 1) * 8);
+   // set-order mass sum: member offsets, per-class cursors, the survivors (at most H) as (class, prefix, hit) twice (merge ping-pong)
+   const int64_t HM = ordered ? H : 0;
+   const size_t p_mof = sz2(ordered ? (R + 1) * 8 : 0), p_cur = sz2(ordered ? R * 4 : 0), p_sk0 = sz2(HM * 8), p_sk1 = sz2(HM * 8), p_sh = sz2(HM * 8),
+                p_tk0 = sz2(HM * 8), p_tk1 = sz2(HM * 8), p_th = sz2(HM * 8);
    if (!c->d_raw2.reserve(need2)) return fail(c, SBQ_ERR_NOMEM, "device allocation failed (class arrays)");
    char* base2 = (char*)c->d_raw2.p;
    CU(cudaMemcpyAsync(base2 + p_co, cls_off.data(), (L + 1) * 8, cudaMemcpyHostToDevice, st));
@@ -1714,6 +1731,22 @@ static int raw_upload(sbq_ctx* c) {
       raw_coord_kernel<<<nbk, 128, 0, st>>>(b);
       raw_member_kernel<<<nbk, 256, 0, st>>>(b);
       raw_mass_kernel<<<nbk, 256, 0, st>>>(b);
+   }
+   if (ordered && R) {   // class masses in set order (SBQ_RAW_MASS_ANY); the number of survivors stays on the device (member_off[R])
+      int64_t* d_mof = (int64_t*)(base2 + p_mof);
+      unsigned long long *k0 = (unsigned long long*)(base2 + p_sk0), *k1 = (unsigned long long*)(base2 + p_sk1);
+      unsigned long long *t0 = (unsigned long long*)(base2 + p_tk0), *t1 = (unsigned long long*)(base2 + p_tk1);
+      int64_t *hh = (int64_t*)(base2 + p_sh), *th = (int64_t*)(base2 + p_th);
+      if (rb_scan(st, b.class_nfrag, R, (long long*)(base2 + p_bs), d_mof)) return fail(c, SBQ_ERR_CUDA, "scan failed");
+      CU(cudaMemsetAsync(base2 + p_cur, 0, R * 4, st));
+      raw_member_scatter_kernel<<<nbk, 256, 0, st>>>(b, d_mof, (int32_t*)(base2 + p_cur), k0, k1, hh);
+      raw_member_tile_sort_kernel<<<(unsigned)((H + RB_SORT_TILE - 1) / RB_SORT_TILE), RB_SORT_TILE / 2, 0, st>>>(b, d_mof + R, k0, k1, hh);
+      const int nbm = std::max(1, std::min<int>((int)((H + 256 * RB_MERGE_PER_THREAD - 1) / (256 * RB_MERGE_PER_THREAD)), c->prop.multiProcessorCount * 16));
+      for (int64_t w = RB_SORT_TILE; w < H; w *= 2) {   // H bounds the survivors: a pass whose runs already cover them all is a copy
+         raw_member_merge_kernel<<<nbm, 256, 0, st>>>(b, d_mof + R, w, k0, k1, hh, t0, t1, th);
+         std::swap(k0, t0); std::swap(k1, t1); std::swap(hh, th);
+      }
+      raw_member_sum_kernel<<<nbc, 256, 0, st>>>(b, R, d_mof, hh);
    }
    if (R) raw_nnz_kernel<<<nbc, 256, 0, st>>>(b, R, d_class_locus);
    CU(cudaGetLastError());

@@ -231,6 +231,7 @@ int multi_upload(sbq_ctx* c) {
          ch->model_emp = c->model_emp;
          ch->model_read_len = c->model_read_len;
          ch->have_model = c->have_model;
+         ch->raw_mass_mode = c->raw_mass_mode;
       }
       const int rcr = multi_for_each(c, [&](int i) { return sbq_upload(m.child[i]); });
       if (rcr) return rcr;

@@ -15,6 +15,7 @@
 //                      (class, code-blind feature list): the reference keeps the members in a std::set under a comparator that
 //                      ignores the op code, so of several equivalent hits only the first inserted one counts
 //   raw_mass_kernel    class mass = sum of the surviving members' masses (float), member count
+//   raw_member_*       RB_MASS_ANY only: the class mass summed in set order instead (scatter, sort, one thread per class)
 //   raw_nnz_kernel / raw_fill_kernel   CSR rows (classes) x columns (isoforms, ascending), integer counts (int)mass, and per
 //                      entry the descriptor of the class under the isoform (segment lengths of the span, implicit-segment mask,
 //                      L_t: ExonBin::bin_under_iso, include/isoform.h:363-411) that weights_kernel turns into alpha. The
@@ -22,11 +23,13 @@
 //                      segment lengths in the descriptor pool (4 B per spanned segment, no per-entry limit)
 //
 // Everything is order-free, so atomics are safe: class ids come from a prefix sum, set semantics from atomicMin on the hit
-// index, and the float mass sum is EXACT (hence independent of the order the reference's std::set imposes) as long as every
-// mass is a multiple of 1/2 and a class holds less than 2^23 of it - true for every BAM read without
-// --allow-multimapped-hits (collapse masses are multiplicities of 0.5 + 0.5). The kernels flag what they cannot reproduce
-// bit-exactly (fractional masses, a 64-bit hash collision) or what the reference asserts on (a class coordinate outside the
-// isoform's segments), and the upload is refused with SBQ_ERR_UNSUPPORTED: the caller then uses the host builder.
+// index. In the default mass mode (RB_MASS_HALVES) the float mass sum is EXACT (hence independent of the order the reference's
+// std::set imposes) as long as every mass is a multiple of 1/2 and a class holds less than 2^23 of it - true for every BAM read
+// without --allow-multimapped-hits (collapse masses are multiplicities of 0.5 + 0.5). With 1/NH masses the float sum depends on
+// the order, so RB_MASS_ANY sorts every class's survivors in set order and adds them in that order. The kernels flag what they
+// cannot reproduce bit-exactly (in the default mode a mass that is not a multiple of 1/2; in RB_MASS_ANY a NaN, infinite or
+// negative mass; a 64-bit hash collision), a class mass (int) cannot hold, or what the reference asserts on (a class coordinate
+// outside the isoform's segments), and the upload is refused with SBQ_ERR_UNSUPPORTED: the caller then uses the host builder.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -34,12 +37,14 @@
 namespace sbq {
 
 enum : int { RB_FLAG_COLLISION = 2, RB_FLAG_MASS = 4, RB_FLAG_NSEG = 8 };
+enum : int { RB_MASS_HALVES = 0, RB_MASS_ANY = 1 };   // SBQ_RAW_MASS_HALVES / SBQ_RAW_MASS_ANY
 constexpr unsigned long long RB_EMPTY = 0xffffffffffffffffull;
 
 struct RawBatch {
    int64_t n_hit;
    int32_t n_loci;
    int32_t long_read;
+   int32_t mass_mode;              // RB_MASS_HALVES: order-free atomic sum of multiples of 1/2; RB_MASS_ANY: sum in set order
    // input (device copies of the staged batch)
    const int32_t* hit_locus;       // [H]
    const int64_t* hit_feat_ptr;    // [H + 1]
@@ -184,7 +189,11 @@ __global__ void __launch_bounds__(128) raw_hit_kernel(RawBatch b) {
       if (ok) {
          const float m = b.hit_mass[h];
          const float m2 = m * 2.0f;
-         if (!(m >= 0.0f && m < 4194304.0f && m2 == floorf(m2))) atomicOr(b.flags, RB_FLAG_MASS);   // not a multiple of 1/2: the order of the sum would matter
+         if (b.mass_mode == RB_MASS_ANY) {
+            if (!(m >= 0.0f && m <= 3.402823466e38f)) atomicOr(b.flags, RB_FLAG_MASS);                  // NaN, infinite or negative
+         } else if (!(m >= 0.0f && m < 4194304.0f && m2 == floorf(m2))) {
+            atomicOr(b.flags, RB_FLAG_MASS);                     // not a multiple of 1/2: the order of the sum would matter
+         }
       }
    }
 }
@@ -279,8 +288,127 @@ __global__ void __launch_bounds__(256) raw_mass_kernel(RawBatch b) {
          continue;
       }
       const int64_t cg = b.loc_cls_off[l] + b.hit_class[h];
-      atomicAdd(&b.class_mass[cg], b.hit_mass[h]);               // exact: multiples of 1/2, class total checked against 2^23 below
+      if (b.mass_mode == RB_MASS_HALVES) atomicAdd(&b.class_mass[cg], b.hit_mass[h]);   // exact: multiples of 1/2, class total checked against 2^23 below
       atomicAdd(&b.class_nfrag[cg], 1);
+   }
+}
+
+// ---- RB_MASS_ANY: the class mass is the float sum of the surviving members in std::set<Contig> order (ExonBin::read_count,
+// include/isoform.h:285-296). The survivors are scattered into per-class segments, the whole array is sorted by (global class,
+// Contig::operator<) - a bitonic sort of 1024-element tiles in shared memory, then merge-path passes that double the sorted
+// runs - and one thread per class adds the masses in that order. Survivors of one class are pairwise non-equivalent, so the
+// order is total and does not depend on the scatter. An element is (k0, k1, hit): k0 = global class, k1 = (ref_id, offset of the
+// first feature), which decide most comparisons; the full feature lists break the remaining ties.
+constexpr int RB_SORT_TILE = 1024;
+constexpr int RB_MERGE_PER_THREAD = 8;
+
+// Contig::operator< (src/contig.cpp:342-347): ref_id, then the feature lists lexicographically by (offset, len), op codes
+// ignored; a proper prefix sorts first
+__device__ __forceinline__ bool rb_contig_less(const RawBatch& b, int64_t x, int64_t y) {
+   if (x < 0 || y < 0) return false;                             // tile padding
+   const int rx = b.hit_ref[x], ry = b.hit_ref[y];
+   if (rx != ry) return rx < ry;
+   const int64_t x0 = b.hit_feat_ptr[x], y0 = b.hit_feat_ptr[y];
+   const int64_t nx = b.hit_feat_ptr[x + 1] - x0, ny = b.hit_feat_ptr[y + 1] - y0;
+   for (int64_t k = 0; k < nx && k < ny; ++k) {
+      const uint32_t ox = b.hf_off[x0 + k], oy = b.hf_off[y0 + k];
+      if (ox != oy) return ox < oy;
+      const uint32_t lx = b.hf_len[x0 + k], ly = b.hf_len[y0 + k];
+      if (lx != ly) return lx < ly;
+   }
+   return nx < ny;
+}
+
+__device__ __forceinline__ bool rb_member_less(const RawBatch& b, unsigned long long a0, unsigned long long a1, int64_t ah, unsigned long long b0,
+                                               unsigned long long b1, int64_t bh) {
+   if (a0 != b0) return a0 < b0;
+   if (a1 != b1) return a1 < b1;
+   return rb_contig_less(b, ah, bh);
+}
+
+// survivors (as raw_mass_kernel finds them) into their class's segment [member_off[c], member_off[c + 1]), in any order
+__global__ void __launch_bounds__(256) raw_member_scatter_kernel(RawBatch b, const int64_t* __restrict__ member_off, int32_t* __restrict__ cursor,
+                                                                 unsigned long long* __restrict__ k0, unsigned long long* __restrict__ k1, int64_t* __restrict__ hit) {
+   for (int64_t h = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; h < b.n_hit; h += (int64_t)gridDim.x * blockDim.x) {
+      if (!b.valid[h]) continue;
+      const int l = b.hit_locus[h];
+      if (b.loc_hit_off[l] + b.min2[b.loc_tab_off[l] + b.slot2[h]] != h) continue;
+      const int64_t cg = b.loc_cls_off[l] + b.hit_class[h];
+      const int64_t k = member_off[cg] + atomicAdd(&cursor[cg], 1);
+      k0[k] = (unsigned long long)cg;
+      k1[k] = (unsigned long long)((uint32_t)b.hit_ref[h] ^ 0x80000000u) << 32 | b.hf_off[b.hit_feat_ptr[h]];
+      hit[k] = h;
+   }
+}
+
+// every 1024-element tile of the n = *n_member elements sorted in place (bitonic network, padded with elements that sort last)
+__global__ void __launch_bounds__(RB_SORT_TILE / 2) raw_member_tile_sort_kernel(RawBatch b, const int64_t* __restrict__ n_member, unsigned long long* __restrict__ k0,
+                                                                              unsigned long long* __restrict__ k1, int64_t* __restrict__ hit) {
+   __shared__ unsigned long long s0[RB_SORT_TILE], s1[RB_SORT_TILE];
+   __shared__ int64_t sh[RB_SORT_TILE];
+   const int64_t n = *n_member;
+   const int64_t base = (int64_t)blockIdx.x * RB_SORT_TILE;
+   if (base >= n) return;
+   for (int e = threadIdx.x; e < RB_SORT_TILE; e += blockDim.x) {
+      const bool in = base + e < n;
+      s0[e] = in ? k0[base + e] : ~0ull;
+      s1[e] = in ? k1[base + e] : ~0ull;
+      sh[e] = in ? hit[base + e] : -1;
+   }
+   __syncthreads();
+   for (int k = 2; k <= RB_SORT_TILE; k <<= 1) {
+      for (int j = k >> 1; j > 0; j >>= 1) {
+         const int t = threadIdx.x;
+         const int e = 2 * t - (t & (j - 1)), p = e + j;
+         const bool asc = (e & k) == 0;
+         if (asc ? rb_member_less(b, s0[p], s1[p], sh[p], s0[e], s1[e], sh[e]) : rb_member_less(b, s0[e], s1[e], sh[e], s0[p], s1[p], sh[p])) {
+            const unsigned long long a0 = s0[e], a1 = s1[e];
+            const int64_t ah = sh[e];
+            s0[e] = s0[p]; s1[e] = s1[p]; sh[e] = sh[p];
+            s0[p] = a0; s1[p] = a1; sh[p] = ah;
+         }
+         __syncthreads();
+      }
+   }
+   for (int e = threadIdx.x; e < RB_SORT_TILE && base + e < n; e += blockDim.x) {
+      k0[base + e] = s0[e];
+      k1[base + e] = s1[e];
+      hit[base + e] = sh[e];
+   }
+}
+
+// one merge-path pass: sorted runs of `width` elements, pairwise merged into runs of 2 width (a run without a partner is copied)
+__global__ void __launch_bounds__(256) raw_member_merge_kernel(RawBatch b, const int64_t* __restrict__ n_member, int64_t width,
+                                                               const unsigned long long* __restrict__ i0, const unsigned long long* __restrict__ i1, const int64_t* __restrict__ ih,
+                                                               unsigned long long* __restrict__ o0, unsigned long long* __restrict__ o1, int64_t* __restrict__ oh) {
+   const int64_t n = *n_member;
+   for (int64_t out = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * RB_MERGE_PER_THREAD; out < n;
+        out += (int64_t)gridDim.x * blockDim.x * RB_MERGE_PER_THREAD) {
+      const int64_t start = out / (2 * width) * (2 * width);
+      const int64_t a = start, na = min(width, n - start), bb = start + na, nb = min(width, n - bb);
+      const int64_t diag = out - start;
+      int64_t lo = max((int64_t)0, diag - nb), hi = min(diag, na);
+      while (lo < hi) {                                          // smallest i with B[diag - 1 - i] < A[i]: A[0, i) and B[0, diag - i) come first
+         const int64_t mid = (lo + hi) >> 1, y = bb + diag - 1 - mid;
+         if (rb_member_less(b, i0[y], i1[y], ih[y], i0[a + mid], i1[a + mid], ih[a + mid])) hi = mid; else lo = mid + 1;
+      }
+      int64_t x = a + lo, y = bb + (diag - lo);
+      const int64_t xe = a + na, ye = bb + nb;
+      const int64_t end = min(out + RB_MERGE_PER_THREAD, start + na + nb);
+      for (int64_t o = out; o < end; ++o) {
+         const bool take_b = x == xe || (y < ye && rb_member_less(b, i0[y], i1[y], ih[y], i0[x], i1[x], ih[x]));
+         const int64_t s = take_b ? y++ : x++;
+         o0[o] = i0[s]; o1[o] = i1[s]; oh[o] = ih[s];
+      }
+   }
+}
+
+// one thread per class: float sum in set order, round to nearest at every step like the reference's `sum += mass`
+__global__ void __launch_bounds__(256) raw_member_sum_kernel(RawBatch b, int64_t n_class, const int64_t* __restrict__ member_off, const int64_t* __restrict__ hit) {
+   for (int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; c < n_class; c += (int64_t)gridDim.x * blockDim.x) {
+      float s = 0.0f;
+      for (int64_t k = member_off[c]; k < member_off[c + 1]; ++k) s = __fadd_rn(s, b.hit_mass[hit[k]]);
+      b.class_mass[c] = s;
    }
 }
 
@@ -320,7 +448,8 @@ __global__ void __launch_bounds__(256) raw_nnz_kernel(RawBatch b, int64_t n_clas
       }
       b.class_nnz[c] = n;
       b.class_nseg[c] = nseg;
-      if (!(b.class_mass[c] < 8388608.0f)) atomicOr(b.flags, RB_FLAG_MASS);
+      // halves: the atomic sum is exact below 2^23; any: (int)mass is defined below 2^31
+      if (!(b.class_mass[c] < (b.mass_mode == RB_MASS_ANY ? 2147483648.0f : 8388608.0f))) atomicOr(b.flags, RB_FLAG_MASS);
    }
 }
 

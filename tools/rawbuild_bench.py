@@ -6,13 +6,16 @@ Batches:
          the human-shaped short-read case, where every hit touches at most 16 segments and every class spans at most 32
   long   200 full-length long-read loci (40-exon genes, one 1500 bp read per fragment), long-read mode: every class touches
          more than 16 segments
+  multimapped  the short batch with every mass m replaced by m / NH (NH seeded from 2..8), as --allow-multimapped-hits gives,
+         uploaded in SBQ_RAW_MASS_ANY mode: class masses summed in the reference's set order on the device
 
   python tools/rawbuild_bench.py --lib new=strawberry_b200/libsbq.so --lib parent=/path/to/parent/strawberry_b200/libsbq.so --out DIR
       every upload leg runs in a child process of its own (SBQ_LIB_PATH selects the library, and the strawberry_b200 package
       next to it is imported when there is one); the legs alternate between the
       libraries for --rounds rounds, each leg times --uploads uploads of the same batch after --warmup untimed ones
       (median and spread of the stats' upload_ms / weights_ms and of the host wall time of sbq_upload); the short-read tables
-      of every library are checked equal to the first one's. A library that refuses the long-read batch is reported as such.
+      of every library are checked equal to the first one's. A library that refuses a batch (the long-read one, or the
+      multimapped one when it has no SBQ_RAW_MASS_ANY) is reported as such.
   python tools/rawbuild_bench.py --shapes
       no GPU: the device memory the descriptors of both batches take, old fixed layout ([H][16] coordinates, 32-slot pool per
       CSR entry) against the variable-length one, counted from the host builder's tables.
@@ -28,6 +31,7 @@ import tempfile
 
 import numpy as np
 
+KINDS = ("short", "long", "multimapped")
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -37,11 +41,14 @@ def make_batch(kind):
     import locusgen
     from strawberry_b200 import builder
     loci = []
-    if kind == "short":
+    if kind in ("short", "multimapped"):
+        rng = np.random.default_rng(30_000)
         for seed in range(4000):
             isoforms, hits, _ = locusgen.random_locus(10_000 + seed)
+            if kind == "multimapped":
+                hits = [(m / float(nh), l, r) for (m, l, r), nh in zip(hits, rng.integers(2, 9, len(hits)))]
             loci.append(([locusgen.transcript_features(ex) for ex in isoforms], [(m, builder.pair_features(l, r)) for m, l, r in hits]))
-        return dict(loci=loci, read_len=50, mean=220.0, sd=40.0, long_read=False)
+        return dict(loci=loci, read_len=50, mean=220.0, sd=40.0, long_read=False, mass_any=kind == "multimapped")
     for seed in range(200):
         rng = np.random.default_rng(20_000 + seed)
         isoforms = locusgen.make_gene(rng, 40, 6, exon_len=(40, 160), intron_len=(100, 600))
@@ -60,6 +67,11 @@ def child(batch_path, uploads, warmup, dump):
     bt = pickle.load(open(batch_path, "rb"))
     q = api.Quantifier(device=0)
     q.set_insert_model(builder.Model.normal(bt["mean"], bt["sd"]), bt["read_len"])
+    if bt.get("mass_any"):
+        if not hasattr(builder, "set_raw_mass_mode"):
+            print(json.dumps(dict(refused=api.SBQ_ERR_UNSUPPORTED, message="this library has no sbq_set_raw_mass_mode")))
+            return
+        builder.set_raw_mass_mode(q, builder.RAW_MASS_ANY)
     for tfe, hl in bt["loci"]:
         builder.submit_raw(q, tfe, hl, read_len=bt["read_len"], long_read=bt["long_read"])
     up, wt, wall = [], [], []
@@ -141,13 +153,13 @@ def main():
                                   capture_output=True, text=True).stdout.strip().splitlines()[:1], legs=[])
     with tempfile.TemporaryDirectory() as tmp:
         paths = {}
-        for kind in ("short", "long"):
+        for kind in KINDS:
             paths[kind] = os.path.join(tmp, f"{kind}.pkl")
             pickle.dump(make_batch(kind), open(paths[kind], "wb"))
         timings = {(n, k): dict(upload_ms=[], weights_ms=[], wall_ms=[], per_leg_median_upload_ms=[]) for n, _ in libs for k in paths}
         refused = {}
         for r in range(a.rounds):
-            for kind in ("short", "long"):
+            for kind in KINDS:
                 for name, path in libs:
                     dump = os.path.join(tmp, f"{name}.npz") if kind == "short" and r == 0 else "-"
                     env = dict(os.environ, SBQ_LIB_PATH=os.path.abspath(path))
