@@ -4,6 +4,7 @@ size-independent properties."""
 import numpy as np
 import pytest
 
+import cluster_paths
 from strawberry_b200 import synth
 from util import assert_matches_oracle, load_golden, theta_close
 
@@ -43,8 +44,17 @@ def test_golden_vectors_from_the_reference(q, oracle_mod):
     assert ok.all(), worst
 
 
+@pytest.fixture(scope="module")
+def golden_capped():
+    """The golden batch after 1, 2 and 5 EM steps, restated in long double (tests/cluster_paths.py)."""
+    b, *_ = load_golden()
+    return {m: cluster_paths.batch_em_longdouble(b, max_iter=m) for m in (1, 2, 5)}
+
+
 @pytest.mark.parametrize("tier,cluster", [(0, 0), (1, 0), (2, 1), (2, 2), (2, 4), (2, 8), (2, 16), (3, 0)])
-def test_every_tier_matches_the_oracle(q, oracle_mod, tier, cluster):
+def test_every_tier_matches_the_oracle(q, oracle_mod, golden_capped, tier, cluster):
+    """Converged, against the oracle at the parity bar; and capped at 1, 2 and 5 EM steps, against the long-double restatement at
+    cluster_paths.CAPPED_REL (a bar the converged check is far too loose to replace: see tests/test_gpu_cluster_paths.py)."""
     b, *_ = load_golden()
     ora = oracle_mod.quantify_batch(b, b["total_mapped_reads"])
     res = run_gpu(q, b, tier, cluster)
@@ -54,6 +64,12 @@ def test_every_tier_matches_the_oracle(q, oracle_mod, tier, cluster):
         assert st["loci_grid"] > 0
     if tier == 2:
         assert st["loci_cta"] > 0
+    for m, ld in golden_capped.items():
+        capped = run_gpu(None, b, tier, cluster, max_iter=m)
+        assert np.array_equal(capped["status"], ld["status"]) and np.array_equal(capped["iters"], ld["iters"]), m
+        ok, worst = cluster_paths.theta_close_ld(capped["theta"], ld["theta"], b, cluster_paths.CAPPED_REL)
+        print(f"capped worst ratio: golden tier {tier} cluster {cluster} max_iter {m}: {worst:.3e}")
+        assert ok.all(), (m, worst)
 
 
 def test_human_shaped_sample_matches_oracle(q, oracle_mod):
