@@ -69,7 +69,7 @@ struct PinnedVec {
 };
 
 struct LaunchClass {      // one kernel launch of the cluster tier
-   int cs, lpr;           // lpr doubles as the thread count of the launch (CL_NT or CL_NT_SMALL)
+   int cs, nt;            // cluster size, threads per CTA
    std::vector<int32_t> loci;
    int max_iso = 0;
    size_t max_slice = 0;  // estimated bytes of the largest per-CTA resident CSR slice
@@ -392,7 +392,7 @@ int plan(sbq_ctx* c) {
          lc->max_slice = std::max(lc->max_slice, slice);
          // shared memory of the launch = the largest need of its loci (the need is not monotone in T: the exchange area of a
          // narrow locus in a big cluster, CS x T, can exceed that of a wide one, 2T)
-         lc->smem = std::max(lc->smem, cluster_class_smem((int)T, slice, lc->lpr, cs));
+         lc->smem = std::max(lc->smem, cluster_class_smem((int)T, slice, lc->nt, cs));
       }
    }
    auto by_size = [&](int32_t a, int32_t b) { return nnz_of[a] != nnz_of[b] ? nnz_of[a] > nnz_of[b] : a < b; };
@@ -431,7 +431,7 @@ int plan(sbq_ctx* c) {
    }
    for (auto& lc : tmp) {
       std::sort(lc.loci.begin(), lc.loci.end(), by_size);
-      if (cluster_stream_groups(lc.max_iso, SMEM_CAP, lc.lpr, 1, 0) <= 0)
+      if (cluster_stream_groups(lc.max_iso, SMEM_CAP, lc.nt, 1, 0) <= 0)
          return fail(c, SBQ_ERR_UNSUPPORTED, "locus with %d isoforms does not fit the cluster tier", lc.max_iso);
       c->classes.push_back(std::move(lc));
    }
@@ -505,9 +505,9 @@ int set_kernel_attrs(sbq_ctx* c, K kernel, size_t smem, bool nonportable) {
    return SBQ_SUCCESS;
 }
 
-template <int NT, int NCACHE, int MINB>
+template <int NT>
 int launch_cluster_class_nt(sbq_ctx* c, const LaunchClass& lc, cudaStream_t st) {
-   auto kernel = em_cluster_kernel<NT, NCACHE, MINB>;
+   auto kernel = em_cluster_kernel<NT>;
    int rc = set_kernel_attrs(c, kernel, lc.smem, lc.cs > 8);
    if (rc) return rc;
    cudaLaunchConfig_t cfg{};
@@ -1225,9 +1225,9 @@ int sbq_solve(sbq_ctx* c, int64_t total_mapped_reads) {
       if (pending) CU(cudaStreamWaitEvent(ss, (i < N_SIDE_STREAMS && c->class_ready[i]) ? c->ev_class_ready[i] : c->ev[1], 0));
       LaunchTimer& t = c->lt[1 + i % N_SIDE_STREAMS];
       CU(cudaEventRecord(t.e0, ss));
-      // register caps (launch bounds) follow the CTAs-per-SM targets of the buckets
-      int rc = lc.lpr == 64 ? launch_cluster_class_nt<64, 0, 8>(c, lc, ss) : lc.lpr == 128 ? launch_cluster_class_nt<128, 0, 4>(c, lc, ss) :
-               lc.lpr == 256 ? launch_cluster_class_nt<256, 0, 2>(c, lc, ss) : launch_cluster_class_nt<CL_NT, 0, 1>(c, lc, ss);
+      // one arm per thread count of BUCKET_NT
+      int rc = lc.nt == 64 ? launch_cluster_class_nt<64>(c, lc, ss) : lc.nt == 128 ? launch_cluster_class_nt<128>(c, lc, ss) :
+               launch_cluster_class_nt<512>(c, lc, ss);
       if (rc) return rc;
       CU(cudaEventRecord(t.e1, ss));
       t.used = true;
@@ -1293,7 +1293,7 @@ int sbq_solve(sbq_ctx* c, int64_t total_mapped_reads) {
    for (size_t i = 0; i < c->classes.size(); ++i) {
       LaunchTimer& t = c->lt[1 + i % N_SIDE_STREAMS];
       CU(cudaEventElapsedTime(&ms, t.e0, t.e1));
-      add_stat(2, c->classes[i].cs, c->classes[i].lpr, c->classes[i].loci, ms, t.e0);
+      add_stat(2, c->classes[i].cs, c->classes[i].nt, c->classes[i].loci, ms, t.e0);
    }
    c->stats.kernel_launches = launches;
    c->solved = true;

@@ -365,8 +365,7 @@ em_warp_kernel(DevParams p, const int32_t* __restrict__ list, int n_list, int ma
 // row pass -> fixed-order sum over groups -> partial theta' exchanged through distributed shared
 // memory (one cluster barrier, double-buffered) -> every CTA forms the same theta' and norm.
 // --------------------------------------------------------------------------------------------
-constexpr int CL_NT = 512;           // threads per CTA of the cluster tier (small single-CTA loci use CL_NT_SMALL)
-constexpr int CL_NT_SMALL = 128;
+constexpr int CL_NT = 512;           // threads per CTA of the cluster tier (small single-CTA loci use 64 or 128, see BUCKET_NT in sbq.cu)
 constexpr int CL_LPR_STREAM = 32;    // lanes per row of the streaming fallback
 
 // Exchange of the partial theta' inside a cluster, two forms. All-to-all: every CTA broadcasts its row of T partials to all peers and
@@ -417,6 +416,40 @@ __host__ __device__ inline size_t cluster_class_smem(int max_iso, size_t slice_b
 // per-CTA resident slice estimate with 12 % slack for the row-granular split
 __host__ __device__ inline size_t cluster_slice_estimate(long long nnz, long long R, int T, int cs) {
    return (size_t)(1.12 * (double)cluster_resident_bytes((size_t)(nnz / cs + 1), (size_t)(R / cs + 1), T)) + 512;
+}
+
+// The path one CTA of em_cluster_kernel takes, from the locus (T, cluster size, slice estimate), the launch (threads, dynamic
+// shared memory) and the CTA's own share of the rows (nrows, non-zeros nnz_c, whether a row is longer than T).
+struct ClusterCtaPath {
+   bool resident;       // the slice sits in shared memory (else it streams from L2 with G accumulator groups)
+   bool csc_in_smem;    // ... with all of its CSC index; otherwise the first n_ent_s entries of the index, the rest in L2
+   unsigned n_ent_s;
+   int G;
+   bool row_slots;      // balanced E-step (nrows <= NT), else four rows per thread
+   bool col_slots;      // balanced M-step (T <= NT), else one thread per column
+   bool a2a;            // all-to-all exchange, else the owner form with B columns per CTA
+   int B;
+};
+__host__ __device__ inline ClusterCtaPath cluster_cta_path(int T, int cs, int nt, int nrows, unsigned nnz_c, bool too_long, size_t slice_est,
+                                                           unsigned smem_launch) {
+   ClusterCtaPath c;
+   // this locus' own shared-memory budget (<= what the launch provides: the class maximum of the same expression)
+   const size_t cls = cluster_class_smem(T, slice_est, nt, cs), smem_bytes = smem_launch < cls ? smem_launch : cls;
+   const size_t used = cluster_fixed_doubles(T, cs, slice_est) * sizeof(double);
+   const size_t csr = cluster_resident_csr_bytes(nnz_c, (size_t)nrows, T);
+   // 16-bit positions and rows; the diagonal table has room for rows of up to T entries (a valid row has no more)
+   const bool small_idx = (uint64_t)nnz_c + (uint64_t)T <= 65535u && nrows <= 65535 && !too_long;
+   c.csc_in_smem = small_idx && used + cluster_resident_bytes(nnz_c, (size_t)nrows, T) <= smem_bytes;
+   c.resident = small_idx && used + csr <= smem_bytes;
+   c.n_ent_s = 0;
+   if (c.csc_in_smem) c.n_ent_s = nnz_c;
+   else if (c.resident) c.n_ent_s = (unsigned)(nnz_c < (smem_bytes - used - csr) / 4 ? nnz_c : (smem_bytes - used - csr) / 4);
+   c.G = c.resident ? 0 : cluster_stream_groups(T, smem_bytes, nt, cs, slice_est);
+   c.row_slots = c.resident && nrows <= nt;
+   c.col_slots = c.resident && T <= nt;
+   c.a2a = cluster_a2a(T, cs, slice_est);
+   c.B = c.a2a ? cluster_a2a_stride(T) : (T + cs - 1) / cs;
+   return c;
 }
 
 // Row accessor of one CTA's slice streamed from global/L2 (fallback when the slice does not fit shared memory).
@@ -511,19 +544,8 @@ struct ResidentSlice {
    unsigned nnz, npos;     // entries, and positions of al/col (entries + one padding slot per diagonal at most)
 };
 
-// lanes per row / column: the largest power of two <= 32 that still gives every item its own lane group
-#ifndef SBQ_MIN_LANES
-#define SBQ_MIN_LANES 1
-#endif
-__device__ __forceinline__ int lanes_for(int items, int nt) {
-   int l = 32;
-   while (l > SBQ_MIN_LANES && (long long)items * l > nt) l >>= 1;
-   return l;
-}
-
 // E-step on the resident slice: d_s = sum_k alpha_k th[col_k]  ->  r_s = n_s / d_s   (one division per row).
-// lpr lanes share a row and take its entries in interleaved groups of four.
-// E-step, generic form for slices with more rows than threads, one lane per row: four rows per thread at a time
+// Generic form for slices with more rows than threads, one lane per row: four rows per thread at a time
 // (rows tid, tid + NT, ... are sorted by descending length, so the first of the four is the longest).
 template <int NT>
 __device__ __forceinline__ void resident_e_pass_rows4(const ResidentSlice& S, const double* th, int& zero) {
@@ -576,100 +598,33 @@ __device__ __forceinline__ void resident_e_pass_rows4(const ResidentSlice& S, co
    }
 }
 
-template <int NT>
-__device__ __forceinline__ void resident_e_pass(const ResidentSlice& S, const double* th, int lpr, int& zero) {
-   const int tid = threadIdx.x, g = tid / lpr, lg = tid % lpr, par = NT / lpr;
-   for (int base = 0; base < S.nrows; base += par) {
-      const int s = base + g;
-      int ne = -1, len = 0;
-      if (s < S.nrows) {
-         ne = S.ne[s];
-         if (ne >= 0) len = S.rlen[s];
-      }
-      double d0 = 0.0, d1 = 0.0;
-      int k = 4 * lg;
-      // eight entries per trip while two full groups of four remain (sixteen loads in flight per lane)
-      for (; k + 4 * lpr + 4 <= len; k += 8 * lpr) {
-         const uint4 o = *reinterpret_cast<const uint4*>(S.jd + k);
-         const uint4 q = *reinterpret_cast<const uint4*>(S.jd + k + 4 * lpr);
-         const unsigned p0 = o.x + s, p1 = o.y + s, p2 = o.z + s, p3 = o.w + s;
-         const unsigned p4 = q.x + s, p5 = q.y + s, p6 = q.z + s, p7 = q.w + s;
-         const int c0 = S.col[p0], c1 = S.col[p1], c2 = S.col[p2], c3 = S.col[p3];
-         const int c4 = S.col[p4], c5 = S.col[p5], c6 = S.col[p6], c7 = S.col[p7];
-         const double a0 = S.al[p0], a1 = S.al[p1], a2 = S.al[p2], a3 = S.al[p3];
-         const double a4 = S.al[p4], a5 = S.al[p5], a6 = S.al[p6], a7 = S.al[p7];
-         const double t0 = th[c0], t1 = th[c1], t2 = th[c2], t3 = th[c3];
-         const double t4 = th[c4], t5 = th[c5], t6 = th[c6], t7 = th[c7];
-         d0 += a0 * t0;
-         d1 += a1 * t1;
-         d0 += a2 * t2;
-         d1 += a3 * t3;
-         d0 += a4 * t4;
-         d1 += a5 * t5;
-         d0 += a6 * t6;
-         d1 += a7 * t7;
-      }
-      for (; k < len; k += 4 * lpr) {                  // last groups: entries past the end read the padding slot
-         const uint4 o = *reinterpret_cast<const uint4*>(S.jd + k);
-         const bool v1 = k + 1 < len, v2 = k + 2 < len, v3 = k + 3 < len;
-         const unsigned p0 = o.x + s, p1 = v1 ? o.y + s : S.npos, p2 = v2 ? o.z + s : S.npos, p3 = v3 ? o.w + s : S.npos;
-         const double a0 = S.al[p0], a1 = S.al[p1], a2 = S.al[p2], a3 = S.al[p3];
-         const int c0 = S.col[p0], c1 = S.col[p1], c2 = S.col[p2], c3 = S.col[p3];
-         const double t0 = a0 * th[c0], t1 = a1 * th[c1], t2 = a2 * th[c2], t3 = a3 * th[c3];
-         d0 += t0;
-         d1 += v1 ? t1 : 0.0;
-         d0 += v2 ? t2 : 0.0;
-         d1 += v3 ? t3 : 0.0;
-      }
-      double d = d0 + d1;
-      for (int o = lpr >> 1; o > 0; o >>= 1) d += __shfl_xor_sync(0xffffffffu, d, o);
-      if (s < S.nrows && lg == 0) {
-         double r = 0.0;
-         if (ne >= 0) {
-            if (d == 0) zero = 1; else r = (double)ne / d;
-         }
-         S.r[s] = r;
-      }
-   }
-}
-
 // M-step on the resident slice through the CSC index: out_j = scale_j * sum_{k in column j} alpha_k r_row(k).
-// Fixed lane assignment and reduction shape -> deterministic, no accumulators, no atomics.
-// Generic form (any T): lpc lanes per column, index entries read from memory.
+// Fixed lane assignment and summation order -> deterministic, no accumulators, no atomics.
+// Generic form (any T): one thread per column, index entries read from memory eight at a time.
 template <int NT, typename Emit>
-__device__ __forceinline__ void resident_col_pass(const ResidentSlice& S, const double* scale, const Emit& emit, int lpc) {
-   const int tid = threadIdx.x, g = tid / lpc, lg = tid % lpc, par = NT / lpc;
+__device__ __forceinline__ void resident_col_pass(const ResidentSlice& S, const double* scale, const Emit& emit) {
    const unsigned pad = ((unsigned)S.nrows << 16) | S.npos;
-   for (int base = 0; base < S.T; base += par) {
-      const int j = base + g;
+   for (int j = threadIdx.x; j < S.T; j += NT) {
       double sum = 0.0;
-      if (j < S.T) {
-         const unsigned x1 = S.cp[j + 1];
-         for (unsigned x = S.cp[j] + lg; x < x1; x += 8 * lpc) {
-            unsigned e[8];
+      const unsigned x1 = S.cp[j + 1];
+      for (unsigned x = S.cp[j]; x < x1; x += 8) {
+         unsigned e[8];
 #pragma unroll
-            for (int u = 0; u < 8; ++u) e[u] = (x + u * lpc < x1) ? S.get_ent(x + u * lpc) : pad;
+         for (int u = 0; u < 8; ++u) e[u] = (x + u < x1) ? S.get_ent(x + u) : pad;
 #pragma unroll
-            for (int u = 0; u < 8; ++u) sum += S.al[e[u] & 0xffffu] * S.r[e[u] >> 16];
-         }
+         for (int u = 0; u < 8; ++u) sum += S.al[e[u] & 0xffffu] * S.r[e[u] >> 16];
       }
-      for (int o = lpc >> 1; o > 0; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
-      if (j < S.T && lg == 0) *emit.ptr(j) = scale ? scale[j] * sum : sum;
+      *emit.ptr(j) = scale ? scale[j] * sum : sum;
    }
 }
 
 // Balanced form (items <= threads): every thread owns one (item, lane) slot for the whole solve. Rows and columns get
-// a power-of-two number of lanes in proportion to their length, so that every lane walks about the same number of
-// entries. With NCACHE > 0 a column lane keeps its first NCACHE index entries in registers (for slices whose CSC index
-// does not fit shared memory and would otherwise be re-read from L2 every iteration).
-template <int NCACHE>
+// a power-of-two number of lanes in proportion to their length, so that every lane walks about the same number of entries.
 struct ColSlot {
    int j;                      // column, or -1 for an idle thread
    int q, lanes, wl;           // this thread is lane q of `lanes`; wl = largest group of the warp
-   unsigned x_tail, x1;        // index entries beyond the cached ones: x_tail, x_tail + lanes, ... < x1
-   int ncache;                 // cached entries that are real (the rest point at the zero padding)
+   unsigned x0, x1;            // index entries of this lane: x0, x0 + lanes, ... < x1
    double* out;                // where lane 0 of the column stores the result
-   unsigned e[NCACHE > 0 ? NCACHE : 1];
 };
 struct RowSlot {
    int s;                      // sorted row, or -1 for an idle thread
@@ -828,35 +783,20 @@ __device__ __forceinline__ void slot_e_pass(const ResidentSlice& S, const RowSlo
    }
 }
 
-template <int NCACHE>
-__device__ __forceinline__ void slot_col_pass(const ResidentSlice& S, const ColSlot<NCACHE>& cs, const double* scale) {
+__device__ __forceinline__ void slot_col_pass(const ResidentSlice& S, const ColSlot& cs, const double* scale) {
    double s0 = 0.0, s1 = 0.0;
-   if (NCACHE > 0) {
+   const unsigned pad = ((unsigned)S.nrows << 16) | S.npos;
+   for (unsigned x = cs.x0; x < cs.x1; x += 8 * cs.lanes) {
+      unsigned e[8];
 #pragma unroll
-      for (int u0 = 0; u0 < NCACHE; u0 += 8) {
-         if (u0 < cs.ncache) {
+      for (int u = 0; u < 8; ++u) e[u] = (x + u * cs.lanes < cs.x1) ? S.get_ent(x + u * cs.lanes) : pad;
+      double a[8], r[8];
 #pragma unroll
-            for (int u = u0; u < u0 + 8; u += 2) {
-               s0 += S.al[cs.e[u] & 0xffffu] * S.r[cs.e[u] >> 16];
-               s1 += S.al[cs.e[u + 1] & 0xffffu] * S.r[cs.e[u + 1] >> 16];
-            }
-         }
-      }
-   }
-   if (cs.x_tail < cs.x1) {                                   // the (rest of the) index comes from memory
-      const unsigned pad = ((unsigned)S.nrows << 16) | S.npos;
-      for (unsigned x = cs.x_tail; x < cs.x1; x += 8 * cs.lanes) {
-         unsigned e[8];
+      for (int u = 0; u < 8; ++u) { a[u] = S.al[e[u] & 0xffffu]; r[u] = S.r[e[u] >> 16]; }
 #pragma unroll
-         for (int u = 0; u < 8; ++u) e[u] = (x + u * cs.lanes < cs.x1) ? S.get_ent(x + u * cs.lanes) : pad;
-         double a[8], r[8];
-#pragma unroll
-         for (int u = 0; u < 8; ++u) { a[u] = S.al[e[u] & 0xffffu]; r[u] = S.r[e[u] >> 16]; }
-#pragma unroll
-         for (int u = 0; u < 8; u += 2) {
-            s0 += a[u] * r[u];
-            s1 += a[u + 1] * r[u + 1];
-         }
+      for (int u = 0; u < 8; u += 2) {
+         s0 += a[u] * r[u];
+         s1 += a[u + 1] * r[u + 1];
       }
    }
    const double sum = group_sum(s0 + s1, cs.q, cs.lanes, cs.wl);
@@ -886,8 +826,9 @@ struct LocalOut {
    __device__ __forceinline__ double* ptr(int j) const { return out + j; }
 };
 
-template <int NT, int NCACHE, int MINB>
-__global__ void __launch_bounds__(NT, MINB)
+// NT = 64 / 128 / 512 threads: eight / four / one CTA per SM (the register cap follows from it)
+template <int NT>
+__global__ void __launch_bounds__(NT, CL_NT / NT)
 em_cluster_kernel(DevParams p, const int32_t* __restrict__ list, int n_list, unsigned smem_launch) {
    cg::cluster_group cluster = cg::this_cluster();
    const unsigned CS = cluster.num_blocks();
@@ -918,9 +859,6 @@ em_cluster_kernel(DevParams p, const int32_t* __restrict__ list, int n_list, uns
    double* cur = bufA;
    double* nxt = bufB;
 
-   // this locus' own shared-memory budget (<= what the launch provides: the class maximum of the same expression)
-   const unsigned smem_bytes = min(smem_launch, (unsigned)cluster_class_smem(T, slice_est, NT, (int)CS));
-
    // rows of this CTA: split by non-zeros (lower_bound on row_ptr)
    if (tid < 2) {
       const int64_t base = rp[0], nnz = rp[R] - base;
@@ -939,16 +877,12 @@ em_cluster_kernel(DevParams p, const int32_t* __restrict__ list, int n_list, uns
    const int64_t k_a = rp[ra];
    const unsigned nnz_c = (unsigned)(rp[rb] - k_a);
 
-   const size_t used = (size_t)((char*)dyn - (char*)smem);
-   const int lpr = lanes_for(nrows, NT), lpc = lanes_for(T, NT);
    // longest row of the slice: the diagonal table has room for rows of up to T entries (a valid row has no more)
    int too_long = 0;
    for (int i = tid; i < nrows; i += NT) too_long |= (rp[ra + i + 1] - rp[ra + i]) > (int64_t)T;
    too_long = __syncthreads_or(too_long);
-   const bool small_idx = (uint64_t)nnz_c + (uint64_t)T <= 65535u && nrows <= 65535 && !too_long;
+   const ClusterCtaPath path = cluster_cta_path(T, (int)CS, NT, nrows, nnz_c, too_long != 0, slice_est, smem_launch);
    const unsigned npos = nnz_c + (unsigned)T;
-   const bool csc_in_smem = small_idx && used + cluster_resident_bytes(nnz_c, (size_t)nrows, T) <= smem_bytes;
-   const bool resident = small_idx && used + cluster_resident_csr_bytes(nnz_c, (size_t)nrows, T) <= smem_bytes;
    const int jdn = cluster_diag_slots(T);
    ResidentSlice S;
    S.al = dyn;
@@ -960,19 +894,15 @@ em_cluster_kernel(DevParams p, const int32_t* __restrict__ list, int n_list, uns
    S.col = S.rlen + nrows;
    S.ent = (unsigned*)(S.col + npos + 1 + ((npos + 1 + nrows) & 1u));                        // 4-byte aligned
    S.ent_g = p.csc + (size_t)k_a;      // the part of the CSC index that does not fit shared memory lives in global scratch (L2)
-   S.n_ent_s = 0;
-   if (csc_in_smem) S.n_ent_s = nnz_c;
-   else if (resident) S.n_ent_s = (unsigned)min((size_t)nnz_c, (smem_bytes - used - cluster_resident_csr_bytes(nnz_c, (size_t)nrows, T)) / 4);
+   S.n_ent_s = path.n_ent_s;
    S.nrows = nrows; S.T = T; S.nnz = nnz_c; S.npos = npos;
    GlobalRows grows{rp + ra, p.alpha + k_a, p.col + k_a, p.neff + r0 + ra, k_a};
-   const int G = resident ? 0 : cluster_stream_groups(T, smem_bytes, NT, (int)CS, slice_est);
+   const int G = path.G;
    double* acc = dyn;                                           // [G][T] (streaming only)
    const int g32 = tid / CL_LPR_STREAM, lg32 = tid % CL_LPR_STREAM;
    double* my_acc = acc + (size_t)(g32 < G ? g32 : 0) * T;
-   const bool use_slots = resident && T <= NT;            // balanced M-step
-   const bool use_row_slots = resident && nrows <= NT;    // balanced E-step
-   ColSlot<NCACHE> slot;
-   slot.j = -1; slot.q = 0; slot.lanes = 1; slot.wl = 1; slot.x_tail = slot.x1 = 0; slot.ncache = 0; slot.out = part;
+   ColSlot slot;
+   slot.j = -1; slot.q = 0; slot.lanes = 1; slot.wl = 1; slot.x0 = slot.x1 = 0; slot.out = part;
    RowSlot rslot;
    rslot.s = -1; rslot.q = 0; rslot.lanes = 1; rslot.n = 1; rslot.len = 0; rslot.ne = -1;
 
@@ -989,7 +919,7 @@ em_cluster_kernel(DevParams p, const int32_t* __restrict__ list, int n_list, uns
 #endif
    long long tot = 0;
    int kept = 0;
-   if (resident) {
+   if (path.resident) {
       // ---- rows sorted by descending length (ties by row index): bitonic sort of (65535 - len) << 16 | row
       unsigned* keys = (unsigned*)S.al;                                    // scratch: alpha is loaded afterwards
       int P = 1;
@@ -1179,7 +1109,7 @@ em_cluster_kernel(DevParams p, const int32_t* __restrict__ list, int n_list, uns
       __shared__ unsigned s_slot[NT];
       __shared__ int s_lanes[NT];
       __shared__ int s_total;
-      if (use_row_slots) {
+      if (path.row_slots) {
          const unsigned info = assign_row_slots<NT>(S.rlen, nrows, nnz_c, s_slot);
          if (info != 0xffffffffu) {
             const int first = (int)(info & 0xffffu), n = (int)((info >> 16) & 0xffu), L = (int)(info >> 24);
@@ -1197,36 +1127,22 @@ em_cluster_kernel(DevParams p, const int32_t* __restrict__ list, int n_list, uns
          }
       }
       SBQ_STICK(4)
-      if (use_slots) {
+      if (path.col_slots) {
          const int len_j = tid < T ? (int)(S.cp[tid + 1] - S.cp[tid]) : 0;
          const unsigned sl = assign_slots<NT>(T, len_j, nnz_c, s_slot, s_lanes, &s_total);
-         const unsigned pad = ((unsigned)nrows << 16) | npos;
          if (sl != 0xffffffffu) {
             slot.j = (int)(sl & 0xffffu);
             slot.lanes = (int)(sl >> 24);
             slot.q = (int)((sl >> 16) & 0xffu);
-            const unsigned x0 = S.cp[slot.j] + (unsigned)slot.q;
+            slot.x0 = S.cp[slot.j] + (unsigned)slot.q;
             slot.x1 = S.cp[slot.j + 1];
-            slot.x_tail = x0 + (unsigned)NCACHE * slot.lanes;
-            if (NCACHE > 0) {
-#pragma unroll
-               for (int u = 0; u < NCACHE; ++u) {
-                  const unsigned x = x0 + (unsigned)u * slot.lanes;
-                  const bool v = x < slot.x1;
-                  slot.e[u] = v ? S.get_ent(x) : pad;
-                  slot.ncache += v;
-               }
-            }
             slot.out = part + slot.j;
-         } else if (NCACHE > 0) {
-#pragma unroll
-            for (int u = 0; u < NCACHE; ++u) slot.e[u] = pad;
          }
          slot.wl = __reduce_max_sync(0xffffffffu, slot.lanes);
          SBQ_STICK(5)
          slot_col_pass(S, slot, nullptr);                                                     // s_j partial (r = keep flag)
       } else {
-         resident_col_pass<NT>(S, nullptr, LocalOut{part}, lpc);
+         resident_col_pass<NT>(S, nullptr, LocalOut{part});
       }
    } else {
       for (int x = tid; x < G * T; x += NT) acc[x] = 0.0;
@@ -1271,9 +1187,9 @@ em_cluster_kernel(DevParams p, const int32_t* __restrict__ list, int n_list, uns
 #endif
    // ---- exchange area: column j belongs to CTA j / B; every CTA pushes its partial theta'_j to the owner, the owner
    //      adds the CS partials in a fixed shape and pushes theta'_j and theta'_j / s_j back to everyone
-   const bool a2a = cluster_a2a(T, (int)CS, slice_est);
+   const bool a2a = path.a2a;
    const int Tp = cluster_a2a_stride(T);
-   const int B = a2a ? Tp : (T + (int)CS - 1) / (int)CS;
+   const int B = path.B;
    double* stage = part;                       // [CS][B]; all-to-all: [CS][Tp], row r = the partials of CTA r
    double* dsq = a2a ? part + (size_t)CS * Tp : part + T + 16;            // [B] squared changes of the owned columns ([NT / 32] per-warp sums)
    double* flags = a2a ? dsq + 16 : part + 2 * T + 32;                    // [CS] zero-denominator flag of every CTA
@@ -1289,15 +1205,14 @@ em_cluster_kernel(DevParams p, const int32_t* __restrict__ list, int n_list, uns
       for (int it = 0; it < p.max_iter; ++it) {
          iters = it + 1;
          int zero = 0;
-         if (resident) {
-            if (use_row_slots) slot_e_pass(S, rslot, th, zero);
-            else if (lpr == 1) resident_e_pass_rows4<NT>(S, th, zero);
-            else resident_e_pass<NT>(S, th, lpr, zero);
+         if (path.resident) {
+            if (path.row_slots) slot_e_pass(S, rslot, th, zero);
+            else resident_e_pass_rows4<NT>(S, th, zero);
             SBQ_TICK(0)
             zero = __syncthreads_or(zero);
             SBQ_TICK(1)
-            if (use_slots) slot_col_pass(S, slot, th);
-            else resident_col_pass<NT>(S, th, own, lpc);
+            if (path.col_slots) slot_col_pass(S, slot, th);
+            else resident_col_pass<NT>(S, th, own);
             SBQ_TICK(2)
          } else {
             if (g32 < G) cluster_em_pass<CL_LPR_STREAM>(grows, nrows, G, g32, lg32, th, my_acc, zero);
@@ -1423,8 +1338,8 @@ em_cluster_kernel(DevParams p, const int32_t* __restrict__ list, int n_list, uns
    if (rank == 0 && (tid == 0 || tid == NT - 32))
       printf("setup: sort %lld jd %lld fill %lld csc %lld rowslots %lld colslots %lld\n", st[0], st[1], st[2], st[3], st[4], st[5]);
    if (rank == 0 && (tid == 0 || tid == NT - 32))
-      printf("locus %d tid %d iters %d resident %d csc_smem %d slots %d/%d lanes %d/%d ncache %d lpr %d lpc %d nrows %d nnz %u setup %lld | E %lld or %lld col %lld csync1 %lld own %lld d2 %lld csync2 %lld chk %lld (cycles/iter)\n", l, tid, iters,
-             (int)resident, (int)csc_in_smem, (int)use_row_slots, (int)use_slots, rslot.lanes, slot.lanes, slot.ncache, lpr, lpc, nrows, nnz_c, t_setup, ph[0] / iters, ph[1] / iters, ph[2] / iters, ph[3] / iters, ph[4] / iters, ph[5] / iters, ph[6] / iters, ph[7] / iters);
+      printf("locus %d tid %d iters %d resident %d csc_smem %d slots %d/%d lanes %d/%d nrows %d nnz %u setup %lld | E %lld or %lld col %lld csync1 %lld own %lld d2 %lld csync2 %lld chk %lld (cycles/iter)\n", l, tid, iters,
+             (int)path.resident, (int)path.csc_in_smem, (int)path.row_slots, (int)path.col_slots, rslot.lanes, slot.lanes, nrows, nnz_c, t_setup, ph[0] / iters, ph[1] / iters, ph[2] / iters, ph[3] / iters, ph[4] / iters, ph[5] / iters, ph[6] / iters, ph[7] / iters);
 #endif
    if (pend_b) cluster_wait();
    cluster.sync();   // no CTA may exit while a peer can still read its shared memory

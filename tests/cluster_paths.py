@@ -3,22 +3,23 @@
 The cluster kernel (strawberry_b200/csrc/sbq_kernels.cuh, em_cluster_kernel) picks its path per CTA at run time, from the
 locus alone and the CTA's share of its rows: whether the slice and its transposed (CSC) index sit in shared memory, how the
 E- and M-passes spread over the threads, and how the partial theta' are exchanged inside the cluster. The planner
-(strawberry_b200/csrc/sbq.cu, plan) picks the cluster size and the thread count. `cta_paths` restates all of it, line by
-line, so that the tests can say which paths a batch reaches and check that a shape still reaches the path it was built for.
+(strawberry_b200/csrc/sbq.cu, plan) picks the cluster size and the thread count. `cta_paths` restates all of it - the per-CTA
+choice is `cta_path`, the restatement of the header's cluster_cta_path - so that the tests can say which paths a batch reaches and
+check that a shape still reaches the path it was built for.
 
 `em_csr_longdouble` is orc_em_csr (oracle/sbq_oracle.c:81-135) in np.longdouble: the yardstick for a few capped EM steps,
 where a double-precision restatement would be no more exact than the kernel it checks.
 """
 import numpy as np
 
-# ---- constants (sbq_kernels.cuh:368-379, sbq.cu:306-323)
-CL_NT = 512                 # sbq_kernels.cuh:368
-CL_LPR_STREAM = 32          # sbq_kernels.cuh:370
-CL_A2A_MAX = 4096           # sbq_kernels.cuh:378
-CL_SMEM_CAP = 220 * 1024    # sbq_kernels.cuh:379
-BUCKET_NT = (64, 128, 512, 512, 512)                        # sbq.cu:307
-SMEM_BUCKET_BOUNDS = (12 * 1024, 24 * 1024, 56 * 1024, 112 * 1024)   # sbq.cu:308
-CLUSTER_NNZ_BOUNDS = (16 * 1024, 32 * 1024, 64 * 1024, 150 * 1024)   # sbq.cu:318-321
+# ---- constants (sbq_kernels.cuh, sbq.cu)
+CL_NT = 512
+CL_LPR_STREAM = 32
+CL_A2A_MAX = 4096
+CL_SMEM_CAP = 220 * 1024
+BUCKET_NT = (64, 128, 512, 512, 512)                        # sbq.cu: BUCKET_NT
+SMEM_BUCKET_BOUNDS = (12 * 1024, 24 * 1024, 56 * 1024, 112 * 1024)   # sbq.cu: smem_bucket
+CLUSTER_NNZ_BOUNDS = (16 * 1024, 32 * 1024, 64 * 1024, 150 * 1024)   # sbq.cu: cluster_size_for
 
 # Bar of the capped-solve checks (theta after max_iter = 1, 2, 5 EM steps against em_csr_longdouble, relative, with the parity floor
 # of util.theta_close). Worst ratio measured on a B200 (1000 W power limit): 1.9e-15, over every tier on the golden batch and the
@@ -35,67 +36,76 @@ def _tdiv(a, b):
     return q if (a >= 0) == (b >= 0) else -q
 
 
-# ---- host-callable functions of the header (sbq_kernels.cuh:380-420)
-def cluster_a2a_stride(T):                                      # :380
+# ---- host-callable functions of the header (sbq_kernels.cuh), one each under the same name
+def cluster_a2a_stride(T):
     return (T + 1) & ~1
 
 
-def cluster_a2a(T, cs, slice_bytes):                             # :381-384
+def cluster_a2a(T, cs, slice_bytes):
     if cs <= 1 or cs * cluster_a2a_stride(T) > CL_A2A_MAX:
         return False
     return (4 * T + cs * cluster_a2a_stride(T) + 64) * 8 + slice_bytes + 256 <= CL_SMEM_CAP
 
 
-def cluster_fixed_doubles(T, cs, slice_bytes):                   # :386-388
+def cluster_fixed_doubles(T, cs, slice_bytes):
     return 4 * T + (cs * cluster_a2a_stride(T) + 64 if cluster_a2a(T, cs, slice_bytes) else 2 * T + 64)
 
 
-def cluster_stream_groups(T, smem_bytes, nt, cs, slice_bytes):   # :391-396
+def cluster_stream_groups(T, smem_bytes, nt, cs, slice_bytes):
     budget = smem_bytes // 8 - cluster_fixed_doubles(T, cs, slice_bytes)
     G = _tdiv(budget, T if T > 0 else 1)
     return min(G, nt // CL_LPR_STREAM)
 
 
-def cluster_diag_slots(T):                                       # :398
+def cluster_diag_slots(T):
     return (T + 7) & ~3
 
 
-def cluster_resident_csr_bytes(nnz_c, nrows, T):                 # :399-402
+def cluster_resident_csr_bytes(nnz_c, nrows, T):
     npos = nnz_c + T
     return (npos + 1) * 8 + (nrows + 2) * 8 + cluster_diag_slots(T) * 4 + nrows * 4 + (T + 1) * 4 + nrows * 2 + npos * 2 + 64
 
 
-def cluster_resident_bytes(nnz_c, nrows, T):                     # :403-405
+def cluster_resident_bytes(nnz_c, nrows, T):
     return cluster_resident_csr_bytes(nnz_c, nrows, T) + nnz_c * 4 + 4
 
 
-def cluster_class_smem(max_iso, slice_bytes, nt, cs):            # :411-416
+def cluster_class_smem(max_iso, slice_bytes, nt, cs):
     fixed = cluster_fixed_doubles(max_iso, cs, slice_bytes) * 8
     stream = (nt // CL_LPR_STREAM) * max_iso * 8
     want = fixed + max(slice_bytes, stream) + 256
     return min(want, CL_SMEM_CAP)
 
 
-def cluster_slice_estimate(nnz, R, T, cs):                       # :418-420 (the product is a C double, as here)
+def cluster_slice_estimate(nnz, R, T, cs):                       # the product is a C double, as here
     return int(1.12 * float(cluster_resident_bytes(nnz // cs + 1, R // cs + 1, T))) + 512
 
 
-def lanes_for(items, nt):                                        # :518-522 (SBQ_MIN_LANES = 1)
-    lanes = 32
-    while lanes > 1 and items * lanes > nt:
-        lanes >>= 1
-    return lanes
+def cta_path(T, cs, nt, nrows, nnz_c, too_long, slice_est, smem_launch):
+    """cluster_cta_path: the path of one CTA with nrows rows and nnz_c non-zeros (too_long: a row has more than T entries)."""
+    smem_bytes = min(smem_launch, cluster_class_smem(T, slice_est, nt, cs))
+    used = cluster_fixed_doubles(T, cs, slice_est) * 8
+    csr = cluster_resident_csr_bytes(nnz_c, nrows, T)
+    small_idx = nnz_c + T <= 65535 and nrows <= 65535 and not too_long
+    csc_in_smem = small_idx and used + cluster_resident_bytes(nnz_c, nrows, T) <= smem_bytes
+    resident = small_idx and used + csr <= smem_bytes
+    n_ent_s = nnz_c if csc_in_smem else min(nnz_c, (smem_bytes - used - csr) // 4) if resident else 0
+    a2a = cluster_a2a(T, cs, slice_est)
+    return dict(resident=resident, csc_in_smem=csc_in_smem, n_ent_s=n_ent_s,
+                G=0 if resident else cluster_stream_groups(T, smem_bytes, nt, cs, slice_est),
+                row_slots=resident and nrows <= nt, col_slots=resident and T <= nt, a2a=a2a,
+                B=cluster_a2a_stride(T) if a2a else (T + cs - 1) // cs)
 
 
-# ---- planner (sbq.cu:306-323, :381-384)
-def smem_bucket(nbytes):                                         # sbq.cu:308
+# ---- planner (sbq.cu: plan)
+def smem_bucket(nbytes):
     for b, bound in enumerate(SMEM_BUCKET_BOUNDS):
         if nbytes <= bound:
             return b
     return len(SMEM_BUCKET_BOUNDS)
 
 
-def cluster_size_for(nnz):                                       # sbq.cu:314-323
+def cluster_size_for(nnz):
     for cs, bound in zip((1, 2, 4, 8), CLUSTER_NNZ_BOUNDS):
         if nnz <= bound:
             return cs
@@ -103,14 +113,14 @@ def cluster_size_for(nnz):                                       # sbq.cu:314-32
 
 
 def plan(T, R, nnz, force_cluster=0):
-    """-> (cluster size, threads per CTA) of a cluster-tier locus (sbq.cu:381-386)."""
+    """-> (cluster size, threads per CTA) of a cluster-tier locus."""
     cs = force_cluster or cluster_size_for(nnz)
     slice_bytes = cluster_slice_estimate(nnz, R, T, cs)
     bucket = smem_bucket(cluster_fixed_doubles(T, 1, slice_bytes) * 8 + slice_bytes + 256) if cs == 1 else len(BUCKET_NT) - 1
     return cs, BUCKET_NT[bucket]
 
 
-# ---- per-CTA path (sbq_kernels.cuh:902-973, :1274-1284)
+# ---- per-CTA path (em_cluster_kernel: the row split, the too_long scan, then cluster_cta_path)
 def cta_paths(T, row_ptr, force_cluster=0):
     """Paths of every CTA that solves the locus (T isoforms, locus-local row_ptr). -> list of dicts, one per rank."""
     rp = np.asarray(row_ptr, np.int64)
@@ -118,16 +128,13 @@ def cta_paths(T, row_ptr, force_cluster=0):
     R = len(rp) - 1
     nnz = int(rp[R])
     CS, NT = plan(T, R, nnz, force_cluster)
-    slice_est = cluster_slice_estimate(nnz, R, T, CS)                          # :914
-    used = cluster_fixed_doubles(T, CS, slice_est) * 8                         # :915, :942
-    smem_bytes = cluster_class_smem(T, slice_est, NT, CS)                      # :922 (the launch provides at least this much)
-    a2a = cluster_a2a(T, CS, slice_est)                                        # :1274
-    B = cluster_a2a_stride(T) if a2a else (T + CS - 1) // CS                   # :1276
+    slice_est = cluster_slice_estimate(nnz, R, T, CS)
+    smem_launch = cluster_class_smem(T, slice_est, NT, CS)                    # the launch provides at least this much
     lens = np.diff(rp)
     out = []
     for rank in range(CS):
         bounds = []
-        for tid in (0, 1):                                                     # :925-936, lower_bound on row_ptr
+        for tid in (0, 1):                                                     # lower_bound on row_ptr
             if rank + tid >= CS:
                 bounds.append(R)
             elif rank + tid == 0:
@@ -138,27 +145,18 @@ def cta_paths(T, row_ptr, force_cluster=0):
         ra, rb = bounds
         nrows = rb - ra
         nnz_c = int(rp[rb] - rp[ra])
-        too_long = bool(nrows and lens[ra:rb].max() > T)                      # :945-947
-        small_idx = nnz_c + T <= 65535 and nrows <= 65535 and not too_long     # :948
-        csc_in_smem = small_idx and used + cluster_resident_bytes(nnz_c, nrows, T) <= smem_bytes      # :950
-        resident = small_idx and used + cluster_resident_csr_bytes(nnz_c, nrows, T) <= smem_bytes     # :951
-        n_ent_s = 0                                                            # :963-965
-        if csc_in_smem:
-            n_ent_s = nnz_c
-        elif resident:
-            n_ent_s = min(nnz_c, (smem_bytes - used - cluster_resident_csr_bytes(nnz_c, nrows, T)) // 4)
-        G = 0 if resident else cluster_stream_groups(T, smem_bytes, NT, CS, slice_est)   # :968
-        lpr = lanes_for(nrows, NT)                                             # :943
-        if not resident:
-            slice_state, e_pass, m_pass = "stream", "stream", "stream"         # :1303-1309
+        too_long = bool(nrows and lens[ra:rb].max() > T)
+        c = cta_path(T, CS, NT, nrows, nnz_c, too_long, slice_est, smem_launch)
+        if not c["resident"]:
+            slice_state, e_pass, m_pass = "stream", "stream", "stream"
         else:
-            slice_state = "csc_smem" if csc_in_smem else "csc_partial"
-            # :972-973, :1293-1295, :1299-1300
-            e_pass = "row_slots" if nrows <= NT else "rows4" if lpr == 1 else "lpr"
-            m_pass = "col_slots" if T <= NT else "generic"
-        out.append(dict(CS=CS, NT=NT, exchange="single" if CS == 1 else "a2a" if a2a else "owner", slice=slice_state,
-                        n_ent_s=n_ent_s, nnz_c=nnz_c, E=e_pass, M=m_pass, rows=(ra, rb), nrows=nrows, G=G, B=B,
-                        owned=max(0, min(B, T - rank * B)) if CS > 1 and not a2a else T))      # :1284
+            slice_state = "csc_smem" if c["csc_in_smem"] else "csc_partial"
+            e_pass = "row_slots" if c["row_slots"] else "rows4"
+            m_pass = "col_slots" if c["col_slots"] else "generic"
+        B = c["B"]
+        out.append(dict(CS=CS, NT=NT, exchange="single" if CS == 1 else "a2a" if c["a2a"] else "owner", slice=slice_state,
+                        n_ent_s=c["n_ent_s"], nnz_c=nnz_c, E=e_pass, M=m_pass, rows=(ra, rb), nrows=nrows, G=c["G"], B=B,
+                        owned=max(0, min(B, T - rank * B)) if CS > 1 and not c["a2a"] else T))
     return out
 
 

@@ -1,6 +1,6 @@
 """CPU checks of tests/cluster_paths.py: the restatement of the cluster kernel's path choice equals the header's own host-callable
-functions, the shapes of tests/test_gpu_cluster_paths.py reach every path listed below, the paths the kernel can never take are
-recorded as such, and the long-double EM restatement agrees with the oracle."""
+functions (cluster_cta_path included), the shapes of tests/test_gpu_cluster_paths.py reach every path listed below, the kernel is
+launched with exactly the planner's thread counts, and the long-double EM restatement agrees with the oracle."""
 import os
 import re
 import shutil
@@ -92,9 +92,21 @@ def test_resident_slices_with_the_csc_index_in_l2(cell_batches):
 
 _SHIM = r"""
 #include <cstdio>
+#include <cstring>
 #include "sbq_kernels.cuh"
 using namespace sbq;
-int main() {
+int main(int argc, char** argv) {
+   if (argc > 1 && !strcmp(argv[1], "path")) {       // cluster_cta_path
+      int T, cs, nt, nrows, too_long;
+      unsigned nnz_c, smem_launch;
+      size_t slice_est;
+      while (scanf("%d %d %d %d %u %d %zu %u", &T, &cs, &nt, &nrows, &nnz_c, &too_long, &slice_est, &smem_launch) == 8) {
+         const ClusterCtaPath c = cluster_cta_path(T, cs, nt, nrows, nnz_c, too_long != 0, slice_est, smem_launch);
+         printf("%d %d %u %d %d %d %d %d\n", (int)c.resident, (int)c.csc_in_smem, c.n_ent_s, c.G, (int)c.row_slots, (int)c.col_slots,
+                (int)c.a2a, c.B);
+      }
+      return 0;
+   }
    int T, cs, nt;
    long long R, nnz, smem;
    while (scanf("%d %lld %lld %d %d %lld", &T, &R, &nnz, &cs, &nt, &smem) == 6) {
@@ -114,14 +126,21 @@ def _nvcc():
     return n if os.path.exists(n) else shutil.which("nvcc")
 
 
-def test_restatement_equals_the_header(tmp_path):
-    """20 000 random (T, R, nnz, CS, NT) through the header's host-callable functions (compiled host-only) and through the restatement."""
+@pytest.fixture(scope="module")
+def shim(tmp_path_factory):
+    """The header's host-callable functions compiled host-only: run(mode args, input text) -> output lines."""
     nvcc = _nvcc()
     if not nvcc:
         pytest.skip("nvcc not found")
-    (tmp_path / "shim.cu").write_text(_SHIM)
-    exe = str(tmp_path / "shim")
-    subprocess.check_call([nvcc, "-arch=sm_100a", "-std=c++17", "-O1", "-I", CSRC, "-o", exe, str(tmp_path / "shim.cu")])
+    d = tmp_path_factory.mktemp("shim")
+    (d / "shim.cu").write_text(_SHIM)
+    exe = str(d / "shim")
+    subprocess.check_call([nvcc, "-arch=sm_100a", "-std=c++17", "-O1", "-I", CSRC, "-o", exe, str(d / "shim.cu")])
+    return lambda args, inp: [o for o in subprocess.run([exe, *args], input=inp, capture_output=True, text=True, check=True).stdout.split("\n") if o]
+
+
+def test_restatement_equals_the_header(shim):
+    """20 000 random (T, R, nnz, CS, NT) through the header's host-callable functions (compiled host-only) and through the restatement."""
     rng = np.random.default_rng(12345)
     n = 20_000
     T = np.minimum(3600, np.exp(rng.uniform(0, np.log(3600), n)).astype(np.int64))
@@ -131,8 +150,8 @@ def test_restatement_equals_the_header(tmp_path):
     nt = rng.choice([64, 128, 256, 512], n)
     smem = rng.integers(0, cp.CL_SMEM_CAP + 1, n)
     inp = "\n".join(f"{a} {b} {c} {d} {e} {f}" for a, b, c, d, e, f in zip(T, R, nnz, cs, nt, smem)) + "\n"
-    out = subprocess.run([exe], input=inp, capture_output=True, text=True, check=True).stdout.split("\n")
-    assert len([o for o in out if o]) == n
+    out = shim([], inp)
+    assert len(out) == n
     for i in range(n):
         t, r, z, c, m = int(T[i]), int(R[i]), int(nnz[i]), int(cs[i]), int(nt[i])
         sl = cp.cluster_slice_estimate(z, r, t, c)
@@ -143,12 +162,52 @@ def test_restatement_equals_the_header(tmp_path):
         assert [int(x) for x in out[i].split()] == want, (t, r, z, c, m, int(smem[i]))
 
 
+_PATH_FIELDS = ("resident", "csc_in_smem", "n_ent_s", "G", "row_slots", "col_slots", "a2a", "B")
+
+
+def test_cta_path_equals_the_kernel_function(shim):
+    """40 000 random CTAs through cluster_cta_path - the function em_cluster_kernel calls to pick a CTA's path - and through
+    cp.cta_path, field by field: every CS and NT, rows and non-zeros of the CTA up to and beyond the 16-bit limit of the resident
+    index, too_long both ways, and launch shared memory anywhere from 0 to the cap."""
+    rng = np.random.default_rng(2027)
+    n = 40_000
+    T = np.minimum(3600, np.exp(rng.uniform(0, np.log(3600), n)).astype(np.int64))
+    cs = rng.choice([1, 2, 4, 8, 16], n)
+    nt = rng.choice([64, 128, 512], n)
+    R = np.exp(rng.uniform(0, np.log(400_000), n)).astype(np.int64) + 1
+    nnz = np.minimum(R * T, (R * np.exp(rng.uniform(0, np.log(100), n))).astype(np.int64))
+    slice_est = [cp.cluster_slice_estimate(int(z), int(r), int(t), int(c)) for z, r, t, c in zip(nnz, R, T, cs)]
+    # the CTA's share of the locus, from a tenth to three times an even share (the row split is by non-zeros), some with no rows
+    f = np.exp(rng.uniform(np.log(0.1), np.log(3.0), n))
+    nrows = np.where(rng.random(n) < 0.02, 0, np.maximum(1, (R / cs * f).astype(np.int64)))
+    nnz_c = np.where(nrows == 0, 0, np.maximum(nrows, (nnz / cs * f).astype(np.int64)))
+    too_long = rng.random(n) < 0.1
+    smem = rng.integers(0, cp.CL_SMEM_CAP + 1, n)
+    rows = list(zip(T, cs, nt, nrows, nnz_c, too_long.astype(int), slice_est, smem))
+    out = shim(["path"], "\n".join(" ".join(str(int(x)) for x in r) for r in rows) + "\n")
+    assert len(out) == n
+    seen = set()
+    for i, (t, c, m, nr, z, tl, sl, sm) in enumerate(rows):
+        want = cp.cta_path(int(t), int(c), int(m), int(nr), int(z), bool(tl), int(sl), int(sm))
+        got = [int(x) for x in out[i].split()]
+        assert got == [int(want[k]) for k in _PATH_FIELDS], (rows[i], dict(zip(_PATH_FIELDS, got)), want)
+        seen.add("stream" if not want["resident"] else "csc_smem" if want["csc_in_smem"] else
+                 "csc_partial, clamped" if want["n_ent_s"] < z else "csc_partial")
+        seen.add(("row_slots", want["row_slots"]))
+        seen.add(("col_slots", want["col_slots"]))
+        seen.add(("a2a", want["a2a"]))
+        if z + t > 65535 or nr > 65535:
+            seen.add("index over 16 bits")
+    assert seen >= {"stream", "csc_smem", "csc_partial, clamped", "index over 16 bits", ("row_slots", True), ("row_slots", False),
+                    ("col_slots", True), ("col_slots", False), ("a2a", True), ("a2a", False)}, seen
+
+
 def _src(name):
     with open(os.path.join(CSRC, name)) as f:
         return f.read()
 
 
-def test_restated_planner_constants_match_the_source():
+def test_restated_planner_and_header_constants_match_the_source():
     """cluster_size_for, smem_bucket / BUCKET_NT (sbq.cu) and the header constants are restated by value: a change there fails here."""
     cu, hdr = _src("sbq.cu"), _src("sbq_kernels.cuh")
     m = re.search(r"const int BUCKET_NT\[N_BUCKETS\] = \{([^}]*)\};", cu)
@@ -162,22 +221,18 @@ def test_restated_planner_constants_match_the_source():
     for name, val in (("CL_NT", cp.CL_NT), ("CL_LPR_STREAM", cp.CL_LPR_STREAM), ("CL_A2A_MAX", cp.CL_A2A_MAX)):
         assert re.search(rf"constexpr int {name} = (\d+);", hdr).group(1) == str(val), name
     assert "constexpr size_t CL_SMEM_CAP = 220 * 1024;" in hdr and cp.CL_SMEM_CAP == 220 * 1024
-    assert "#define SBQ_MIN_LANES 1\n" in hdr
 
 
-def test_dead_paths_stay_dead():
-    """Three paths of the cluster kernel are never taken, recorded here so that a change that revives one is noticed:
-    - resident_e_pass with lpr > 1: lanes_for(nrows, NT) > 1 needs 2 nrows <= NT, and nrows <= NT takes the row slots first;
-    - every NCACHE > 0 instantiation of em_cluster_kernel: the launches pass NCACHE = 0;
-    - the 256-thread launch: BUCKET_NT has no 256."""
-    for nt in set(cp.BUCKET_NT):
-        for nrows in range(0, 4 * nt + 2):
-            if cp.lanes_for(nrows, nt) > 1:
-                assert nrows <= nt
+def test_launch_arms_are_the_bucket_thread_counts():
+    """sbq.cu launches em_cluster_kernel through one arm per thread count: exactly the values of BUCKET_NT, each arm taken for the
+    thread count it instantiates."""
     cu = _src("sbq.cu")
-    inst = re.findall(r"launch_cluster_class_nt<(\w+), (\w+), (\w+)>", cu)
-    assert inst and all(ncache == "0" for _, ncache, _ in inst), inst
-    assert 256 not in cp.BUCKET_NT
+    m = re.search(r"int rc = (lc\.nt == .*?);\n", cu, re.S)
+    arms = re.findall(r"lc\.nt == (\d+) \? launch_cluster_class_nt<(\d+)>\(c, lc, ss\)", m.group(1))
+    assert arms and all(a == b for a, b in arms), arms
+    last = re.findall(r":\s*launch_cluster_class_nt<(\d+)>\(c, lc, ss\)$", m.group(1))
+    assert sorted({int(a) for a, _ in arms} | {int(x) for x in last}) == sorted(set(cp.BUCKET_NT)), m.group(1)
+    assert len(re.findall(r"launch_cluster_class_nt<", cu)) == len(set(cp.BUCKET_NT)), "a launch arm outside the dispatch"
 
 
 def test_streaming_always_has_a_group():
