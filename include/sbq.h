@@ -235,6 +235,21 @@ int  sbq_em_solve(sbq_ctx*, const sbq_locus* locus, double* theta, int32_t* iter
 int  sbq_set_covariates(sbq_ctx*, const double* x, int64_t n_row, int32_t n_cov);
 int  sbq_bias_results(sbq_ctx*, double* beta, int32_t* outer_iters);
 
+/* Bootstrap replicates (OUR definition, DESIGN.md "Bootstrap replicates"; the reference has none). Replicate b redraws each locus'
+ * N = sum n_i fragments from its own classes (multinomial, conditional on N, by a counter-based hash of (seed, b, submit position
+ * of the locus)) and runs the same EM + epilogue on those counts; total_mapped_reads and the point estimate stay as they are.
+ * Needs a resident batch solved by sbq_solve; SBQ_ERR_UNSUPPORTED in bias mode. Device memory per replicate: 16 n_iso + 8 n_loci
+ * bytes (SBQ_ERR_NOMEM leaves the context usable). */
+/* Bootstrap replicates first .. first + n - 1 of the resident, solved batch (our definition, DESIGN.md). */
+int  sbq_bootstrap(sbq_ctx*, uint64_t seed, int64_t first, int32_t n);
+/* Replicates of the last sbq_bootstrap, submit order: theta / tpm [n][n_iso], iters / status [n][n_loci]; any pointer may be NULL. */
+int  sbq_bootstrap_results(sbq_ctx*, double* theta, double* tpm, int32_t* iters, int32_t* status);
+/* Test aid: the resampled counts of one replicate, n_row values in submit row order (needs a resident batch only). */
+int  sbq_bootstrap_counts(sbq_ctx*, uint64_t seed, int64_t replicate, int32_t* count);
+/* Device time of the last sbq_bootstrap (CUDA events; multi-GPU: the slowest device). */
+typedef struct { int64_t first, n; double resample_ms, em_ms, total_ms; } sbq_bootstrap_stat;
+int  sbq_bootstrap_stats(const sbq_ctx*, sbq_bootstrap_stat* out);
+
 /* Planner knobs, mainly for tests: force a tier (0 = auto, 1 = warp, 2 = CTA/cluster, 3 = grid) and
  * the cluster size of the CTA tier (0 = auto, else 1, 2, 4, 8, 16). */
 int  sbq_set_plan(sbq_ctx*, int force_tier, int force_cluster);

@@ -31,6 +31,7 @@ ABI_SYMBOLS = [
     "sbq_upload", "sbq_upload_begin", "sbq_solve", "sbq_download", "sbq_run", "sbq_fpkm_sum", "sbq_fpkm_sum_to_device",
     "sbq_finalize_tpm", "sbq_results", "sbq_get_stats", "sbq_get_launch_stats", "sbq_em_solve", "sbq_set_plan",
     "sbq_set_covariates", "sbq_bias_results", "sbq_partition_lpt", "sbq_locus_devices", "sbq_synth_giant", "sbq_fetch_batch",
+    "sbq_bootstrap", "sbq_bootstrap_results", "sbq_bootstrap_counts", "sbq_bootstrap_stats",
 ]
 
 
@@ -76,6 +77,14 @@ class LaunchStat(ctypes.Structure):
                 ("alg_bytes", ctypes.c_int64), ("frag_iters", ctypes.c_int64), ("max_iters", ctypes.c_int64), ("start_ms", ctypes.c_double)]
 
 
+class BootstrapStat(ctypes.Structure):
+    _fields_ = [("first", ctypes.c_int64), ("n", ctypes.c_int64), ("resample_ms", ctypes.c_double), ("em_ms", ctypes.c_double),
+                ("total_ms", ctypes.c_double)]
+
+    def as_dict(self):
+        return {n: getattr(self, n) for n, _ in self._fields_}
+
+
 _lib = None
 
 
@@ -116,6 +125,10 @@ def lib():
         L.sbq_locus_devices.argtypes = [ctypes.c_void_p, ctypes.c_void_p]
         L.sbq_synth_giant.argtypes = [ctypes.c_void_p, ctypes.POINTER(SynthGiantSpec)]
         L.sbq_fetch_batch.argtypes = [ctypes.c_void_p] + [ctypes.c_void_p] * 7
+        L.sbq_bootstrap.argtypes = [ctypes.c_void_p, ctypes.c_uint64, ctypes.c_int64, ctypes.c_int32]
+        L.sbq_bootstrap_results.argtypes = [ctypes.c_void_p] + [ctypes.c_void_p] * 4
+        L.sbq_bootstrap_counts.argtypes = [ctypes.c_void_p, ctypes.c_uint64, ctypes.c_int64, ctypes.c_void_p]
+        L.sbq_bootstrap_stats.argtypes = [ctypes.c_void_p, ctypes.POINTER(BootstrapStat)]
         _lib = L
     return _lib
 
@@ -330,6 +343,28 @@ class Quantifier:
                    keep=np.empty(ni, np.int32), iters=np.empty(nl, np.int32), status=np.empty(nl, np.int32))
         self._chk(self._L.sbq_results(self._h, *[_ptr(out[k]) for k in ("theta", "fpkm", "frac", "tpm", "keep", "iters", "status")]))
         return out
+
+    def bootstrap(self, seed, n, first=0):
+        """Bootstrap replicates first .. first + n - 1 of the solved, resident batch (DESIGN.md "Bootstrap replicates"): theta and
+        tpm shaped (n, n_iso), iters and status shaped (n, n_loci), submit order. The point estimate (results()) is unchanged."""
+        self._chk(self._L.sbq_bootstrap(self._h, int(seed) & (2**64 - 1), int(first), int(n)))
+        st = self.stats()
+        ni, nl = st["n_iso"], st["n_loci"]
+        out = dict(theta=np.empty((n, ni)), tpm=np.empty((n, ni)), iters=np.empty((n, nl), np.int32), status=np.empty((n, nl), np.int32))
+        self._chk(self._L.sbq_bootstrap_results(self._h, *[_ptr(out[k]) for k in ("theta", "tpm", "iters", "status")]))
+        return out
+
+    def bootstrap_counts(self, seed, replicate):
+        """The resampled class counts of one replicate, per row in submit order (needs a resident batch only)."""
+        out = np.empty(self.stats()["n_row"], np.int32)
+        self._chk(self._L.sbq_bootstrap_counts(self._h, int(seed) & (2**64 - 1), int(replicate), _ptr(out) if out.size else ctypes.c_void_p(1)))
+        return out
+
+    def bootstrap_stats(self):
+        """Device time of the last bootstrap(): resample_ms, em_ms (EM + FPKM sum, all replicates) and total_ms."""
+        s = BootstrapStat()
+        self._chk(self._L.sbq_bootstrap_stats(self._h, ctypes.byref(s)))
+        return s.as_dict()
 
     def em_solve(self, n_iso, row_ptr, col, alpha, count):
         rp, c, a, n = _c(row_ptr, np.int64), _c(col, np.int32), _c(alpha, np.float64), _c(count, np.int32)

@@ -30,6 +30,7 @@
 #include "sbq_weights.cuh"
 #include "sbq_synth.cuh"
 #include "sbq_rawbuild.cuh"
+#include "sbq_bootstrap.cuh"
 
 using namespace sbq;
 
@@ -213,6 +214,20 @@ struct sbq_ctx {
 
    sbq_stats stats{};
    bool stats_stale = false;
+
+   // bootstrap replicates (sbq_bootstrap): draw offsets of the resident batch (built once per upload), per-replicate scratch and the
+   // replicate matrices of the last call
+   struct Boot {
+      DevBuf prefix, scratch, out, sums;
+      bool prefix_ready = false;
+      int64_t* draw_off = nullptr;       // [n_row + 1] exclusive prefix of the counts
+      int64_t* loc_draw_off = nullptr;   // [n_loci + 1] the same at the locus boundaries
+      int32_t* d_lid = nullptr;          // [n_loci] hash position of every locus (multi-GPU children)
+      std::vector<int32_t> lid;          // multi-GPU children: the parent's submit position of each locus; empty = own index
+      bool done = false;                 // the replicate matrices in `out` belong to the resident batch
+      sbq_bootstrap_stat stat{};
+      std::vector<cudaEvent_t> ev;
+   } boot;
 };
 
 namespace {
@@ -285,6 +300,7 @@ void reset_batch(sbq_ctx* c) {
    c->raw_mode = false;
    c->h_wseg.clear(); c->h_wn.clear(); c->h_wmask.clear(); c->h_wpool.clear(); c->h_wlen.clear(); c->h_wpool_off.clear();
    c->resident = c->solved = c->downloaded = false;
+   c->boot.prefix_ready = c->boot.done = false;
 }
 
 int ensure_origin(sbq_ctx* c) {
@@ -611,6 +627,12 @@ int submit_locked(sbq_ctx* c, const sbq_locus* loci, int64_t n_loci) {
    return SBQ_SUCCESS;
 }
 
+// bootstrap replicates on one device (defined with sbq_bootstrap at the end of this file); the caller holds c->mu
+int boot_em_locked(sbq_ctx* c, uint64_t seed, int64_t first, int32_t n);
+int boot_finish_locked(sbq_ctx* c);
+int boot_counts_locked(sbq_ctx* c, uint64_t seed, int64_t rep, int32_t* count);
+int boot_results_locked(sbq_ctx* c, double* theta, double* tpm, int32_t* iters, int32_t* status);
+
 }  // namespace
 
 #include "sbq_multi.cuh"
@@ -734,6 +756,8 @@ void sbq_destroy(sbq_ctx* c) {
    if (c->grid[1].st) cudaStreamSynchronize(c->grid[1].st), cudaStreamDestroy(c->grid[1].st);   // grid[0] runs on c->stream
    c->h_cov.release(); c->r_beta.release(); c->r_outer.release();
    c->h_wseg.release(); c->h_wn.release(); c->h_wmask.release(); c->h_wpool.release(); c->h_wlen.release(); c->h_wpool_off.release(); c->d_weights.release();
+   c->boot.prefix.release(); c->boot.scratch.release(); c->boot.out.release(); c->boot.sums.release();
+   for (auto& e : c->boot.ev) cudaEventDestroy(e);
    for (auto& e : c->ev) if (e) cudaEventDestroy(e);
    if (c->ev_fork) cudaEventDestroy(c->ev_fork);
    for (auto& e : c->ev_join) if (e) cudaEventDestroy(e);
@@ -885,6 +909,7 @@ static int upload_begin(sbq_ctx* c) {
    cudaStream_t st = c->copy_st;
    c->upload_pending = true;
    c->resident = c->solved = c->downloaded = false;
+   c->boot.prefix_ready = c->boot.done = false;
    CU(cudaEventRecord(c->ev[0], st));
    CU(cudaMemcpyAsync(d_lro, loc_row_off(c), (c->n_loci + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
    CU(cudaMemcpyAsync(d_lio, loc_iso_off(c), (c->n_loci + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
@@ -980,6 +1005,90 @@ static int upload_wait(sbq_ctx* c) {
    float ms = 0;
    CU(cudaEventElapsedTime(&ms, c->ev[0], c->ev[1]));
    c->stats.upload_ms = ms;
+   return SBQ_SUCCESS;
+}
+
+// The EM launches of one solve of the resident batch, into the outputs c->dp points at: grid tier, cluster classes and warp tier
+// forked from c->stream and joined back onto it. sbq_solve runs it once, sbq_bootstrap once per replicate with dp.count pointing at
+// the replicate's counts. pending: the launches wait for the copies of an asynchronous upload.
+static int launch_em(sbq_ctx* c, bool pending, int64_t& launches) {
+   cudaStream_t st = c->stream;
+   CU(cudaEventRecord(c->ev_fork, st));
+   for (auto& t : c->lt) t.used = false;
+   if (!(c->grid[0].list.empty() && c->grid[1].list.empty())) {
+      // the 16-bit slot array is shared by both classes (indexed by non-zero): sized here, so that neither launch re-allocates it
+      // under the other
+      const size_t need16 = (size_t)c->nnz * 2 + 256;
+      if (need16 > c->d_col16.cap) {
+         if (!c->d_col16.reserve(need16)) return fail(c, SBQ_ERR_NOMEM, "device allocation failed (16-bit slots)");
+         c->col16_ready = false;
+      }
+   }
+   // grid tier first: the full grid on the main stream (it owns the whole GPU while it runs), then the sub-grid on its own stream,
+   // launched before the cluster classes so that it is resident when they fill the other SMs
+   for (int k = 0; k < 2; ++k) {
+      GridClass& g = c->grid[k];
+      g.lt.used = false;
+      if (g.list.empty()) continue;
+      CU(cudaStreamWaitEvent(g.st, c->ev_fork, 0));
+      if (k == 1 && c->grid[0].lt.used) CU(cudaStreamWaitEvent(g.st, c->grid[0].lt.e1, 0));   // the full-grid class owns the GPU first
+      if (pending) CU(cudaStreamWaitEvent(g.st, c->grid_ready ? c->ev_grid_ready : c->ev[1], 0));
+      CU(cudaEventRecord(g.lt.e0, g.st));
+      int n_launch = 0;
+      const int rc = launch_grid_class(c, g, n_launch);
+      if (rc != 0) {
+         // the one-off layout passes permute alpha inside each giant row IN PLACE: after a failure the resident copy can no
+         // longer be trusted to match the column arrays, so the batch has to be uploaded again
+         c->resident = false;
+         c->col16_ready = false;
+         return fail(c, rc < -6 ? SBQ_ERR_CUDA : rc, "grid tier launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+      }
+      launches += n_launch;
+      CU(cudaEventRecord(g.lt.e1, g.st));
+      g.lt.used = true;
+   }
+   if (!(c->grid[0].list.empty() && c->grid[1].list.empty())) c->col16_ready = true;
+   // Launch order: the cluster classes (biggest clusters first, see plan()), then the warp tier. The work distributor serves
+   // kernels roughly in launch order, 16- and 8-CTA clusters strand a few SMs per GPC that only single CTAs can use, and the
+   // many small loci have critical paths of their own (~1 ms): see DESIGN.md section 5 for the measured timelines.
+   const int ncls = (int)c->classes.size();
+   for (int i = 0; i < ncls; ++i) {
+      const LaunchClass& lc = c->classes[i];
+      cudaStream_t ss = c->side[i % N_SIDE_STREAMS];
+      if (i < N_SIDE_STREAMS) CU(cudaStreamWaitEvent(ss, c->ev_fork, 0));
+      if (pending) CU(cudaStreamWaitEvent(ss, (i < N_SIDE_STREAMS && c->class_ready[i]) ? c->ev_class_ready[i] : c->ev[1], 0));
+      LaunchTimer& t = c->lt[1 + i % N_SIDE_STREAMS];
+      CU(cudaEventRecord(t.e0, ss));
+      // one arm per thread count of BUCKET_NT
+      int rc = lc.nt == 64 ? launch_cluster_class_nt<64>(c, lc, ss) : lc.nt == 128 ? launch_cluster_class_nt<128>(c, lc, ss) :
+               launch_cluster_class_nt<512>(c, lc, ss);
+      if (rc) return rc;
+      CU(cudaEventRecord(t.e1, ss));
+      t.used = true;
+      ++launches;
+   }
+   if (!c->warp_list.empty()) {
+      const size_t smem = warp_tier_smem_bytes(c->warp_max_iso);
+      CU(cudaFuncSetAttribute(em_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      const int n = (int)c->warp_list.size();
+      int per_sm = 1;
+      CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, em_warp_kernel, WT_WARPS * 32, smem));
+      const int grid = std::max(1, std::min((n + WT_WARPS - 1) / WT_WARPS, per_sm * c->prop.multiProcessorCount));   // persistent warps: the grid only sets the parallelism
+      int* queue = (int*)((char*)c->d_fpkm_sum + 64);
+      if (pending) CU(cudaStreamWaitEvent(st, c->ev[1], 0));   // many small loci all over the batch: they need everything
+      CU(cudaMemsetAsync(queue, 0, sizeof(int), st));
+      CU(cudaEventRecord(c->lt[0].e0, st));
+      em_warp_kernel<<<grid, WT_WARPS * 32, smem, st>>>(c->dp, c->d_lists_p + c->warp_list_off, n, c->warp_max_iso, queue);
+      CU(cudaGetLastError());
+      CU(cudaEventRecord(c->lt[0].e1, st));
+      c->lt[0].used = true;
+      ++launches;
+   }
+   for (int i = 0; i < std::min(ncls, N_SIDE_STREAMS); ++i) {
+      CU(cudaEventRecord(c->ev_join[i], c->side[i]));
+      CU(cudaStreamWaitEvent(st, c->ev_join[i], 0));
+   }
+   if (c->grid[1].lt.used) CU(cudaStreamWaitEvent(st, c->grid[1].lt.e1, 0));
    return SBQ_SUCCESS;
 }
 
@@ -1177,84 +1286,12 @@ int sbq_solve(sbq_ctx* c, int64_t total_mapped_reads) {
       return SBQ_SUCCESS;
    }
    CU(cudaEventRecord(c->ev[2], st));
-   CU(cudaEventRecord(c->ev_fork, st));
    c->stats.grid_em_ms = 0;
-   for (auto& t : c->lt) t.used = false;
    const bool pending = c->upload_pending;   // asynchronous upload in flight: every launch waits for the copies it needs only
-   if (!(c->grid[0].list.empty() && c->grid[1].list.empty())) {
-      // the 16-bit slot array is shared by both classes (indexed by non-zero): sized here, so that neither launch re-allocates it
-      // under the other
-      const size_t need16 = (size_t)c->nnz * 2 + 256;
-      if (need16 > c->d_col16.cap) {
-         if (!c->d_col16.reserve(need16)) return fail(c, SBQ_ERR_NOMEM, "device allocation failed (16-bit slots)");
-         c->col16_ready = false;
-      }
-   }
-   // grid tier first: the full grid on the main stream (it owns the whole GPU while it runs), then the sub-grid on its own stream,
-   // launched before the cluster classes so that it is resident when they fill the other SMs
-   for (int k = 0; k < 2; ++k) {
-      GridClass& g = c->grid[k];
-      g.lt.used = false;
-      if (g.list.empty()) continue;
-      CU(cudaStreamWaitEvent(g.st, c->ev_fork, 0));
-      if (k == 1 && c->grid[0].lt.used) CU(cudaStreamWaitEvent(g.st, c->grid[0].lt.e1, 0));   // the full-grid class owns the GPU first
-      if (pending) CU(cudaStreamWaitEvent(g.st, c->grid_ready ? c->ev_grid_ready : c->ev[1], 0));
-      CU(cudaEventRecord(g.lt.e0, g.st));
-      int n_launch = 0;
-      const int rc = launch_grid_class(c, g, n_launch);
-      if (rc != 0) {
-         // the one-off layout passes permute alpha inside each giant row IN PLACE: after a failure the resident copy can no
-         // longer be trusted to match the column arrays, so the batch has to be uploaded again
-         c->resident = false;
-         c->col16_ready = false;
-         return fail(c, rc < -6 ? SBQ_ERR_CUDA : rc, "grid tier launch failed: %s", cudaGetErrorString(cudaGetLastError()));
-      }
-      launches += n_launch;
-      CU(cudaEventRecord(g.lt.e1, g.st));
-      g.lt.used = true;
-   }
-   if (!(c->grid[0].list.empty() && c->grid[1].list.empty())) c->col16_ready = true;
-   // Launch order: the cluster classes (biggest clusters first, see plan()), then the warp tier. The work distributor serves
-   // kernels roughly in launch order, 16- and 8-CTA clusters strand a few SMs per GPC that only single CTAs can use, and the
-   // many small loci have critical paths of their own (~1 ms): see DESIGN.md section 5 for the measured timelines.
-   const int ncls = (int)c->classes.size();
-   for (int i = 0; i < ncls; ++i) {
-      const LaunchClass& lc = c->classes[i];
-      cudaStream_t ss = c->side[i % N_SIDE_STREAMS];
-      if (i < N_SIDE_STREAMS) CU(cudaStreamWaitEvent(ss, c->ev_fork, 0));
-      if (pending) CU(cudaStreamWaitEvent(ss, (i < N_SIDE_STREAMS && c->class_ready[i]) ? c->ev_class_ready[i] : c->ev[1], 0));
-      LaunchTimer& t = c->lt[1 + i % N_SIDE_STREAMS];
-      CU(cudaEventRecord(t.e0, ss));
-      // one arm per thread count of BUCKET_NT
-      int rc = lc.nt == 64 ? launch_cluster_class_nt<64>(c, lc, ss) : lc.nt == 128 ? launch_cluster_class_nt<128>(c, lc, ss) :
-               launch_cluster_class_nt<512>(c, lc, ss);
+   {
+      const int rc = launch_em(c, pending, launches);
       if (rc) return rc;
-      CU(cudaEventRecord(t.e1, ss));
-      t.used = true;
-      ++launches;
    }
-   if (!c->warp_list.empty()) {
-      const size_t smem = warp_tier_smem_bytes(c->warp_max_iso);
-      CU(cudaFuncSetAttribute(em_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      const int n = (int)c->warp_list.size();
-      int per_sm = 1;
-      CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, em_warp_kernel, WT_WARPS * 32, smem));
-      const int grid = std::max(1, std::min((n + WT_WARPS - 1) / WT_WARPS, per_sm * c->prop.multiProcessorCount));   // persistent warps: the grid only sets the parallelism
-      int* queue = (int*)((char*)c->d_fpkm_sum + 64);
-      if (pending) CU(cudaStreamWaitEvent(st, c->ev[1], 0));   // many small loci all over the batch: they need everything
-      CU(cudaMemsetAsync(queue, 0, sizeof(int), st));
-      CU(cudaEventRecord(c->lt[0].e0, st));
-      em_warp_kernel<<<grid, WT_WARPS * 32, smem, st>>>(c->dp, c->d_lists_p + c->warp_list_off, n, c->warp_max_iso, queue);
-      CU(cudaGetLastError());
-      CU(cudaEventRecord(c->lt[0].e1, st));
-      c->lt[0].used = true;
-      ++launches;
-   }
-   for (int i = 0; i < std::min(ncls, N_SIDE_STREAMS); ++i) {
-      CU(cudaEventRecord(c->ev_join[i], c->side[i]));
-      CU(cudaStreamWaitEvent(st, c->ev_join[i], 0));
-   }
-   if (c->grid[1].lt.used) CU(cudaStreamWaitEvent(st, c->grid[1].lt.e1, 0));
    CU(cudaEventRecord(c->ev[3], st));
    fpkm_sum_kernel<<<1, 1024, 0, st>>>(dp.locus_fpkm, c->n_loci, c->d_fpkm_sum);
    CU(cudaGetLastError());
@@ -1603,6 +1640,7 @@ int rb_scan(cudaStream_t st, const int32_t* v, int64_t n, long long* block_tmp, 
 static int raw_upload(sbq_ctx* c) {
    CU(cudaSetDevice(c->device));
    if (!c->have_model && !c->raw.long_read) return fail(c, SBQ_ERR_STATE, "raw loci need sbq_set_insert_model()");
+   c->boot.prefix_ready = c->boot.done = false;
    auto& r = c->raw;
    const int64_t L = c->n_loci, H = (int64_t)r.hit_locus.size(), T = c->n_iso, S = (int64_t)r.seg_left.size();
    const int64_t* lio = c->h_loc_iso_off.p;
@@ -2130,6 +2168,229 @@ void* sbq_host_alloc(size_t bytes) {
 }
 void sbq_host_free(void* p) {
    if (p) cudaFreeHost(p);
+}
+
+}  // extern "C"
+
+// ================================================================================================
+// Bootstrap replicates (sbq_bootstrap.cuh; DESIGN.md "Bootstrap replicates")
+namespace {
+
+struct BootOut {
+   double *theta, *tpm;
+   int32_t *iters, *status;
+};
+
+size_t boot_out_bytes(const sbq_ctx* c, int64_t n) { return 2 * align_up((size_t)n * c->n_iso * 8) + 2 * align_up((size_t)n * c->n_loci * 4); }
+
+BootOut boot_out(const sbq_ctx* c, int64_t n) {
+   char* q = (char*)c->boot.out.p;
+   BootOut o;
+   o.theta = (double*)q; q += align_up((size_t)n * c->n_iso * 8);
+   o.tpm = (double*)q; q += align_up((size_t)n * c->n_iso * 8);
+   o.iters = (int32_t*)q; q += align_up((size_t)n * c->n_loci * 4);
+   o.status = (int32_t*)q;
+   return o;
+}
+
+// draw offsets of the resident batch (once per upload: the counts do not change) and the loci's hash positions (every call: a
+// multi-GPU parent sets them before it calls)
+int boot_prefix(sbq_ctx* c) {
+   sbq_ctx::Boot& B = c->boot;
+   cudaStream_t st = c->stream;
+   const int64_t L = c->n_loci, R = c->n_row;
+   if (!B.prefix_ready) {
+      for (int64_t l = 0; l < L && l < (int64_t)c->meta.size(); ++l)
+         if (c->meta[l].frags > INT32_MAX)
+            return fail(c, SBQ_ERR_UNSUPPORTED, "locus %lld holds %lld fragments: a resampled class count must fit int32", (long long)l, (long long)c->meta[l].frags);
+      const int64_t nb = (R + RB_SCAN_BLOCK - 1) / RB_SCAN_BLOCK;
+      const size_t b_row = align_up((R + 1) * 8), b_loc = align_up((L + 1) * 8), b_lid = align_up(L * 4 + 4), b_tmp = align_up((nb + 1) * 8);
+      if (!B.prefix.reserve(b_row + b_loc + b_lid + b_tmp)) {
+         cudaGetLastError();   // a failed allocation is not an error of the context
+         return fail(c, SBQ_ERR_NOMEM, "device allocation failed (bootstrap draw offsets)");
+      }
+      char* q = (char*)B.prefix.p;
+      B.draw_off = (int64_t*)q; q += b_row;
+      B.loc_draw_off = (int64_t*)q; q += b_loc;
+      B.d_lid = (int32_t*)q; q += b_lid;
+      if (rb_scan(st, c->dp.count, R, (long long*)q, B.draw_off)) return fail(c, SBQ_ERR_CUDA, "bootstrap count prefix: %s", cudaGetErrorString(cudaGetLastError()));
+      rb_gather_kernel<<<(unsigned)((L + 1 + 255) / 256), 256, 0, st>>>(B.draw_off, c->dp.loc_row_off, L + 1, B.loc_draw_off);
+      CU(cudaGetLastError());
+      B.prefix_ready = true;
+   }
+   if (!B.lid.empty()) CU(cudaMemcpyAsync(B.d_lid, B.lid.data(), (size_t)L * 4, cudaMemcpyHostToDevice, st));
+   return SBQ_SUCCESS;
+}
+
+// the counts of replicate `rep` into out[n_row], on c->stream
+int boot_resample(sbq_ctx* c, uint64_t seed, uint64_t rep, int32_t* out) {
+   const sbq_ctx::Boot& B = c->boot;
+   cudaStream_t st = c->stream;
+   if (c->n_row) CU(cudaMemsetAsync(out, 0, (size_t)c->n_row * 4, st));
+   boot_resample_kernel<<<c->prop.multiProcessorCount * 8, 256, 0, st>>>(B.draw_off, B.loc_draw_off, c->dp.loc_row_off, c->n_loci,
+                                                                        B.lid.empty() ? nullptr : B.d_lid, seed, rep, out);
+   CU(cudaGetLastError());
+   return SBQ_SUCCESS;
+}
+
+// replicate scratch: counts [n_row], frac [n_iso], keep [n_iso], locus FPKM [n_loci]
+size_t boot_scratch_bytes(const sbq_ctx* c) { return align_up(c->n_row * 4 + 4) + align_up(c->n_iso * 8 + 8) + align_up(c->n_iso * 4 + 4) + align_up(c->n_loci * 8 + 8); }
+
+// resample + EM + FPKM sum of every replicate; dp points at replicate j's slots while its launches are enqueued (c->dp is
+// restored by the caller)
+int boot_replicates(sbq_ctx* c, uint64_t seed, int64_t first, int32_t n) {
+   sbq_ctx::Boot& B = c->boot;
+   DevParams& dp = c->dp;
+   cudaStream_t st = c->stream;
+   const size_t ni = c->n_iso, nl = c->n_loci;
+   char* q = (char*)B.scratch.p;
+   int32_t* cnt = (int32_t*)q; q += align_up(c->n_row * 4 + 4);
+   dp.frac = (double*)q; q += align_up(ni * 8 + 8);
+   dp.keep = (int32_t*)q; q += align_up(ni * 4 + 4);
+   dp.locus_fpkm = (double*)q;
+   dp.count = cnt;
+   const BootOut o = boot_out(c, n);
+   double* sums = (double*)B.sums.p;
+   int64_t launches = 0;
+   for (int32_t j = 0; j < n; ++j) {
+      CU(cudaEventRecord(B.ev[2 * j], st));
+      int rc = boot_resample(c, seed, (uint64_t)first + (uint64_t)j, cnt);
+      if (rc) return rc;
+      CU(cudaEventRecord(B.ev[2 * j + 1], st));
+      dp.theta = o.theta + j * ni;
+      dp.fpkm = o.tpm + j * ni;   // FPKM now, TPM after the last replicate (boot_finish_locked)
+      dp.iters = o.iters + j * nl;
+      dp.status = o.status + j * nl;
+      if ((rc = launch_em(c, false, launches))) return rc;
+      fpkm_sum_kernel<<<1, 1024, 0, st>>>(dp.locus_fpkm, c->n_loci, sums + j);
+      CU(cudaGetLastError());
+   }
+   CU(cudaEventRecord(B.ev[2 * n], st));
+   return SBQ_SUCCESS;
+}
+
+}  // namespace
+
+namespace {
+
+int boot_em_locked(sbq_ctx* c, uint64_t seed, int64_t first, int32_t n) {
+   CU(cudaSetDevice(c->device));
+   if (!c->resident || !c->solved) return fail(c, SBQ_ERR_STATE, "sbq_bootstrap before sbq_solve");
+   sbq_ctx::Boot& B = c->boot;
+   B.done = false;
+   int rc = boot_prefix(c);
+   if (rc) return rc;
+   if (!B.scratch.reserve(boot_scratch_bytes(c)) || !B.sums.reserve((size_t)n * 8) || !B.out.reserve(boot_out_bytes(c, n))) {
+      cudaGetLastError();
+      return fail(c, SBQ_ERR_NOMEM, "device allocation failed (%d bootstrap replicates: %zu MB)", n, (boot_out_bytes(c, n) + boot_scratch_bytes(c)) >> 20);
+   }
+   while (B.ev.size() < 2 * (size_t)n + 2) {
+      cudaEvent_t e = nullptr;
+      CU(cudaEventCreate(&e));
+      B.ev.push_back(e);
+   }
+   B.stat = sbq_bootstrap_stat{first, n, 0.0, 0.0, 0.0};
+   const DevParams point = c->dp;
+   rc = boot_replicates(c, seed, first, n);
+   c->dp = point;
+   return rc;
+}
+
+// TPM of every replicate from its FPKM sum in B.sums (multi-GPU: all-reduced), then the timing
+int boot_finish_locked(sbq_ctx* c) {
+   sbq_ctx::Boot& B = c->boot;
+   CU(cudaSetDevice(c->device));
+   cudaStream_t st = c->stream;
+   const int64_t n = B.stat.n, tot = n * c->n_iso;
+   if (tot) {
+      const int blocks = (int)std::min<int64_t>((tot + 255) / 256, (int64_t)c->prop.multiProcessorCount * 16);
+      boot_tpm_kernel<<<blocks, 256, 0, st>>>(boot_out(c, n).tpm, c->n_iso, n, (const double*)B.sums.p);
+      CU(cudaGetLastError());
+   }
+   CU(cudaEventRecord(B.ev[2 * n + 1], st));
+   CU(cudaStreamSynchronize(st));
+   float ms = 0;
+   for (int64_t j = 0; j < n; ++j) {
+      CU(cudaEventElapsedTime(&ms, B.ev[2 * j], B.ev[2 * j + 1]));
+      B.stat.resample_ms += ms;
+      CU(cudaEventElapsedTime(&ms, B.ev[2 * j + 1], B.ev[2 * j + 2]));
+      B.stat.em_ms += ms;
+   }
+   CU(cudaEventElapsedTime(&ms, B.ev[0], B.ev[2 * n + 1]));
+   B.stat.total_ms = ms;
+   B.done = true;
+   return SBQ_SUCCESS;
+}
+
+int boot_counts_locked(sbq_ctx* c, uint64_t seed, int64_t rep, int32_t* count) {
+   CU(cudaSetDevice(c->device));
+   if (!c->resident) return fail(c, SBQ_ERR_STATE, "sbq_bootstrap_counts before sbq_upload");
+   int rc = upload_wait(c);
+   if (!rc) rc = boot_prefix(c);
+   if (rc) return rc;
+   if (!c->boot.scratch.reserve(boot_scratch_bytes(c))) {
+      cudaGetLastError();
+      return fail(c, SBQ_ERR_NOMEM, "device allocation failed (bootstrap counts)");
+   }
+   int32_t* d = (int32_t*)c->boot.scratch.p;
+   if ((rc = boot_resample(c, seed, (uint64_t)rep, d))) return rc;
+   if (c->n_row) CU(cudaMemcpyAsync(count, d, (size_t)c->n_row * 4, cudaMemcpyDeviceToHost, c->stream));
+   CU(cudaStreamSynchronize(c->stream));
+   return SBQ_SUCCESS;
+}
+
+int boot_results_locked(sbq_ctx* c, double* theta, double* tpm, int32_t* iters, int32_t* status) {
+   CU(cudaSetDevice(c->device));
+   if (!c->boot.done) return fail(c, SBQ_ERR_STATE, "sbq_bootstrap_results before sbq_bootstrap");
+   const int64_t n = c->boot.stat.n;
+   const BootOut o = boot_out(c, n);
+   cudaStream_t st = c->stream;
+   const size_t bi = (size_t)n * c->n_iso, bl = (size_t)n * c->n_loci;
+   if (theta && bi) CU(cudaMemcpyAsync(theta, o.theta, bi * 8, cudaMemcpyDeviceToHost, st));
+   if (tpm && bi) CU(cudaMemcpyAsync(tpm, o.tpm, bi * 8, cudaMemcpyDeviceToHost, st));
+   if (iters && bl) CU(cudaMemcpyAsync(iters, o.iters, bl * 4, cudaMemcpyDeviceToHost, st));
+   if (status && bl) CU(cudaMemcpyAsync(status, o.status, bl * 4, cudaMemcpyDeviceToHost, st));
+   CU(cudaStreamSynchronize(st));
+   return SBQ_SUCCESS;
+}
+
+}  // namespace
+
+extern "C" {
+
+int sbq_bootstrap(sbq_ctx* c, uint64_t seed, int64_t first, int32_t n) {
+   if (!c) return SBQ_ERR_INVALID;
+   if (c->cfg.bias_mode == 1) return fail(c, SBQ_ERR_UNSUPPORTED, "bootstrap replicates are defined for the reference EM only (bias_mode = 0)");
+   if (n < 1 || first < 0) return fail(c, SBQ_ERR_INVALID, "sbq_bootstrap: n = %d, first = %lld", n, (long long)first);
+   if (c->multi) return multi_bootstrap(c, seed, first, n);
+   std::lock_guard<std::mutex> lk(c->mu);
+   int rc = boot_em_locked(c, seed, first, n);
+   if (!rc) rc = boot_finish_locked(c);
+   return rc;
+}
+
+int sbq_bootstrap_results(sbq_ctx* c, double* theta, double* tpm, int32_t* iters, int32_t* status) {
+   if (!c) return SBQ_ERR_INVALID;
+   if (c->multi) return multi_bootstrap_results(c, theta, tpm, iters, status);
+   std::lock_guard<std::mutex> lk(c->mu);
+   return boot_results_locked(c, theta, tpm, iters, status);
+}
+
+int sbq_bootstrap_counts(sbq_ctx* c, uint64_t seed, int64_t replicate, int32_t* count) {
+   if (!c) return SBQ_ERR_INVALID;
+   if (!count || replicate < 0) return fail(c, SBQ_ERR_INVALID, "sbq_bootstrap_counts: null output or replicate < 0");
+   if (c->multi) return multi_bootstrap_counts(c, seed, replicate, count);
+   std::lock_guard<std::mutex> lk(c->mu);
+   return boot_counts_locked(c, seed, replicate, count);
+}
+
+int sbq_bootstrap_stats(const sbq_ctx* cc, sbq_bootstrap_stat* out) {
+   if (!cc || !out) return SBQ_ERR_INVALID;
+   sbq_ctx* c = const_cast<sbq_ctx*>(cc);
+   std::lock_guard<std::mutex> lk(c->mu);
+   if (!c->boot.done) return fail(c, SBQ_ERR_STATE, "sbq_bootstrap_stats before sbq_bootstrap");
+   *out = c->boot.stat;
+   return SBQ_SUCCESS;
 }
 
 }  // extern "C"

@@ -224,6 +224,7 @@ int multi_upload(sbq_ctx* c) {
    MultiState& m = *c->multi;
    std::lock_guard<std::mutex> lk(c->mu);
    if (c->n_loci == 0) return fail(c, SBQ_ERR_STATE, "nothing submitted");
+   c->boot.done = false;
    if (c->raw_mode) {   // the loci already sit in their devices' contexts
       for (sbq_ctx* ch : m.child) {
          sbq_set_plan(ch, c->force_tier, c->force_cluster);
@@ -378,6 +379,122 @@ int multi_download(sbq_ctx* c) {
    c->r_fpkm_sum = m.global_sum;
    c->downloaded = true;
    return SBQ_SUCCESS;
+}
+
+// Offsets of the parent batch's rows (what = 0) or isoforms (what = 1) in submit order, rebuilt from the children (the parent's host
+// arrays may be gone: borrowed batch; raw loci never had them)
+std::vector<int64_t> multi_offsets(sbq_ctx* c, int what) {
+   MultiState& m = *c->multi;
+   std::vector<int64_t> off((size_t)c->n_loci + 1, 0);
+   for (size_t i = 0; i < m.child.size(); ++i)
+      for (size_t x = 0; x < m.loci_of[i].size(); ++x) off[m.loci_of[i][x] + 1] = what ? m.child[i]->meta[x].T : m.child[i]->meta[x].R;
+   for (size_t l = 0; l < (size_t)c->n_loci; ++l) off[l + 1] += off[l];
+   return off;
+}
+
+// Bootstrap replicates on N devices. Every child resamples its loci under their PARENT submit positions, so a replicate does not
+// depend on the partition; the n replicate FPKM sums then meet in ONE ncclAllReduce (count n) before every device's TPM pass.
+int multi_bootstrap(sbq_ctx* c, uint64_t seed, int64_t first, int32_t n) {
+   MultiState& m = *c->multi;
+   std::lock_guard<std::mutex> lk(c->mu);
+   if (!c->resident || !c->solved) return fail(c, SBQ_ERR_STATE, "sbq_bootstrap before sbq_solve");
+   c->boot.done = false;
+   const int nd = (int)m.child.size();
+   for (int i = 0; i < nd; ++i) m.child[i]->boot.lid = m.loci_of[i];
+   int rc = multi_for_each(c, [&](int i) {
+      std::lock_guard<std::mutex> lk2(m.child[i]->mu);
+      return boot_em_locked(m.child[i], seed, first, n);
+   });
+   if (rc) return rc;
+   for (int i = 0; i < nd; ++i) {   // devices without loci join the all-reduce with zeros
+      if (!m.loci_of[i].empty()) continue;
+      sbq_ctx* ch = m.child[i];
+      CU(cudaSetDevice(m.devices[i]));
+      if (!ch->boot.sums.reserve((size_t)n * 8)) {
+         cudaGetLastError();
+         return fail(c, SBQ_ERR_NOMEM, "device %d: allocation failed (bootstrap sums)", m.devices[i]);
+      }
+      CU(cudaMemsetAsync(ch->boot.sums.p, 0, (size_t)n * 8, ch->stream));
+   }
+   ncclResult_t r = g_nccl.GroupStart();
+   for (int i = 0; i < nd && r == ncclSuccess; ++i)
+      r = g_nccl.AllReduce(m.child[i]->boot.sums.p, m.child[i]->boot.sums.p, (size_t)n, ncclDouble, ncclSum, m.comm[i], m.child[i]->stream);
+   const ncclResult_t r2 = g_nccl.GroupEnd();
+   if (r != ncclSuccess || r2 != ncclSuccess) return fail(c, SBQ_ERR_CUDA, "ncclAllReduce failed: %s", g_nccl.GetErrorString(r != ncclSuccess ? r : r2));
+   rc = multi_for_each(c, [&](int i) {
+      std::lock_guard<std::mutex> lk2(m.child[i]->mu);
+      return boot_finish_locked(m.child[i]);
+   });
+   if (rc) return rc;
+   sbq_bootstrap_stat s{first, n, 0.0, 0.0, 0.0};   // device times: the slowest device's
+   for (int i = 0; i < nd; ++i) {
+      if (m.loci_of[i].empty()) continue;
+      const sbq_bootstrap_stat& t = m.child[i]->boot.stat;
+      s.resample_ms = std::max(s.resample_ms, t.resample_ms);
+      s.em_ms = std::max(s.em_ms, t.em_ms);
+      s.total_ms = std::max(s.total_ms, t.total_ms);
+   }
+   c->boot.stat = s;
+   c->boot.done = true;
+   return SBQ_SUCCESS;
+}
+
+// the children's replicate matrices, scattered back into submit order like multi_download
+int multi_bootstrap_results(sbq_ctx* c, double* theta, double* tpm, int32_t* iters, int32_t* status) {
+   MultiState& m = *c->multi;
+   std::lock_guard<std::mutex> lk(c->mu);
+   if (!c->boot.done) return fail(c, SBQ_ERR_STATE, "sbq_bootstrap_results before sbq_bootstrap");
+   const int64_t n = c->boot.stat.n, NI = c->n_iso, NL = c->n_loci;
+   const std::vector<int64_t> lio = multi_offsets(c, 1);
+   return multi_for_each(c, [&](int i) {
+      sbq_ctx* ch = m.child[i];
+      const int64_t ni = ch->n_iso, nl = ch->n_loci;
+      std::vector<double> th(theta ? n * ni : 0), tp(tpm ? n * ni : 0);
+      std::vector<int32_t> it(iters ? n * nl : 0), stt(status ? n * nl : 0);
+      {
+         std::lock_guard<std::mutex> lk2(ch->mu);
+         const int r = boot_results_locked(ch, theta ? th.data() : nullptr, tpm ? tp.data() : nullptr, iters ? it.data() : nullptr, status ? stt.data() : nullptr);
+         if (r) return r;
+      }
+      for (int64_t b = 0; b < n; ++b) {
+         int64_t o = 0;
+         for (size_t x = 0; x < m.loci_of[i].size(); ++x) {
+            const int32_t l = m.loci_of[i][x];
+            const int64_t T = lio[l + 1] - lio[l], d = b * NI + lio[l], s = b * ni + o;
+            if (theta) memcpy(theta + d, th.data() + s, T * 8);
+            if (tpm) memcpy(tpm + d, tp.data() + s, T * 8);
+            if (iters) iters[b * NL + l] = it[b * nl + x];
+            if (status) status[b * NL + l] = stt[b * nl + x];
+            o += T;
+         }
+      }
+      return 0;
+   });
+}
+
+int multi_bootstrap_counts(sbq_ctx* c, uint64_t seed, int64_t rep, int32_t* count) {
+   MultiState& m = *c->multi;
+   std::lock_guard<std::mutex> lk(c->mu);
+   if (!c->resident) return fail(c, SBQ_ERR_STATE, "sbq_bootstrap_counts before sbq_upload");
+   for (size_t i = 0; i < m.child.size(); ++i) m.child[i]->boot.lid = m.loci_of[i];
+   const std::vector<int64_t> lro = multi_offsets(c, 0);
+   return multi_for_each(c, [&](int i) {
+      sbq_ctx* ch = m.child[i];
+      std::vector<int32_t> h((size_t)ch->n_row);
+      {
+         std::lock_guard<std::mutex> lk2(ch->mu);
+         const int r = boot_counts_locked(ch, seed, rep, h.data());
+         if (r) return r;
+      }
+      int64_t o = 0;
+      for (size_t x = 0; x < m.loci_of[i].size(); ++x) {
+         const int32_t l = m.loci_of[i][x];
+         const int64_t R = lro[l + 1] - lro[l];
+         memcpy(count + lro[l], h.data() + o, R * 4);
+         o += R;
+      }
+      return 0;
+   });
 }
 
 // aggregate: counts and bytes add up, device times are the slowest device's (the devices run concurrently)
