@@ -250,6 +250,21 @@ int  sbq_bootstrap_counts(sbq_ctx*, uint64_t seed, int64_t replicate, int32_t* c
 typedef struct { int64_t first, n; double resample_ms, em_ms, total_ms; } sbq_bootstrap_stat;
 int  sbq_bootstrap_stats(const sbq_ctx*, sbq_bootstrap_stat* out);
 
+/* Gibbs posterior samples (OUR definition, DESIGN.md "Gibbs posterior samples"; the reference has none). A data-augmentation
+ * Gibbs chain per locus, started from the resident point estimate: every round assigns each kept fragment to an isoform of its
+ * class and redraws the locus' proportions from Dirichlet(counts + prior). Sample s is the state after round
+ * burn_in + (s + 1) * thin; its theta is N_kept * pi, its FPKM / TPM come from the usual epilogue. Loci whose point status is
+ * NO_ROWS or ZERO_DENOM are not sampled (every sample repeats their epilogue). Needs a resident batch solved by sbq_solve;
+ * SBQ_ERR_UNSUPPORTED in bias mode. Device memory: 16 nnz + 16 n_iso per sample + O(n_row + n_iso) bytes (SBQ_ERR_NOMEM leaves
+ * the context usable); the point estimate and later solves / bootstraps are unchanged. */
+int  sbq_gibbs(sbq_ctx*, uint64_t seed, int32_t n, int32_t thin, int32_t burn_in, double prior);
+/* Samples of the last sbq_gibbs, submit order: theta / tpm [n][n_iso], status [n][n_loci] (the point estimate's); any pointer may be NULL. */
+int  sbq_gibbs_results(sbq_ctx*, double* theta, double* tpm, int32_t* status);
+/* Device time of the last sbq_gibbs (CUDA events; multi-GPU: the slowest device). colsum_ms: the one-off setup (weights back in
+ * submitted order, column sums, heavy-row offsets, phi^0); assign_ms / theta_ms: summed over all rounds. */
+typedef struct { int64_t n, rounds; double colsum_ms, assign_ms, theta_ms, total_ms; } sbq_gibbs_stat;
+int  sbq_gibbs_stats(const sbq_ctx*, sbq_gibbs_stat* out);
+
 /* Planner knobs, mainly for tests: force a tier (0 = auto, 1 = warp, 2 = CTA/cluster, 3 = grid) and
  * the cluster size of the CTA tier (0 = auto, else 1, 2, 4, 8, 16). */
 int  sbq_set_plan(sbq_ctx*, int force_tier, int force_cluster);

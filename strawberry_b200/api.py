@@ -32,6 +32,7 @@ ABI_SYMBOLS = [
     "sbq_finalize_tpm", "sbq_results", "sbq_get_stats", "sbq_get_launch_stats", "sbq_em_solve", "sbq_set_plan",
     "sbq_set_covariates", "sbq_bias_results", "sbq_partition_lpt", "sbq_locus_devices", "sbq_synth_giant", "sbq_fetch_batch",
     "sbq_bootstrap", "sbq_bootstrap_results", "sbq_bootstrap_counts", "sbq_bootstrap_stats",
+    "sbq_gibbs", "sbq_gibbs_results", "sbq_gibbs_stats",
 ]
 
 
@@ -85,6 +86,14 @@ class BootstrapStat(ctypes.Structure):
         return {n: getattr(self, n) for n, _ in self._fields_}
 
 
+class GibbsStat(ctypes.Structure):
+    _fields_ = [("n", ctypes.c_int64), ("rounds", ctypes.c_int64), ("colsum_ms", ctypes.c_double), ("assign_ms", ctypes.c_double),
+                ("theta_ms", ctypes.c_double), ("total_ms", ctypes.c_double)]
+
+    def as_dict(self):
+        return {n: getattr(self, n) for n, _ in self._fields_}
+
+
 _lib = None
 
 
@@ -129,6 +138,9 @@ def lib():
         L.sbq_bootstrap_results.argtypes = [ctypes.c_void_p] + [ctypes.c_void_p] * 4
         L.sbq_bootstrap_counts.argtypes = [ctypes.c_void_p, ctypes.c_uint64, ctypes.c_int64, ctypes.c_void_p]
         L.sbq_bootstrap_stats.argtypes = [ctypes.c_void_p, ctypes.POINTER(BootstrapStat)]
+        L.sbq_gibbs.argtypes = [ctypes.c_void_p, ctypes.c_uint64, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.c_double]
+        L.sbq_gibbs_results.argtypes = [ctypes.c_void_p] + [ctypes.c_void_p] * 3
+        L.sbq_gibbs_stats.argtypes = [ctypes.c_void_p, ctypes.POINTER(GibbsStat)]
         _lib = L
     return _lib
 
@@ -364,6 +376,24 @@ class Quantifier:
         """Device time of the last bootstrap(): resample_ms, em_ms (EM + FPKM sum, all replicates) and total_ms."""
         s = BootstrapStat()
         self._chk(self._L.sbq_bootstrap_stats(self._h, ctypes.byref(s)))
+        return s.as_dict()
+
+    def gibbs(self, seed, n, thin=16, burn_in=16, prior=0.01):
+        """n Gibbs posterior samples of the solved, resident batch (DESIGN.md "Gibbs posterior samples"): sample s is the chain's
+        state after round burn_in + (s + 1) * thin, every chain started from the point estimate. theta and tpm shaped (n, n_iso),
+        status (the point estimate's) shaped (n, n_loci), submit order. The point estimate (results()) is unchanged.
+        The defaults (thin 16, burn_in 16, a symmetric Dirichlet(0.01) prior) are this project's choice, not the reference's."""
+        self._chk(self._L.sbq_gibbs(self._h, int(seed) & (2**64 - 1), int(n), int(thin), int(burn_in), float(prior)))
+        st = self.stats()
+        ni, nl = st["n_iso"], st["n_loci"]
+        out = dict(theta=np.empty((n, ni)), tpm=np.empty((n, ni)), status=np.empty((n, nl), np.int32))
+        self._chk(self._L.sbq_gibbs_results(self._h, *[_ptr(out[k]) for k in ("theta", "tpm", "status")]))
+        return out
+
+    def gibbs_stats(self):
+        """Device time of the last gibbs(): n, rounds, colsum_ms (one-off setup), assign_ms and theta_ms (all rounds), total_ms."""
+        s = GibbsStat()
+        self._chk(self._L.sbq_gibbs_stats(self._h, ctypes.byref(s)))
         return s.as_dict()
 
     def em_solve(self, n_iso, row_ptr, col, alpha, count):

@@ -7,7 +7,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libsbq.so")
 SOURCES = ["sbq.cu", "sbq_builder.cpp"]
-DEPS = ["sbq.cu", "sbq_kernels.cuh", "sbq_grid.cuh", "sbq_grid_tma.cuh", "sbq_grid_dual.cuh", "sbq_bias.cuh", "sbq_weights.cuh", "sbq_multi.cuh", "sbq_synth.cuh", "sbq_rawbuild.cuh", "sbq_bootstrap.cuh", "sbq_builder.cpp", os.path.join("..", "..", "include", "sbq.h"),
+DEPS = ["sbq.cu", "sbq_kernels.cuh", "sbq_grid.cuh", "sbq_grid_tma.cuh", "sbq_grid_dual.cuh", "sbq_bias.cuh", "sbq_weights.cuh", "sbq_multi.cuh", "sbq_synth.cuh", "sbq_rawbuild.cuh", "sbq_bootstrap.cuh", "sbq_gibbs.cuh", "sbq_builder.cpp", os.path.join("..", "..", "include", "sbq.h"),
         os.path.join("..", "..", "include", "sbq_builder.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared", "-cudart", "static"]

@@ -31,6 +31,7 @@
 #include "sbq_synth.cuh"
 #include "sbq_rawbuild.cuh"
 #include "sbq_bootstrap.cuh"
+#include "sbq_gibbs.cuh"
 
 using namespace sbq;
 
@@ -228,6 +229,14 @@ struct sbq_ctx {
       sbq_bootstrap_stat stat{};
       std::vector<cudaEvent_t> ev;
    } boot;
+
+   // Gibbs posterior samples (sbq_gibbs): setup + per-round scratch and the sample matrices of the last call
+   struct Gibbs {
+      DevBuf scratch, out, sums;
+      bool done = false;                 // the sample matrices in `out` belong to the resident batch
+      sbq_gibbs_stat stat{};
+      std::vector<cudaEvent_t> ev;       // start, setup end, end, then a ring of (round start, assigned, done) triples
+   } gibbs;
 };
 
 namespace {
@@ -300,7 +309,7 @@ void reset_batch(sbq_ctx* c) {
    c->raw_mode = false;
    c->h_wseg.clear(); c->h_wn.clear(); c->h_wmask.clear(); c->h_wpool.clear(); c->h_wlen.clear(); c->h_wpool_off.clear();
    c->resident = c->solved = c->downloaded = false;
-   c->boot.prefix_ready = c->boot.done = false;
+   c->boot.prefix_ready = c->boot.done = c->gibbs.done = false;
 }
 
 int ensure_origin(sbq_ctx* c) {
@@ -632,6 +641,10 @@ int boot_em_locked(sbq_ctx* c, uint64_t seed, int64_t first, int32_t n);
 int boot_finish_locked(sbq_ctx* c);
 int boot_counts_locked(sbq_ctx* c, uint64_t seed, int64_t rep, int32_t* count);
 int boot_results_locked(sbq_ctx* c, double* theta, double* tpm, int32_t* iters, int32_t* status);
+// Gibbs samples on one device (defined with sbq_gibbs at the end of this file); the caller holds c->mu
+int gibbs_run_locked(sbq_ctx* c, uint64_t seed, int32_t n, int32_t thin, int32_t burn_in, double prior);
+int gibbs_finish_locked(sbq_ctx* c);
+int gibbs_results_locked(sbq_ctx* c, double* theta, double* tpm, int32_t* status);
 
 }  // namespace
 
@@ -758,6 +771,8 @@ void sbq_destroy(sbq_ctx* c) {
    c->h_wseg.release(); c->h_wn.release(); c->h_wmask.release(); c->h_wpool.release(); c->h_wlen.release(); c->h_wpool_off.release(); c->d_weights.release();
    c->boot.prefix.release(); c->boot.scratch.release(); c->boot.out.release(); c->boot.sums.release();
    for (auto& e : c->boot.ev) cudaEventDestroy(e);
+   c->gibbs.scratch.release(); c->gibbs.out.release(); c->gibbs.sums.release();
+   for (auto& e : c->gibbs.ev) cudaEventDestroy(e);
    for (auto& e : c->ev) if (e) cudaEventDestroy(e);
    if (c->ev_fork) cudaEventDestroy(c->ev_fork);
    for (auto& e : c->ev_join) if (e) cudaEventDestroy(e);
@@ -909,7 +924,7 @@ static int upload_begin(sbq_ctx* c) {
    cudaStream_t st = c->copy_st;
    c->upload_pending = true;
    c->resident = c->solved = c->downloaded = false;
-   c->boot.prefix_ready = c->boot.done = false;
+   c->boot.prefix_ready = c->boot.done = c->gibbs.done = false;
    CU(cudaEventRecord(c->ev[0], st));
    CU(cudaMemcpyAsync(d_lro, loc_row_off(c), (c->n_loci + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
    CU(cudaMemcpyAsync(d_lio, loc_iso_off(c), (c->n_loci + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
@@ -1640,7 +1655,7 @@ int rb_scan(cudaStream_t st, const int32_t* v, int64_t n, long long* block_tmp, 
 static int raw_upload(sbq_ctx* c) {
    CU(cudaSetDevice(c->device));
    if (!c->have_model && !c->raw.long_read) return fail(c, SBQ_ERR_STATE, "raw loci need sbq_set_insert_model()");
-   c->boot.prefix_ready = c->boot.done = false;
+   c->boot.prefix_ready = c->boot.done = c->gibbs.done = false;
    auto& r = c->raw;
    const int64_t L = c->n_loci, H = (int64_t)r.hit_locus.size(), T = c->n_iso, S = (int64_t)r.seg_left.size();
    const int64_t* lio = c->h_loc_iso_off.p;
@@ -2390,6 +2405,245 @@ int sbq_bootstrap_stats(const sbq_ctx* cc, sbq_bootstrap_stat* out) {
    std::lock_guard<std::mutex> lk(c->mu);
    if (!c->boot.done) return fail(c, SBQ_ERR_STATE, "sbq_bootstrap_stats before sbq_bootstrap");
    *out = c->boot.stat;
+   return SBQ_SUCCESS;
+}
+
+}  // extern "C"
+
+// ================================================================================================
+// Gibbs posterior samples (sbq_gibbs.cuh; DESIGN.md "Gibbs posterior samples")
+namespace {
+
+constexpr int GIBBS_RING = 256;   // rounds whose events are in flight before the oldest is read back
+
+struct GibbsOut {
+   double *theta, *tpm;
+   int32_t* status;
+};
+
+size_t gibbs_out_bytes(const sbq_ctx* c, int64_t n) { return 2 * align_up((size_t)n * c->n_iso * 8) + align_up((size_t)n * c->n_loci * 4); }
+
+GibbsOut gibbs_out(const sbq_ctx* c, int64_t n) {
+   char* q = (char*)c->gibbs.out.p;
+   GibbsOut o;
+   o.theta = (double*)q; q += align_up((size_t)n * c->n_iso * 8);
+   o.tpm = (double*)q; q += align_up((size_t)n * c->n_iso * 8);
+   o.status = (int32_t*)q;
+   return o;
+}
+
+// scratch of one call: weights in submitted order and running sums [nnz]; s, phi, gammas / sample theta, NA flags, frac [n_iso];
+// counts, keep [n_iso]; gn, hv, row -> locus [n_row]; heavy-draw offsets [n_row + 1]; scan blocks; N_kept, locus FPKM [n_loci];
+// iters [n_loci]
+struct GibbsScratch {
+   double *ga, *cum, *s, *phi, *gbuf, *nabuf, *frac, *nkept, *lfpkm;
+   int32_t *cnt, *keep, *gn, *hv, *row_loc, *iters;
+   int64_t* hoff;
+   long long* scan_tmp;
+};
+
+size_t gibbs_scratch_layout(const sbq_ctx* c, GibbsScratch* g) {
+   const size_t nz = align_up(c->nnz * 8 + 8), di = align_up(c->n_iso * 8 + 8), ii = align_up(c->n_iso * 4 + 4);
+   const size_t ri = align_up(c->n_row * 4 + 4), ro = align_up((c->n_row + 1) * 8);
+   const size_t nb = align_up(((c->n_row + RB_SCAN_BLOCK - 1) / RB_SCAN_BLOCK + 1) * 8);
+   const size_t ld = align_up(c->n_loci * 8 + 8), li = align_up(c->n_loci * 4 + 4);
+   const size_t total = 2 * nz + 5 * di + 2 * ii + 3 * ri + ro + nb + 2 * ld + li;
+   if (!g) return total;
+   char* q = (char*)c->gibbs.scratch.p;
+   auto take = [&](size_t b) { char* r = q; q += b; return r; };
+   g->ga = (double*)take(nz); g->cum = (double*)take(nz);
+   g->s = (double*)take(di); g->phi = (double*)take(di); g->gbuf = (double*)take(di); g->nabuf = (double*)take(di); g->frac = (double*)take(di);
+   g->cnt = (int32_t*)take(ii); g->keep = (int32_t*)take(ii);
+   g->gn = (int32_t*)take(ri); g->hv = (int32_t*)take(ri); g->row_loc = (int32_t*)take(ri);
+   g->hoff = (int64_t*)take(ro);
+   g->scan_tmp = (long long*)take(nb);
+   g->nkept = (double*)take(ld); g->lfpkm = (double*)take(ld);
+   g->iters = (int32_t*)take(li);
+   return total;
+}
+
+// The one-off setup of a call on c->stream: ga = alpha in submitted CSR order (the giant tier's layout passes reorder rows in
+// place), column sums, row filter, heavy-draw offsets, phi^0 = theta_hat / s.
+int gibbs_setup(sbq_ctx* c, const GibbsScratch& g) {
+   cudaStream_t st = c->stream;
+   const DevParams& dp = c->dp;
+   const int sms = c->prop.multiProcessorCount;
+   if (c->nnz) CU(cudaMemcpyAsync(g.ga, dp.alpha, (size_t)c->nnz * 8, cudaMemcpyDeviceToDevice, st));
+   if (c->col16_ready) {
+      for (const GridClass& gc : c->grid) {
+         const int32_t* list = c->d_lists_p + gc.list_off;
+         const unsigned short* c16 = (const unsigned short*)c->d_col16.p;
+         if (gc.n_dual) gibbs_unpermute_kernel<<<sms * 8, 256, 0, st>>>(dp, list, (int)gc.n_dual, c16, 1, g.ga);
+         if (gc.n_tma) gibbs_unpermute_kernel<<<sms * 8, 256, 0, st>>>(dp, list + gc.n_dual, (int)gc.n_tma, c16, 0, g.ga);
+         CU(cudaGetLastError());
+      }
+   }
+   if (c->n_iso) CU(cudaMemsetAsync(g.s, 0, (size_t)c->n_iso * 8, st));
+   if (c->n_iso) CU(cudaMemsetAsync(g.cnt, 0, (size_t)c->n_iso * 4, st));
+   if (c->n_loci) {
+      gibbs_colsum_kernel<<<(unsigned)std::min<int64_t>((c->n_loci + 7) / 8, (int64_t)sms * 16), 256, 0, st>>>(dp, g.ga, c->n_loci, g.s, g.gn, g.hv, g.row_loc, g.nkept);
+      CU(cudaGetLastError());
+   }
+   if (rb_scan(st, g.hv, c->n_row, g.scan_tmp, g.hoff)) return fail(c, SBQ_ERR_CUDA, "gibbs heavy-draw prefix: %s", cudaGetErrorString(cudaGetLastError()));
+   if (c->n_iso) {
+      gibbs_init_kernel<<<(unsigned)std::min<int64_t>((c->n_iso + 255) / 256, (int64_t)sms * 16), 256, 0, st>>>(dp.theta, g.s, c->n_iso, g.phi);
+      CU(cudaGetLastError());
+   }
+   return SBQ_SUCCESS;
+}
+
+// elapsed times of ring slot `slot` into the stat
+int gibbs_read_slot(sbq_ctx* c, int slot) {
+   cudaEvent_t* e = c->gibbs.ev.data() + 3 + 3 * slot;
+   float a = 0, t = 0;
+   CU(cudaEventSynchronize(e[2]));
+   CU(cudaEventElapsedTime(&a, e[0], e[1]));
+   CU(cudaEventElapsedTime(&t, e[1], e[2]));
+   c->gibbs.stat.assign_ms += a;
+   c->gibbs.stat.theta_ms += t;
+   return SBQ_SUCCESS;
+}
+
+int gibbs_run_locked(sbq_ctx* c, uint64_t seed, int32_t n, int32_t thin, int32_t burn_in, double prior) {
+   CU(cudaSetDevice(c->device));
+   if (!c->resident || !c->solved) return fail(c, SBQ_ERR_STATE, "sbq_gibbs before sbq_solve");
+   sbq_ctx::Gibbs& G = c->gibbs;
+   G.done = false;
+   int rc = boot_prefix(c);   // draw offsets (and the 2^31-fragment refusal) and the loci's hash positions
+   if (rc) return rc;
+   const size_t sb = gibbs_scratch_layout(c, nullptr);
+   if (!G.scratch.reserve(sb) || !G.sums.reserve((size_t)n * 8) || !G.out.reserve(gibbs_out_bytes(c, n))) {
+      cudaGetLastError();   // a failed allocation is not an error of the context
+      return fail(c, SBQ_ERR_NOMEM, "device allocation failed (%d Gibbs samples: %zu MB)", n, (gibbs_out_bytes(c, n) + sb) >> 20);
+   }
+   while (G.ev.size() < 3 + 3 * (size_t)GIBBS_RING) {
+      cudaEvent_t e = nullptr;
+      CU(cudaEventCreate(&e));
+      G.ev.push_back(e);
+   }
+   GibbsScratch g;
+   gibbs_scratch_layout(c, &g);
+   const int64_t rounds = (int64_t)burn_in + (int64_t)n * thin;
+   G.stat = sbq_gibbs_stat{n, rounds, 0.0, 0.0, 0.0, 0.0};
+   cudaStream_t st = c->stream;
+   const sbq_ctx::Boot& B = c->boot;
+   const int32_t* lid = B.lid.empty() ? nullptr : B.d_lid;
+   const int sms = c->prop.multiProcessorCount;
+   CU(cudaEventRecord(G.ev[0], st));
+   if ((rc = gibbs_setup(c, g))) return rc;
+   CU(cudaEventRecord(G.ev[1], st));
+   const GibbsOut o = gibbs_out(c, n);
+   const uint64_t skey = sm64(seed ^ GIBBS_SALT);
+   const unsigned row_blocks = (unsigned)std::max<int64_t>(1, std::min<int64_t>((c->n_row + 255) / 256, (int64_t)sms * 16));
+   const unsigned loc_blocks = (unsigned)std::max<int64_t>(1, std::min<int64_t>(c->n_loci, (int64_t)sms * 8));
+   DevParams sp = c->dp;   // the sample's slots: theta / FPKM / status of the output matrices, the rest scratch
+   sp.frac = g.frac;
+   sp.keep = g.keep;
+   sp.iters = g.iters;
+   sp.locus_fpkm = g.lfpkm;
+   for (int64_t r = 1; r <= rounds; ++r) {
+      const int slot = (int)((r - 1) % GIBBS_RING);
+      if (r > GIBBS_RING && (rc = gibbs_read_slot(c, slot))) return rc;
+      cudaEvent_t* e = G.ev.data() + 3 + 3 * slot;
+      const uint64_t rkey = sm64(skey + (uint64_t)r);
+      CU(cudaEventRecord(e[0], st));
+      if (c->n_row) {
+         gibbs_assign_kernel<<<row_blocks, 256, 0, st>>>(c->dp, g.ga, g.gn, g.row_loc, B.draw_off, B.loc_draw_off, lid, g.phi, rkey, c->n_row, g.cum, g.cnt);
+         gibbs_heavy_kernel<<<sms * 8, 256, 0, st>>>(c->dp, g.hoff, c->n_row, g.row_loc, B.draw_off, B.loc_draw_off, lid, rkey, g.cum, g.cnt);
+         CU(cudaGetLastError());
+      }
+      CU(cudaEventRecord(e[1], st));
+      const int64_t sr = r - burn_in;
+      const int sample = sr > 0 && sr % thin == 0;
+      const int64_t s = sample ? sr / thin - 1 : 0;
+      if (sample) {
+         sp.theta = o.theta + s * c->n_iso;
+         sp.fpkm = o.tpm + s * c->n_iso;   // FPKM now, TPM after the last round (gibbs_finish_locked)
+         sp.status = o.status + s * c->n_loci;
+      }
+      if (c->n_loci) {
+         gibbs_theta_kernel<<<loc_blocks, GIBBS_NT, 0, st>>>(sp, c->n_loci, c->dp.theta, c->dp.status, g.s, g.nkept, lid, rkey, prior, sample, g.cnt, g.phi, g.gbuf, g.nabuf);
+         CU(cudaGetLastError());
+      }
+      if (sample) {
+         fpkm_sum_kernel<<<1, 1024, 0, st>>>(g.lfpkm, c->n_loci, (double*)G.sums.p + s);
+         CU(cudaGetLastError());
+      }
+      CU(cudaEventRecord(e[2], st));
+   }
+   return SBQ_SUCCESS;
+}
+
+// TPM of every sample from its FPKM sum in G.sums (multi-GPU: all-reduced), then the timing
+int gibbs_finish_locked(sbq_ctx* c) {
+   sbq_ctx::Gibbs& G = c->gibbs;
+   CU(cudaSetDevice(c->device));
+   cudaStream_t st = c->stream;
+   const int64_t n = G.stat.n, tot = n * c->n_iso;
+   if (tot) {
+      const int blocks = (int)std::min<int64_t>((tot + 255) / 256, (int64_t)c->prop.multiProcessorCount * 16);
+      boot_tpm_kernel<<<blocks, 256, 0, st>>>(gibbs_out(c, n).tpm, c->n_iso, n, (const double*)G.sums.p);
+      CU(cudaGetLastError());
+   }
+   CU(cudaEventRecord(G.ev[2], st));
+   CU(cudaStreamSynchronize(st));
+   const int64_t rounds = G.stat.rounds;
+   for (int64_t r = std::max<int64_t>(1, rounds - GIBBS_RING + 1); r <= rounds; ++r) {
+      const int rc = gibbs_read_slot(c, (int)((r - 1) % GIBBS_RING));
+      if (rc) return rc;
+   }
+   float ms = 0;
+   CU(cudaEventElapsedTime(&ms, G.ev[0], G.ev[1]));
+   G.stat.colsum_ms = ms;
+   CU(cudaEventElapsedTime(&ms, G.ev[0], G.ev[2]));
+   G.stat.total_ms = ms;
+   G.done = true;
+   return SBQ_SUCCESS;
+}
+
+int gibbs_results_locked(sbq_ctx* c, double* theta, double* tpm, int32_t* status) {
+   CU(cudaSetDevice(c->device));
+   if (!c->gibbs.done) return fail(c, SBQ_ERR_STATE, "sbq_gibbs_results before sbq_gibbs");
+   const int64_t n = c->gibbs.stat.n;
+   const GibbsOut o = gibbs_out(c, n);
+   cudaStream_t st = c->stream;
+   const size_t bi = (size_t)n * c->n_iso, bl = (size_t)n * c->n_loci;
+   if (theta && bi) CU(cudaMemcpyAsync(theta, o.theta, bi * 8, cudaMemcpyDeviceToHost, st));
+   if (tpm && bi) CU(cudaMemcpyAsync(tpm, o.tpm, bi * 8, cudaMemcpyDeviceToHost, st));
+   if (status && bl) CU(cudaMemcpyAsync(status, o.status, bl * 4, cudaMemcpyDeviceToHost, st));
+   CU(cudaStreamSynchronize(st));
+   return SBQ_SUCCESS;
+}
+
+}  // namespace
+
+extern "C" {
+
+int sbq_gibbs(sbq_ctx* c, uint64_t seed, int32_t n, int32_t thin, int32_t burn_in, double prior) {
+   if (!c) return SBQ_ERR_INVALID;
+   if (c->cfg.bias_mode == 1) return fail(c, SBQ_ERR_UNSUPPORTED, "Gibbs samples are defined for the reference EM only (bias_mode = 0)");
+   if (n < 1 || thin < 1 || burn_in < 0 || !(prior > 0.0 && prior < INFINITY))
+      return fail(c, SBQ_ERR_INVALID, "sbq_gibbs: n = %d, thin = %d, burn_in = %d, prior = %g", n, thin, burn_in, prior);
+   if (c->multi) return multi_gibbs(c, seed, n, thin, burn_in, prior);
+   std::lock_guard<std::mutex> lk(c->mu);
+   int rc = gibbs_run_locked(c, seed, n, thin, burn_in, prior);
+   if (!rc) rc = gibbs_finish_locked(c);
+   return rc;
+}
+
+int sbq_gibbs_results(sbq_ctx* c, double* theta, double* tpm, int32_t* status) {
+   if (!c) return SBQ_ERR_INVALID;
+   if (c->multi) return multi_gibbs_results(c, theta, tpm, status);
+   std::lock_guard<std::mutex> lk(c->mu);
+   return gibbs_results_locked(c, theta, tpm, status);
+}
+
+int sbq_gibbs_stats(const sbq_ctx* cc, sbq_gibbs_stat* out) {
+   if (!cc || !out) return SBQ_ERR_INVALID;
+   sbq_ctx* c = const_cast<sbq_ctx*>(cc);
+   std::lock_guard<std::mutex> lk(c->mu);
+   if (!c->gibbs.done) return fail(c, SBQ_ERR_STATE, "sbq_gibbs_stats before sbq_gibbs");
+   *out = c->gibbs.stat;
    return SBQ_SUCCESS;
 }
 

@@ -224,7 +224,7 @@ int multi_upload(sbq_ctx* c) {
    MultiState& m = *c->multi;
    std::lock_guard<std::mutex> lk(c->mu);
    if (c->n_loci == 0) return fail(c, SBQ_ERR_STATE, "nothing submitted");
-   c->boot.done = false;
+   c->boot.done = c->gibbs.done = false;
    if (c->raw_mode) {   // the loci already sit in their devices' contexts
       for (sbq_ctx* ch : m.child) {
          sbq_set_plan(ch, c->force_tier, c->force_cluster);
@@ -492,6 +492,86 @@ int multi_bootstrap_counts(sbq_ctx* c, uint64_t seed, int64_t rep, int32_t* coun
          const int64_t R = lro[l + 1] - lro[l];
          memcpy(count + lro[l], h.data() + o, R * 4);
          o += R;
+      }
+      return 0;
+   });
+}
+
+// Gibbs samples on N devices, as multi_bootstrap: every child samples its loci under their PARENT submit positions, the n sample
+// FPKM sums meet in ONE ncclAllReduce before every device's TPM pass.
+int multi_gibbs(sbq_ctx* c, uint64_t seed, int32_t n, int32_t thin, int32_t burn_in, double prior) {
+   MultiState& m = *c->multi;
+   std::lock_guard<std::mutex> lk(c->mu);
+   if (!c->resident || !c->solved) return fail(c, SBQ_ERR_STATE, "sbq_gibbs before sbq_solve");
+   c->gibbs.done = false;
+   const int nd = (int)m.child.size();
+   for (int i = 0; i < nd; ++i) m.child[i]->boot.lid = m.loci_of[i];
+   int rc = multi_for_each(c, [&](int i) {
+      std::lock_guard<std::mutex> lk2(m.child[i]->mu);
+      return gibbs_run_locked(m.child[i], seed, n, thin, burn_in, prior);
+   });
+   if (rc) return rc;
+   for (int i = 0; i < nd; ++i) {   // devices without loci join the all-reduce with zeros
+      if (!m.loci_of[i].empty()) continue;
+      sbq_ctx* ch = m.child[i];
+      CU(cudaSetDevice(m.devices[i]));
+      if (!ch->gibbs.sums.reserve((size_t)n * 8)) {
+         cudaGetLastError();
+         return fail(c, SBQ_ERR_NOMEM, "device %d: allocation failed (Gibbs sums)", m.devices[i]);
+      }
+      CU(cudaMemsetAsync(ch->gibbs.sums.p, 0, (size_t)n * 8, ch->stream));
+   }
+   ncclResult_t r = g_nccl.GroupStart();
+   for (int i = 0; i < nd && r == ncclSuccess; ++i)
+      r = g_nccl.AllReduce(m.child[i]->gibbs.sums.p, m.child[i]->gibbs.sums.p, (size_t)n, ncclDouble, ncclSum, m.comm[i], m.child[i]->stream);
+   const ncclResult_t r2 = g_nccl.GroupEnd();
+   if (r != ncclSuccess || r2 != ncclSuccess) return fail(c, SBQ_ERR_CUDA, "ncclAllReduce failed: %s", g_nccl.GetErrorString(r != ncclSuccess ? r : r2));
+   rc = multi_for_each(c, [&](int i) {
+      std::lock_guard<std::mutex> lk2(m.child[i]->mu);
+      return gibbs_finish_locked(m.child[i]);
+   });
+   if (rc) return rc;
+   sbq_gibbs_stat s{n, (int64_t)burn_in + (int64_t)n * thin, 0.0, 0.0, 0.0, 0.0};   // device times: the slowest device's
+   for (int i = 0; i < nd; ++i) {
+      if (m.loci_of[i].empty()) continue;
+      const sbq_gibbs_stat& t = m.child[i]->gibbs.stat;
+      s.colsum_ms = std::max(s.colsum_ms, t.colsum_ms);
+      s.assign_ms = std::max(s.assign_ms, t.assign_ms);
+      s.theta_ms = std::max(s.theta_ms, t.theta_ms);
+      s.total_ms = std::max(s.total_ms, t.total_ms);
+   }
+   c->gibbs.stat = s;
+   c->gibbs.done = true;
+   return SBQ_SUCCESS;
+}
+
+// the children's sample matrices, scattered back into submit order like multi_bootstrap_results
+int multi_gibbs_results(sbq_ctx* c, double* theta, double* tpm, int32_t* status) {
+   MultiState& m = *c->multi;
+   std::lock_guard<std::mutex> lk(c->mu);
+   if (!c->gibbs.done) return fail(c, SBQ_ERR_STATE, "sbq_gibbs_results before sbq_gibbs");
+   const int64_t n = c->gibbs.stat.n, NI = c->n_iso, NL = c->n_loci;
+   const std::vector<int64_t> lio = multi_offsets(c, 1);
+   return multi_for_each(c, [&](int i) {
+      sbq_ctx* ch = m.child[i];
+      const int64_t ni = ch->n_iso, nl = ch->n_loci;
+      std::vector<double> th(theta ? n * ni : 0), tp(tpm ? n * ni : 0);
+      std::vector<int32_t> stt(status ? n * nl : 0);
+      {
+         std::lock_guard<std::mutex> lk2(ch->mu);
+         const int r = gibbs_results_locked(ch, theta ? th.data() : nullptr, tpm ? tp.data() : nullptr, status ? stt.data() : nullptr);
+         if (r) return r;
+      }
+      for (int64_t b = 0; b < n; ++b) {
+         int64_t o = 0;
+         for (size_t x = 0; x < m.loci_of[i].size(); ++x) {
+            const int32_t l = m.loci_of[i][x];
+            const int64_t T = lio[l + 1] - lio[l], d = b * NI + lio[l], s = b * ni + o;
+            if (theta) memcpy(theta + d, th.data() + s, T * 8);
+            if (tpm) memcpy(tpm + d, tp.data() + s, T * 8);
+            if (status) status[b * NL + l] = stt[b * nl + x];
+            o += T;
+         }
       }
       return 0;
    });
